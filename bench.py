@@ -11,7 +11,7 @@ fits one GPU, so N = 1 runs the same workload; for N > 1 the entity table, its o
 sharded BY ROW over the ranks (trainer.RowShardedAllEntityStepper: three O(batch * d) all-reduces per step) and the
 per-step batch stays 1,024 triples: strong scaling.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line.  `value`: batches resident in HBM, CUDA-event timed, max over ranks.  `e2e`: the same step through
 the REFERENCE's own job object (baseline/_ref, unmodified `TrainingJob1vsAll` created by `Job.create` with the B200
@@ -140,7 +140,7 @@ def run_cpu_reference(batches, steps, warmup, job=None):
             "loss_step0": losses[0], "job": job}
 
 
-def reference_cuda(batches, local_rank, steps=5, warmup=2):
+def reference_cuda(batches, local_rank, steps, warmup=2):
     """SURVEY.md 8(d), last paragraph: the reference's own CUDA path -- the UNMODIFIED reference with its stock model and
     torch.optim.Adagrad, job.device cuda -- on the same GPU, same config and batches: 'same API, stock kernels'.  Timed like
     the e2e figure (pinned host triples in, loss read back by the job) with CUDA events around the steps."""
@@ -179,8 +179,8 @@ def reference_arm(args):
     if not ref_env.available():
         print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref is not installed (baseline/install_ref.sh)"}))
         return
-    # a reference step at this shape takes tens of seconds: the run is bounded to a few minutes
-    steps, warm = max(1, min(args.steps, 3)), min(args.warmup, 1)
+    # a reference step at this shape takes tens of seconds on the host: --steps 20 runs for several minutes
+    steps, warm = args.steps, min(args.warmup, 1)
     batches = make_batches(steps + warm)
     res = run_cpu_reference(batches, steps, warm)
     print(json.dumps({
@@ -217,6 +217,43 @@ def device_batch(t: torch.Tensor, dev):
     z = torch.zeros(len(t), dtype=torch.int32, device=dev)
     return (torch.cat((s, o)), torch.cat((p, p)), torch.cat((z, z + 1)),
             torch.arange(2 * len(t) + 1, dtype=torch.int64, device=dev), torch.cat((o, s)))
+
+
+DUMP_SAMPLE_ROWS, DUMP_SAMPLE_SEED = 32768, 11
+# where the tables the timed steps start from come from (index = initial_tables.npy of --dump-outputs)
+INITIAL_TABLES = ("KgeModel under torch.manual_seed(0)",
+                  "the reference's TrainingJob1vsAll with the plug-in model on the GPU (baseline/_ref), after one step "
+                  "that captures the stepper",
+                  "as 1, with the CPU reference job's tables loaded first (--cpu-steps > 0)")
+
+
+def dump_outputs(out_dir, st, loss, last_batch, initial_tables, rank, world):
+    """Writes what the timed step hands its caller after the last timed step as float32 .npy files under out_dir (about
+    36 MB): the batch's loss, the relation table and its Adagrad state, and rows of the entity table and of its Adagrad
+    state -- the rows of the step's own entities (`*_batch`) and a fixed, seeded sample of all rows (`*_sample`; the
+    whole table is 2.36 GB).  The row ids go along as float64, and initial_tables.npy holds the index into INITIAL_TABLES
+    of the path that made the starting tables: that path depends on whether baseline/_ref is installed.  Runs of two
+    builds on the same arguments and the same path start from the same tables and batches, so their files can be compared
+    array by array."""
+    if world > 1:
+        st.sync_tables()          # every rank then holds the whole, current entity table and its state
+    if rank != 0:
+        return
+    ent, rel = st.ent.detach(), st.rel.detach()
+    s_ent, s_rel = st.opt.state[st.ent]["sum"], st.opt.state[st.rel]["sum"]
+    batch_ids = torch.unique(torch.cat((last_batch[:, 0], last_batch[:, 2]))).to(ent.device)
+    rng = np.random.default_rng(DUMP_SAMPLE_SEED)
+    sample_ids = np.sort(rng.choice(E, min(E, DUMP_SAMPLE_ROWS), replace=False))
+    sample_ids = torch.from_numpy(sample_ids).to(ent.device)
+    arrays = {"loss": loss.detach().reshape(()), "relation_table": rel, "relation_adagrad_sum": s_rel,
+              "initial_tables": torch.tensor(float(initial_tables), dtype=torch.float64)}
+    for tag, ids in (("batch", batch_ids), ("sample", sample_ids)):
+        arrays[f"entity_ids_{tag}"] = ids.double()
+        arrays[f"entity_rows_{tag}"] = ent[ids]
+        arrays[f"entity_adagrad_sum_{tag}"] = s_ent[ids]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def kernel_roofline(kb, st, rows, n_ent, step_ms, world):
@@ -349,6 +386,7 @@ def our_arm(args):
 
     ref_job, parity, cpu = None, None, None
     use_ref = world == 1 and ref_env.available() and not args.no_reference_job
+    initial_tables = 0 if not use_ref else (2 if args.cpu_steps > 0 else 1)
     if use_ref:
         # the reference's own TrainingJob1vsAll, created by its factories with the plug-in model on cuda
         ref_job = reference_job(f"cuda:{local_rank}", plugin=True, plugin_args={"math": "bf16", "captured_step": True})
@@ -416,9 +454,12 @@ def our_arm(args):
         for i in range(steps):
             set_batch(warm + i)
             evs[i][0].record()
-            st.step()
+            loss = st.step()
             evs[i][1].record()
         barrier()
+    if args.dump_outputs:
+        # here: the e2e leg below trains the tables further
+        dump_outputs(args.dump_outputs, st, loss, batches[warm + steps - 1], initial_tables, rank, world)
     total_ms = float(np.sum([a.elapsed_time(b) for a, b in evs]))
     if world > 1:
         t = torch.tensor([total_ms], device=dev)
@@ -458,11 +499,11 @@ def our_arm(args):
     extra = None
     if world == 1 and not args.skip_extra:
         del dev_inputs
-        fb_args = bench_fb237.parser().parse_args(["--steps", str(max(steps, 20)), "--warmup", "5", "--cpu-steps", "3"])
+        fb_args = bench_fb237.parser().parse_args(["--steps", str(steps), "--warmup", "5", "--cpu-steps", "3"])
         with quiet():
             extra = {"fb15k237": bench_fb237.run(fb_args)}
         if use_ref and not args.skip_reference_cuda:
-            extra["reference_cuda"] = reference_cuda(batches, local_rank)
+            extra["reference_cuda"] = reference_cuda(batches, local_rank, steps=steps)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -475,6 +516,7 @@ def our_arm(args):
         "details": {"math": "bf16 tensor tiles (tcgen05, bf16 mirror of the table), fp32 accumulate, fp32 master tables "
                             "and optimizer", "cuda_graph": True, "final_loss": final_loss,
                     "flash_fallbacks": getattr(st, "flash_fallbacks", None),
+                    "initial_tables": INITIAL_TABLES[initial_tables],
                     "stepper": type(st).__name__ + (" inside the reference's TrainingJob1vsAll" if use_ref else ""),
                     "exchange": (None if world == 1 else ("one-shot all-reduce kernels over NVLink peer memory inside the "
                                  "step's CUDA graph (kgeb_p2p_allreduce)" if getattr(st, "px", None) is not None else
@@ -504,7 +546,9 @@ def our_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed training steps of each workload and arm (the CPU sample inside a GPU run: --cpu-steps; "
+                         "the roofline times single kernels separately)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cpu-steps", type=int, default=1, help="timed steps of the bounded CPU-baseline sample (N = 1)")
@@ -512,7 +556,12 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true", help="tuning runs: device-resident value + kernel roofline only")
     ap.add_argument("--skip-extra", action="store_true", help="do not run the FB15k-237 workload (extra key)")
     ap.add_argument("--no-reference-job", action="store_true", help="e2e through this repo's stepper instead of the reference's job object")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, tables and Adagrad state after the last timed step as .npy files to DIR "
+                         "(entity rows: the step's own and a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         reference_arm(args)
     else:

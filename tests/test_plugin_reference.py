@@ -1,6 +1,7 @@
-"""The reference-side plug-in (kge-1_b200/libkge_plugin.py) against the real reference, in the build container only
-(/root/reference does not travel to the GPU box: skipped there).  CPU: checks discovery through the reference's own
-factories, the class contract, checkpoint-key compatibility and that the CUDA path fails loudly without a GPU."""
+"""The reference-side plug-in (kge-1_b200/libkge_plugin.py) against the real reference, the unmodified LibKGE fork that
+baseline/install_ref.sh installs into the git-ignored baseline/_ref (skipped where it is not installed).  CPU: checks
+discovery through the reference's own factories, the class contract, checkpoint-key compatibility and that the CUDA path
+fails loudly without a GPU."""
 import os
 import sys
 import tempfile
@@ -9,16 +10,15 @@ import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "kge")), reason="the reference tree is not on this machine")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+from baseline import ref_env  # noqa: E402
+
+pytestmark = pytest.mark.skipif(not ref_env.available(), reason="baseline/_ref is not installed")
 
 
 @pytest.fixture(scope="module")
 def ref():
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    import ref_import
-    ref_import.install(REF)
-    import kge  # noqa: F401
+    ref_env.install()
     import kgeb200
     kgeb200.libkge_plugin.register()
     kgeb200.libkge_plugin.register()      # idempotent
