@@ -4,6 +4,7 @@ parity-test shapes, not the bench line (bench.py is the contract's benchmark); r
 profiles/extra_workloads_r1.jsonl and summarised in DESIGN.md.
 
     python bench_extra.py --workload wd5m-1vsall | wnrr-rotate-ns | wd5m-eval-transe | wd5m-eval-complex [--scale F]
+    python bench_extra.py --workload wd5m-1vsall-reciprocal --batch 1024
 """
 import argparse
 import json
@@ -104,6 +105,54 @@ def wd5m_1vsall(args):
             "roofline": {"tensor_tflops": flops / (ms * 1e-3) / 1e12, "tensor_frac_of_bf16_sustained": flops / (ms * 1e-3) / 1e12 / tf,
                          "hbm_gbs": bytes_step / (ms * 1e-3) / 1e9, "hbm_frac": bytes_step / (ms * 1e-3) / 1e9 / hbm,
                          "algorithmic_bytes_per_step": bytes_step, "algorithmic_flops_per_step": flops}}
+
+
+def wd5m_1vsall_reciprocal(args):
+    """DistMult with reciprocal relations (2 R relation rows, _po queries as sp_ queries on p + R), 1vsAll + KL, d=128,
+    E=4.6M (scaled by --scale), --batch triples per step, against plain DistMult in the same process: both captured steps
+    build their batch from the triples on the device (onevsall_triples), so the two differ only in the batch builder
+    (kgeb_onevsall_batch_build_inv with R vs 0) and in the relation table's row count.  The two steppers are timed in
+    alternating rounds of --steps steps; the medians are reported."""
+    E, R, d, B = int(4_600_000 * args.scale), 822, 128, args.batch
+    dev = torch.device("cuda")
+    math_mode = {"bf16": kb.lib.MATH_BF16, "tf32": kb.lib.MATH_TF32, "fp32": kb.lib.MATH_FP32}[args.math]
+    arms = {}
+    for name in ("plain", "reciprocal"):
+        torch.manual_seed(0)
+        if name == "plain":
+            model = kb.KgeModel("distmult", E, R, d).to(dev)
+        else:
+            model = kb.model.ReciprocalRelationsModel("distmult", E, R, d).to(dev)
+        opt = kb.optim.create("Adagrad", model.parameters(), lr=0.2)
+        st = kb.trainer.FusedAllEntityStepper(model, opt, 2 * B, 2 * B, kb.lib.LOSS_KL, B, math_mode=math_mode,
+                                              onevsall_triples=True, reciprocal=name == "reciprocal")
+        gen = torch.Generator(device=dev).manual_seed(1)
+        batches = [torch.stack((torch.randint(0, E, (B,), device=dev, generator=gen),
+                                torch.randint(0, R, (B,), device=dev, generator=gen),
+                                torch.randint(0, E, (B,), device=dev, generator=gen)), 1) for _ in range(8)]
+        arms[name] = dict(st=st, batches=batches, i=0, ms=[])
+
+    def stepper_fn(arm):
+        def step():
+            arm["st"].set_triples(arm["batches"][arm["i"] % len(arm["batches"])])
+            arm["i"] += 1
+            arm["st"].step()
+        return step
+
+    fns = {name: stepper_fn(arm) for name, arm in arms.items()}
+    for _ in range(5):
+        for name in ("plain", "reciprocal"):
+            arms[name]["ms"].append(timed(fns[name], args.steps, args.warmup))
+    med = {name: float(np.median(arm["ms"])) for name, arm in arms.items()}
+    gpu = torch.cuda.get_device_properties(dev).name
+    return {"workload": f"DistMult reciprocal relations 1vsAll+KL d=128 E={E} R={R} (2R={2 * R} relation rows) B={B} "
+                        f"triples ({2 * B} query rows) {args.math}, captured step with the batch built on the device; "
+                        "plain DistMult in the same process, alternating rounds",
+            "metric": "training triples/s", "value": B / (med["reciprocal"] * 1e-3), "ms_per_step": med["reciprocal"],
+            "ms_per_step_plain": med["plain"], "ratio_reciprocal_over_plain": med["reciprocal"] / med["plain"],
+            "ms_rounds": {name: arm["ms"] for name, arm in arms.items()},
+            "flash_fallbacks": {name: arm["st"].flash_fallbacks for name, arm in arms.items()},
+            "loss": {name: arm["st"].loss.item() for name, arm in arms.items()}, "gpu": gpu}
 
 
 def wnrr_rotate_ns(args):
@@ -232,6 +281,8 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", int(os.environ["LOCAL_RANK"])))
     if args.workload == "wd5m-1vsall":
         res = wd5m_1vsall(args)
+    elif args.workload == "wd5m-1vsall-reciprocal":
+        res = wd5m_1vsall_reciprocal(args)
     elif args.workload == "wnrr-rotate-ns":
         res = wnrr_rotate_ns(args)
     elif args.workload == "wd5m-eval-transe":

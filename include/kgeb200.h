@@ -237,6 +237,11 @@ int kgeb_zero_if(const int32_t* flag, float* buf, int64_t numel, void* stream);
  * the LAST non-empty query type survives): rows_loss[B] from kgeb_loss_from_rowstat, row_type[B] (0 = sp_, 1 = _po);
  * out[0] = sum of all rows (the cost that was back-propagated), out[1] = sum over the rows of the highest type present. */
 int kgeb_loss_report(const float* rows_loss, const int32_t* row_type, int64_t B, float* out, void* stream);
+/* Same for a reciprocal relations model whose _po rows were rewritten to sp_ rows on relation p + R (the *_inv batch
+ * builders): a row counts as _po when row_type != 0 or p_idx[row] >= inv_rel_offset (> 0).  inv_rel_offset = 0 (p_idx
+ * may be NULL) is kgeb_loss_report. */
+int kgeb_loss_report_inv(const float* rows_loss, const int32_t* row_type, const int64_t* p_idx, int64_t inv_rel_offset,
+                         int64_t B, float* out, void* stream);
 /* fp32 -> bf16 (round to nearest even) mirror of a table / query matrix for KGEB_MATH_BF16 */
 int kgeb_to_bf16(const float* src, void* dst, int64_t numel, void* stream);
 int64_t kgeb_fused_workspace_bytes(int64_t B, int d, int64_t num_shard_entities, int64_t nnz);
@@ -332,6 +337,14 @@ int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po
                             int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
                             int32_t* p_perm, int32_t* lab_perm, int32_t* overflow, void* workspace,
                             int64_t workspace_bytes, void* stream);
+/* Reciprocal relations model (relation table of 2 R rows, reciprocal_relations_model.py:70-83): with inv_rel_offset = R > 0
+ * every po-query (p, o) is written as the sp-query (o, p + R) -- a_idx = o, p_idx = p + R, row_combine = KGEB_SP_ -- with
+ * the same labels, and p_perm is the stable argsort of the shifted ids.  inv_rel_offset = 0 is kgeb_kvsall_batch_build. */
+int kgeb_kvsall_batch_build_inv(const kgeb_index_t* sp_index, const kgeb_index_t* po_index, const int64_t* example_ids,
+                                int64_t B, int64_t capacity, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
+                                int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
+                                int32_t* p_perm, int32_t* lab_perm, int32_t* overflow, void* workspace,
+                                int64_t workspace_bytes, int64_t inv_rel_offset, void* stream);
 
 /* The 1vsAll batch (train.py:1032-1062: an sp_ pass with label o and a _po pass with label s over the same triples) from
  * the [B, 3] int64 triples: the same eight arrays as kgeb_kvsall_batch_build, 2 B rows (sp_ rows first), one label per
@@ -340,6 +353,11 @@ int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po
 int kgeb_onevsall_batch_build(const int64_t* triples, int64_t B, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
                               int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
                               int32_t* p_perm, int32_t* lab_perm, void* stream);
+/* Same with inv_rel_offset = R > 0: rows B..2B-1 are the sp_ queries (o, p + R) of a reciprocal relations model (label s,
+ * row_combine = KGEB_SP_), p_perm sorts the shifted ids.  inv_rel_offset = 0 is kgeb_onevsall_batch_build. */
+int kgeb_onevsall_batch_build_inv(const int64_t* triples, int64_t B, int64_t num_entities, int64_t num_relations,
+                                  int64_t* a_idx, int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col,
+                                  int32_t* a_perm, int32_t* p_perm, int32_t* lab_perm, int64_t inv_rel_offset, void* stream);
 
 /* ---- 8f-2: on-device negative sampling (kge/util/sampler.py).  Philox4x32-10, counter-based: results depend only on
  * state = {seed, offset} (device memory, so CUDA-graph replays draw fresh numbers; kgeb_philox_advance bumps the offset

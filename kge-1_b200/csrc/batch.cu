@@ -74,8 +74,10 @@ filter_fill_kernel(IndexSet set, int64_t B, const int64_t* __restrict__ src_row,
 
 // KvsAll training batch: example id < n_sp is the sp-query with key row id of the sp index, the others are po-queries
 // (train.py:611-640: queries = the key pair, labels = the values of that key).
+// inv_rel_offset = R > 0 (reciprocal relations model, reciprocal_relations_model.py:70-83): a po-query (p, o) becomes the
+// sp-query (o, p + R) with the same labels.
 __global__ void kvsall_count_kernel(kgeb_index_t sp, kgeb_index_t po, const int64_t* __restrict__ ids, int64_t B,
-                                    int64_t* __restrict__ a_idx, int64_t* __restrict__ p_idx,
+                                    int64_t inv_rel_offset, int64_t* __restrict__ a_idx, int64_t* __restrict__ p_idx,
                                     int32_t* __restrict__ row_combine, int64_t* __restrict__ len) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (i >= B) return;
@@ -85,8 +87,8 @@ __global__ void kvsall_count_kernel(kgeb_index_t sp, kgeb_index_t po, const int6
   const int64_t r = is_sp ? id : id - sp.num_keys;
   // sp key = (s, p): entity first; po key = (p, o): entity second
   a_idx[i] = is_sp ? ix.keys[2 * r] : ix.keys[2 * r + 1];
-  p_idx[i] = is_sp ? ix.keys[2 * r + 1] : ix.keys[2 * r];
-  row_combine[i] = is_sp ? KGEB_SP_ : KGEB__PO;
+  p_idx[i] = is_sp ? ix.keys[2 * r + 1] : ix.keys[2 * r] + inv_rel_offset;
+  row_combine[i] = (is_sp || inv_rel_offset > 0) ? KGEB_SP_ : KGEB__PO;
   len[i] = ix.offsets[r + 1] - ix.offsets[r];
 }
 
@@ -139,12 +141,14 @@ static size_t build_cub_bytes(int64_t n) {
 // ------------------------------------------------------------------------------------------
 // 1vsAll batch (train.py:1032-1062) straight from the [B, 3] triples: the static inputs of the captured step and the
 // three stable argsorts, one block, no host work.  Rows 0..B-1 are the sp_ queries (label = o), rows B..2B-1 the _po
-// queries (label = s); every row has exactly one label.
+// queries (label = s); every row has exactly one label.  inv_rel_offset = R > 0: rows B..2B-1 are the sp_ queries (o, p + R)
+// of a reciprocal relations model instead (label = s).
 // ------------------------------------------------------------------------------------------
 constexpr int kOvaThreads = 1024, kOvaItems = 8, kOvaMax = kOvaThreads * kOvaItems;   // 2 B <= 8192
 
 __global__ void __launch_bounds__(kOvaThreads, 1)
-onevsall_build_kernel(const int64_t* __restrict__ triples, int B, int64_t* __restrict__ a_idx, int64_t* __restrict__ p_idx,
+onevsall_build_kernel(const int64_t* __restrict__ triples, int B, int64_t inv_rel_offset, int64_t* __restrict__ a_idx,
+                      int64_t* __restrict__ p_idx,
                       int32_t* __restrict__ row_combine, int64_t* __restrict__ lab_off, int64_t* __restrict__ lab_col,
                       int32_t* __restrict__ a_perm, int32_t* __restrict__ p_perm, int32_t* __restrict__ lab_perm) {
   using Sort = cub::BlockRadixSort<unsigned, kOvaThreads, kOvaItems, int>;
@@ -154,9 +158,9 @@ onevsall_build_kernel(const int64_t* __restrict__ triples, int B, int64_t* __res
     const int r = i < B ? i : i - B;
     const int64_t s = triples[3 * r], p = triples[3 * r + 1], o = triples[3 * r + 2];
     a_idx[i] = i < B ? s : o;
-    p_idx[i] = p;
+    p_idx[i] = i < B ? p : p + inv_rel_offset;
     lab_col[i] = i < B ? o : s;
-    row_combine[i] = i < B ? 0 : 1;
+    row_combine[i] = (i < B || inv_rel_offset > 0) ? 0 : 1;
     lab_off[i] = i;
   }
   if (t == 0) lab_off[n] = n;
@@ -172,6 +176,7 @@ onevsall_build_kernel(const int64_t* __restrict__ triples, int B, int64_t* __res
         const int r = i < B ? i : i - B;
         const int col = which == 1 ? 1 : ((which == 0) == (i < B) ? 0 : 2);   // a: s | o ;  p: p | p ;  labels: o | s
         k = (unsigned)triples[3 * r + col];
+        if (which == 1 && i >= B) k += (unsigned)inv_rel_offset;
       }
       key[j] = k;
       val[j] = i;
@@ -237,7 +242,7 @@ int kgeb_kvsall_batch_count(const kgeb_index_t* sp_index, const kgeb_index_t* po
                "kvsall_batch_count: bad arguments");
   KGEB_REQUIRE(index_ok(*sp_index) && index_ok(*po_index), "kvsall_batch_count: index has NULL arrays");
   if (B == 0) return KGEB_OK;
-  kvsall_count_kernel<<<(unsigned)((B + 127) / 128), 128, 0, as_stream(stream)>>>(*sp_index, *po_index, example_ids, B,
+  kvsall_count_kernel<<<(unsigned)((B + 127) / 128), 128, 0, as_stream(stream)>>>(*sp_index, *po_index, example_ids, B, 0,
                                                                                  a_idx, p_idx, row_combine, len);
   KGEB_LAUNCH_CHECK("kvsall_count");
   return KGEB_OK;
@@ -260,11 +265,11 @@ int64_t kgeb_kvsall_build_workspace_bytes(int64_t B, int64_t capacity) {
   return (int64_t)(up256((size_t)n * 8) + up256((size_t)n * 4) + up256(build_cub_bytes(n)) + 1024);
 }
 
-int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po_index, const int64_t* example_ids,
-                            int64_t B, int64_t capacity, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
-                            int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
-                            int32_t* p_perm, int32_t* lab_perm, int32_t* overflow, void* workspace,
-                            int64_t workspace_bytes, void* stream) {
+int kgeb_kvsall_batch_build_inv(const kgeb_index_t* sp_index, const kgeb_index_t* po_index, const int64_t* example_ids,
+                                int64_t B, int64_t capacity, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
+                                int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
+                                int32_t* p_perm, int32_t* lab_perm, int32_t* overflow, void* workspace,
+                                int64_t workspace_bytes, int64_t inv_rel_offset, void* stream) {
   KGEB_REQUIRE(sp_index && po_index && example_ids && a_idx && p_idx && row_combine && lab_off && lab_col && a_perm &&
                    p_perm && lab_perm && overflow && workspace,
                "kvsall_batch_build: NULL argument");
@@ -272,6 +277,7 @@ int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po
                "kvsall_batch_build: batch size / label capacity out of range");
   KGEB_REQUIRE(index_ok(*sp_index) && index_ok(*po_index), "kvsall_batch_build: index has NULL arrays");
   KGEB_REQUIRE(workspace_bytes >= kgeb_kvsall_build_workspace_bytes(B, capacity), "kvsall_batch_build: workspace too small");
+  KGEB_REQUIRE(inv_rel_offset >= 0, "kvsall_batch_build: negative inverse relation offset");
   cudaStream_t st = as_stream(stream);
   const int64_t n = (B > capacity ? B : capacity) + 1;
   char* wp = reinterpret_cast<char*>(workspace);
@@ -282,8 +288,8 @@ int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po
   w.cub_bytes = build_cub_bytes(n);
   cudaError_t e;
   iota_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(w.iota, n, lab_off);
-  kvsall_count_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(*sp_index, *po_index, example_ids, B, a_idx, p_idx,
-                                                                  row_combine, lab_off + 1);
+  kvsall_count_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(*sp_index, *po_index, example_ids, B, inv_rel_offset,
+                                                                  a_idx, p_idx, row_combine, lab_off + 1);
   KGEB_LAUNCH_CHECK("kvsall_count");
   size_t bytes = w.cub_bytes;
   e = cub::DeviceScan::InclusiveSum(w.cub_tmp, bytes, lab_off + 1, lab_off + 1, (int)B, st);
@@ -295,7 +301,7 @@ int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po
                                                              lab_col, overflow);
   KGEB_LAUNCH_CHECK("kvsall_fill");
   // the three stable argsorts (ids of the batch are known here, so the step's scatters need no sort)
-  const int eb = bits_needed(num_entities), rb = bits_needed(num_relations);
+  const int eb = bits_needed(num_entities), rb = bits_needed(num_relations + inv_rel_offset);
   bytes = w.cub_bytes;
   e = cub::DeviceRadixSort::SortPairs(w.cub_tmp, bytes, (const int64_t*)a_idx, w.keys_tmp, (const int32_t*)w.iota, a_perm,
                                       (int)B, 0, eb, st);
@@ -311,19 +317,38 @@ int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po
   return KGEB_OK;
 }
 
-int kgeb_onevsall_batch_build(const int64_t* triples, int64_t B, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
-                              int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
-                              int32_t* p_perm, int32_t* lab_perm, void* stream) {
+int kgeb_kvsall_batch_build(const kgeb_index_t* sp_index, const kgeb_index_t* po_index, const int64_t* example_ids,
+                            int64_t B, int64_t capacity, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
+                            int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
+                            int32_t* p_perm, int32_t* lab_perm, int32_t* overflow, void* workspace,
+                            int64_t workspace_bytes, void* stream) {
+  return kgeb_kvsall_batch_build_inv(sp_index, po_index, example_ids, B, capacity, num_entities, num_relations, a_idx, p_idx,
+                                     row_combine, lab_off, lab_col, a_perm, p_perm, lab_perm, overflow, workspace,
+                                     workspace_bytes, 0, stream);
+}
+
+int kgeb_onevsall_batch_build_inv(const int64_t* triples, int64_t B, int64_t num_entities, int64_t num_relations,
+                                  int64_t* a_idx, int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col,
+                                  int32_t* a_perm, int32_t* p_perm, int32_t* lab_perm, int64_t inv_rel_offset, void* stream) {
   KGEB_REQUIRE(triples && a_idx && p_idx && row_combine && lab_off && lab_col && a_perm && p_perm && lab_perm,
                "onevsall_batch_build: NULL buffer");
   KGEB_REQUIRE(B >= 1 && 2 * B <= kgeb::kOvaMax, "onevsall_batch_build: 1 <= batch <= %d (got %lld)", kgeb::kOvaMax / 2,
                (long long)B);
-  KGEB_REQUIRE(num_entities < ((int64_t)1 << 32) - 1 && num_relations < ((int64_t)1 << 32) - 1,
+  KGEB_REQUIRE(inv_rel_offset >= 0, "onevsall_batch_build: negative inverse relation offset");
+  KGEB_REQUIRE(num_entities < ((int64_t)1 << 32) - 1 && num_relations + inv_rel_offset < ((int64_t)1 << 32) - 1,
                "onevsall_batch_build: ids must fit 32 bits");
-  kgeb::onevsall_build_kernel<<<1, kgeb::kOvaThreads, 0, as_stream(stream)>>>(triples, (int)B, a_idx, p_idx, row_combine,
-                                                                             lab_off, lab_col, a_perm, p_perm, lab_perm);
+  kgeb::onevsall_build_kernel<<<1, kgeb::kOvaThreads, 0, as_stream(stream)>>>(triples, (int)B, inv_rel_offset, a_idx, p_idx,
+                                                                             row_combine, lab_off, lab_col, a_perm, p_perm,
+                                                                             lab_perm);
   KGEB_LAUNCH_CHECK("onevsall_batch_build");
   return KGEB_OK;
+}
+
+int kgeb_onevsall_batch_build(const int64_t* triples, int64_t B, int64_t num_entities, int64_t num_relations, int64_t* a_idx,
+                              int64_t* p_idx, int32_t* row_combine, int64_t* lab_off, int64_t* lab_col, int32_t* a_perm,
+                              int32_t* p_perm, int32_t* lab_perm, void* stream) {
+  return kgeb_onevsall_batch_build_inv(triples, B, num_entities, num_relations, a_idx, p_idx, row_combine, lab_off, lab_col,
+                                       a_perm, p_perm, lab_perm, 0, stream);
 }
 
 }  // extern "C"

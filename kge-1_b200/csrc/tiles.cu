@@ -1085,16 +1085,17 @@ int kgeb_loss_from_rowstat(int loss, const float* rowstat, const int64_t* lab_of
 
 // train.py:747 overwrites the reported avg_loss once per query type: what the job logs for a batch is the value of the
 // LAST non-empty query type (sp_ = 0, _po = 1).  out[0] = sum of all rows, out[1] = sum of the rows of the highest type
-// present; one block, fixed order.
+// present; one block, fixed order.  inv_rel_offset = R > 0: a row with relation id p_idx >= R is a _po query of a
+// reciprocal relations model, rewritten to an sp_ query on p + R.
 __global__ void __launch_bounds__(1024)
-loss_report_kernel(const float* __restrict__ rows_loss, const int32_t* __restrict__ row_type, int64_t B,
-                   float* __restrict__ out) {
+loss_report_kernel(const float* __restrict__ rows_loss, const int32_t* __restrict__ row_type,
+                   const int64_t* __restrict__ p_idx, int64_t inv_rel_offset, int64_t B, float* __restrict__ out) {
   __shared__ float red[3][1024];
   float all = 0.f, t1 = 0.f, any1 = 0.f;
   for (int64_t r = threadIdx.x; r < B; r += blockDim.x) {
     const float v = rows_loss[r];
     all += v;
-    if (row_type[r] != 0) { t1 += v; any1 = 1.f; }
+    if (row_type[r] != 0 || (inv_rel_offset > 0 && p_idx[r] >= inv_rel_offset)) { t1 += v; any1 = 1.f; }
   }
   red[0][threadIdx.x] = all; red[1][threadIdx.x] = t1; red[2][threadIdx.x] = any1;
   __syncthreads();
@@ -1112,11 +1113,17 @@ loss_report_kernel(const float* __restrict__ rows_loss, const int32_t* __restric
   }
 }
 
-int kgeb_loss_report(const float* rows_loss, const int32_t* row_type, int64_t B, float* out, void* stream) {
+int kgeb_loss_report_inv(const float* rows_loss, const int32_t* row_type, const int64_t* p_idx, int64_t inv_rel_offset,
+                         int64_t B, float* out, void* stream) {
   KGEB_REQUIRE(rows_loss && row_type && out && B >= 0, "loss_report: bad arguments");
-  loss_report_kernel<<<1, 1024, 0, as_stream(stream)>>>(rows_loss, row_type, B, out);
+  KGEB_REQUIRE(inv_rel_offset >= 0 && (inv_rel_offset == 0 || p_idx), "loss_report: inverse relation offset without ids");
+  loss_report_kernel<<<1, 1024, 0, as_stream(stream)>>>(rows_loss, row_type, p_idx, inv_rel_offset, B, out);
   KGEB_LAUNCH_CHECK("loss_report");
   return KGEB_OK;
+}
+
+int kgeb_loss_report(const float* rows_loss, const int32_t* row_type, int64_t B, float* out, void* stream) {
+  return kgeb_loss_report_inv(rows_loss, row_type, nullptr, 0, B, out, stream);
 }
 
 int kgeb_to_bf16(const float* src, void* dst, int64_t numel, void* stream) {

@@ -152,8 +152,13 @@ class TrainingJobKvsAll(TrainingJob):
             raise NotImplementedError("per-batch renormalisation (normalize_p) is served by the autograd path only")
         self.stepper = FusedAllEntityStepper(self.model, self.optimizer, batch_size, nnz_max, self.loss.kind,
                                              batch_size, self.loss.offset, self.label_smoothing, self.math_mode,
-                                             use_graph, self.shard, dp_group, dp_p2p)
+                                             use_graph, self.shard, dp_group, dp_p2p,
+                                             reciprocal=isinstance(self.model, ReciprocalRelationsModel))
         return self.stepper
+
+    def _inv_rel(self) -> int:
+        """R for a reciprocal relations model (its _po queries become sp_ rows on relation p + R), else 0."""
+        return self.model.num_relations if isinstance(self.model, ReciprocalRelationsModel) else 0
 
     # -- on-device batch construction (SURVEY.md 8f-1): the host sends example ids only ----------------------------
     def enable_device_collate(self, sp_index: KvsAllIndex, po_index: KvsAllIndex):
@@ -194,11 +199,11 @@ class TrainingJobKvsAll(TrainingJob):
     def _build_batch(self, slot: int):
         dc, st = self._dc, self.stepper
         v = st.input_views(dc["staging"][slot])
-        lib.call("kgeb_kvsall_batch_build", dc["descs"][0], dc["descs"][1], dc["ids"][slot].data_ptr(), st.rows,
+        lib.call("kgeb_kvsall_batch_build_inv", dc["descs"][0], dc["descs"][1], dc["ids"][slot].data_ptr(), st.rows,
                  max(st.nnz_max, 1), self.num_entities, self.num_relations, v["a_idx"].data_ptr(), v["p_idx"].data_ptr(),
                  v["row_combine"].data_ptr(), v["lab_off"].data_ptr(), v["lab_col"].data_ptr(), v["a_perm"].data_ptr(),
                  v["p_perm"].data_ptr(), v["lab_perm"].data_ptr(), dc["overflow"][slot].data_ptr(),
-                 dc["ws"].data_ptr(), dc["ws"].numel(), torch.cuda.current_stream().cuda_stream)
+                 dc["ws"].data_ptr(), dc["ws"].numel(), self._inv_rel(), torch.cuda.current_stream().cuda_stream)
 
     def prefetch_ids(self, example_ids: torch.Tensor):
         """Enqueues the construction of the batch with these example ids (host pinned or device int64 [batch_size])."""
@@ -239,7 +244,7 @@ class TrainingJobKvsAll(TrainingJob):
         q = batch["queries"].to(self.device, non_blocking=True)
         qt = batch["query_type_indexes"].to(self.device, non_blocking=True)
         coords = batch["label_coords"].to(self.device, non_blocking=True)
-        a, p, rc = kvsall_rows(q, qt)
+        a, p, rc = kvsall_rows(q, qt, self._inv_rel())
         lab_off, lab_col = fused.csr_from_coords(coords, len(q))
         return a, p, rc, lab_off, lab_col, self.stepper.batch_perms(a, p, lab_col)
 
@@ -248,7 +253,7 @@ class TrainingJobKvsAll(TrainingJob):
         tensors): query rows, per-row combine flags and the label CSR laid out in one pinned buffer."""
         from .trainer import kvsall_rows
         q, qt = batch["queries"], batch["query_type_indexes"]
-        a, p, rc = kvsall_rows(q, qt)
+        a, p, rc = kvsall_rows(q, qt, self._inv_rel())
         lab_off, lab_col = fused.csr_from_coords(batch["label_coords"], len(q))
         return {"packed": self.stepper.pack_host_batch(a, p, rc, lab_off, lab_col), "size": len(q)}
 
@@ -377,7 +382,8 @@ class TrainingJobNegativeSampling(TrainingJob):
         from .trainer import FusedNegSamplingStepper
         self.stepper = FusedNegSamplingStepper(self.model, self.optimizer, batch_size, num_neg_s, num_neg_o,
                                                self.loss.kind, self.loss.offset, use_graph, dp_group, segment_bwd,
-                                               fused_slot, deterministic)
+                                               fused_slot, deterministic,
+                                               reciprocal=isinstance(self.model, ReciprocalRelationsModel))
         return self.stepper
 
     def enable_device_sampling(self, sampler):

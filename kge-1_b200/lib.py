@@ -51,11 +51,13 @@ SIGNATURES = {
     "kgeb_fused_bwd_update": [_i, _p, _l, _i, _p, _l, _l, _l, _p, _f, _f, _p, _f, _p, _p, _p, _f, _f, _p, _p, _p, _p, _l, _p],
     "kgeb_touched_update": [_p, _p, _p, _p, _p, _p, _l, _p, _p, _i, _f, _f, _p, _p],
     "kgeb_onevsall_batch_build": [_p, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p],
+    "kgeb_onevsall_batch_build_inv": [_p, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p],
     "kgeb_fused_bwd_wait_tiles": [_p],
     "kgeb_to_bf16": [_p, _p, _l, _p],
     "kgeb_loss_from_rowstat": [_i, _p, _p, _l, _f, _l, _f, _p, _p, _p, _p],
     "kgeb_zero_if": [_p, _p, _l, _p],
     "kgeb_loss_report": [_p, _p, _l, _p, _p],
+    "kgeb_loss_report_inv": [_p, _p, _p, _l, _l, _p, _p],
     "kgeb_rank_count": [_i, _i, _p, _l, _i, _p, _l, _l, _p, _p, _i, _p, _p, _p, _p, _p, _p],
     "kgeb_scatter_add_rows": [_p, _i, _p, _l, _i, _p, _l, _p, _l, _p],
     "kgeb_scatter_add_rows_perm": [_p, _i, _p, _p, _l, _i, _p, _l, _p, _l, _p],
@@ -69,6 +71,7 @@ SIGNATURES = {
     "kgeb_kvsall_batch_count": [_p, _p, _p, _l, _p, _p, _p, _p, _p],
     "kgeb_kvsall_batch_fill": [_p, _p, _p, _l, _p, _l, _p, _p, _p],
     "kgeb_kvsall_batch_build": [_p, _p, _p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p],
+    "kgeb_kvsall_batch_build_inv": [_p, _p, _p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _l, _p],
     "kgeb_philox_words": [_u, _u, _u, _l, _p, _p],
     "kgeb_philox_advance": [_p, _u, _p],
     "kgeb_sample_uniform": [_p, _l, _l, _p, _p],

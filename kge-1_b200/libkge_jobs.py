@@ -134,12 +134,17 @@ class _EmbedderView:
 
 
 class _ModelView:
-    """A reference KgeModel (plug-in class) as trainer.FusedAllEntityStepper / jobs.EntityRankingJob see a model."""
+    """A reference KgeModel (plug-in class) as trainer.FusedAllEntityStepper / jobs.EntityRankingJob see a model.
+    For the reciprocal relations model (`reciprocal`) the view declares the wrapper (`reciprocal_relations`) and its R =
+    the dataset's relation count; the relation table it exposes is the base model's 2 R-row table."""
 
-    def __init__(self, ref_model, base: str):
+    def __init__(self, ref_model, base: str, reciprocal: bool = False):
         self.ref, self.model = ref_model, base
         self._ent = _EmbedderView(ref_model.get_s_embedder())
         self._rel = _EmbedderView(ref_model.get_p_embedder())
+        self.reciprocal_relations = bool(reciprocal)
+        if reciprocal:
+            self.num_relations = ref_model.dataset.num_relations()
 
     def get_s_embedder(self): return self._ent
     def get_o_embedder(self): return self._ent
@@ -150,10 +155,11 @@ class _ModelView:
 # ---------------------------------------------------------------------------------------------
 # level 2: captured step on the job object
 # ---------------------------------------------------------------------------------------------
-def _install_captured_step(job, model, base: str, loss_kind: int, offset: float, math_mode: int):
+def _install_captured_step(job, model, base: str, loss_kind: int, offset: float, math_mode: int, reciprocal: bool = False):
     from kge.job.train import TrainingJob, TrainingJob1vsAll, TrainingJobKvsAll
     from .trainer import FusedAllEntityStepper, kvsall_rows
-    view = _ModelView(model, base)
+    view = _ModelView(model, base, reciprocal)
+    inv_rel = view.num_relations if reciprocal else 0         # _po queries -> sp_ rows on relation p + R
     dev = view.get_s_embedder().weight.device
     ref_body = type(job)._process_batch            # the reference's own batch body (other batch sizes)
     state = {"stepper": None}
@@ -171,7 +177,7 @@ def _install_captured_step(job, model, base: str, loss_kind: int, offset: float,
         if st is None:
             st = FusedAllEntityStepper(view, job.optimizer, rows, nnz_max, loss_kind, job.batch_size if not is_1vsall else rows // 2,
                                        offset, label_smoothing, math_mode, use_graph=True,
-                                       onevsall_triples=is_1vsall and rows <= 8192)
+                                       onevsall_triples=is_1vsall and rows <= 8192, reciprocal=reciprocal)
             state["stepper"] = st
             model._b200_stepper = st
         return st
@@ -192,7 +198,7 @@ def _install_captured_step(job, model, base: str, loss_kind: int, offset: float,
                 t = triples.to(dev, non_blocking=True)
                 s, p, o = t[:, 0], t[:, 1], t[:, 2]
                 zeros = torch.zeros(b, dtype=torch.int32, device=dev)
-                st.set_inputs(torch.cat((s, o)), torch.cat((p, p)), torch.cat((zeros, zeros + 1)),
+                st.set_inputs(torch.cat((s, o)), torch.cat((p, p + inv_rel)), torch.cat((zeros, zeros + (0 if inv_rel else 1))),
                               torch.arange(2 * b + 1, dtype=torch.int64, device=dev), torch.cat((o, s)))
             size = b
         else:
@@ -206,7 +212,7 @@ def _install_captured_step(job, model, base: str, loss_kind: int, offset: float,
             if st is None:   # label capacity from the first full batch with head room; larger batches take the autograd path
                 st = stepper_for(size, max(2 * nnz, 4 * size))
             qd = q.to(dev, non_blocking=True)
-            a, p, rc = kvsall_rows(qd, batch["query_type_indexes"].to(dev, non_blocking=True))
+            a, p, rc = kvsall_rows(qd, batch["query_type_indexes"].to(dev, non_blocking=True), inv_rel)
             lab_off, lab_col = fused.csr_from_coords(batch["label_coords"].to(dev, non_blocking=True), size)
             st.set_inputs(a, p, rc, lab_off, lab_col)
         prepare = time.time() - t0
@@ -240,8 +246,9 @@ def captured_penalties(model, base_penalty, **kwargs):
     return out
 
 
-def prepare_training_job(job, model, base: str, options: dict):
-    """Called from the plug-in model's prepare_job for training jobs.  Idempotent."""
+def prepare_training_job(job, model, base: str, options: dict, reciprocal: bool = False):
+    """Called from the plug-in model's prepare_job for training jobs (`reciprocal`: from the reciprocal relations model,
+    whose base model's own prepare_job must not install anything).  Idempotent."""
     from kge.job.train import TrainingJob1vsAll, TrainingJobKvsAll
     if getattr(job, "_b200_installed", False):
         return
@@ -261,7 +268,7 @@ def prepare_training_job(job, model, base: str, options: dict):
     model._b200_lazy_jobs = getattr(model, "_b200_lazy_jobs", 0) + 1
     model._b200_math = math_mode
     if options.get("captured_step", False):
-        _install_captured_step(job, model, base, loss_kind, offset, math_mode)
+        _install_captured_step(job, model, base, loss_kind, offset, math_mode, reciprocal)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -357,7 +364,7 @@ def make_entity_ranking_job(RefEntityRankingJob):
             model.eval()
             self.config.log("Evaluating on " + self.eval_split + " data (epoch {})...".format(self.epoch))
             filter_with_test = "test" not in self.filter_splits and self.filter_with_test
-            view = _ModelView(model, model._b200_base)
+            view = _ModelView(model, model._b200_base, getattr(model, "_b200_reciprocal", False))
             scorer = view.get_scorer()
             math_mode = getattr(model, "_b200_eval_math", lib.MATH_FP32)
             filt_idx = [self._b200_indexes(split) for split in self.filter_splits]

@@ -6,6 +6,8 @@ job code (TrainingJob1vsAll / KvsAll / NegativeSampling, EntityRankingJob) runs 
     kgeb200.libkge_plugin.configure(config, "complex")     # config.model = "b200_complex"
     job = Job.create(config, dataset)                      # the reference's own factory
 
+    kgeb200.libkge_plugin.configure_reciprocal(config, "distmult")   # reciprocal_relations_model over b200_distmult
+
 How the reference discovers a model (SURVEY.md 8b): `config.get("model")` -> `<model>.class_name` -> attribute of module
 `kge.model` (kge_model.py:469-487).  `register()` therefore puts the classes on `kge.model`; `configure()` copies the base
 model's option tree to `b200_<base>` (same embedder options, dims, initialisation, penalties) and points `class_name` at
@@ -43,6 +45,7 @@ def register():
     """Defines the plug-in classes against the caller's `kge` package and hangs them on `kge.model`; idempotent."""
     import kge.model as km
     from kge.model.kge_model import KgeModel as RefKgeModel, RelationalScorer as RefScorer
+    from kge.model.reciprocal_relations_model import ReciprocalRelationsModel as RefReciprocal
 
     if getattr(km, "_b200_registered", False):
         return km
@@ -68,6 +71,14 @@ def register():
 
         emb.embed, emb.embed_all = embed, embed_all
         return emb
+
+    def _lazy_scores(self) -> bool:
+        """score_sp / score_po hand out a LazyScores handle only inside a training job whose loss was wrapped by
+        FusedKgeLoss (libkge_jobs.prepare_training_job), in training mode with autograd on, for the DOT scorers,
+        without embedder dropout (lookup_embedder.py:97-100 applies it to the whole table)."""
+        return (getattr(self, "_b200_lazy_jobs", 0) > 0 and self.training and torch.is_grad_enabled()
+                and self._scorer._impl.kind == _lib.DOT and self._entity_embedder.dropout.p == 0
+                and self._relation_embedder.dropout.p == 0)
 
     def make(base):
         class Model(RefKgeModel):
@@ -102,13 +113,7 @@ def register():
                         out[k] = default
                 return out
 
-            def _b200_lazy(self) -> bool:
-                """score_sp / score_po hand out a LazyScores handle only inside a training job whose loss was wrapped by
-                FusedKgeLoss (libkge_jobs.prepare_training_job), in training mode with autograd on, for the DOT scorers,
-                without embedder dropout (lookup_embedder.py:97-100 applies it to the whole table)."""
-                return (getattr(self, "_b200_lazy_jobs", 0) > 0 and self.training and torch.is_grad_enabled()
-                        and self._scorer._impl.kind == _lib.DOT and self._entity_embedder.dropout.p == 0
-                        and self._relation_embedder.dropout.p == 0)
+            _b200_lazy = _lazy_scores
 
             def score_sp(self, s, p, o=None):
                 if o is None and self._b200_lazy():
@@ -135,8 +140,52 @@ def register():
         Model.__name__ = Model.__qualname__ = _class_name(base)
         return Model
 
+    class B200ReciprocalRelationsModel(RefReciprocal):
+        """The reference's reciprocal_relations_model (its constructor, modules, state_dict keys, score_spo / score_sp_po)
+        over a `b200_<base>` base model (configure_reciprocal), with the fused seams of the plug-in: score_sp / score_po
+        hand out LazyScores in training -- score_po as the sp_ query (o, p + R) of reciprocal_relations_model.py:70-83 --,
+        1vsAll / KvsAll jobs get the captured step with `reciprocal=True`, the fused evaluation ranks the _po side as
+        sp_ queries on p + R."""
+
+        def __init__(self, config, dataset, configuration_key=None, init_for_load_only=False):
+            super().__init__(config=config, dataset=dataset, configuration_key=configuration_key,
+                             init_for_load_only=init_for_load_only)
+            base = getattr(self._base_model, "_b200_base", None)
+            if base is None:
+                raise ValueError("B200ReciprocalRelationsModel needs a b200_<base> base model (configure_reciprocal)")
+            self._b200_base = base
+            self._b200_reciprocal = True
+            self._b200_eval_math = self._base_model._b200_eval_math
+
+        _b200_lazy = _lazy_scores
+
+        def score_sp(self, s, p, o=None):
+            if o is None and self._b200_lazy():
+                q = _ops.query_build(self._b200_base, _lib.SP_, self.get_s_embedder().embed(s), self.get_p_embedder().embed(p))
+                return _jobs.LazyScores(_lib.DOT, q, self.get_o_embedder()._embeddings.weight, self._b200_math)
+            return super().score_sp(s, p, o)
+
+        def score_po(self, p, o, s=None):
+            if s is None and self._b200_lazy():
+                p_inv = self.get_p_embedder().embed(p + self.dataset.num_relations())
+                q = _ops.query_build(self._b200_base, _lib.SP_, self.get_o_embedder().embed(o), p_inv)
+                return _jobs.LazyScores(_lib.DOT, q, self.get_s_embedder()._embeddings.weight, self._b200_math)
+            return super().score_po(p, o, s)
+
+        def prepare_job(self, job, **kwargs):
+            """The fused seams are installed for THIS model first: the base model's own installation, reached through the
+            reference's prepare_job, then finds the job prepared and leaves it alone (it would treat _po as _po)."""
+            from kge.job.train import TrainingJob
+            if isinstance(job, TrainingJob):
+                _jobs.prepare_training_job(job, self, self._b200_base, self._base_model._b200_options(), reciprocal=True)
+            super().prepare_job(job, **kwargs)
+
+        def penalty(self, **kwargs):
+            return _jobs.captured_penalties(self, super().penalty, **kwargs)
+
     for base in BASES:
         setattr(km, _class_name(base), make(base))
+    km.B200ReciprocalRelationsModel = B200ReciprocalRelationsModel
     km.B200Scorer = B200Scorer
     km._b200_registered = True
     _jobs.register_jobs()
@@ -160,4 +209,21 @@ def configure(config, base: str, math: str = "fp32", eval_math: str = "fp32", ca
     config.set("model", name)
     if kernel_optimizer and config.get("train.optimizer") in ("Adagrad", "Adam"):
         config.set("train.optimizer", "B200" + config.get("train.optimizer"))     # torch.optim.B200Adagrad / B200Adam
+    return name
+
+
+def configure_reciprocal(config, base: str, math: str = "fp32", eval_math: str = "fp32", captured_step: bool = False,
+                         kernel_optimizer: bool = True) -> str:
+    """Points `config` at the reference's reciprocal relations model over the plug-in model of `base`: configure() builds
+    the `b200_<base>` tree (and rewrites the optimizer); the option tree of `reciprocal_relations_model` is copied to
+    `b200_reciprocal_relations_model` with `base_model.type: b200_<base>` and `class_name` B200ReciprocalRelationsModel, and
+    `model` is set to it.  The `b200.*` options are read from the base model's tree.  Returns the model name."""
+    configure(config, base, math=math, eval_math=eval_math, captured_step=captured_step, kernel_optimizer=kernel_optimizer)
+    name = "b200_reciprocal_relations_model"
+    config._import("reciprocal_relations_model")
+    tree = copy.deepcopy(config.options["reciprocal_relations_model"])
+    tree["class_name"] = "B200ReciprocalRelationsModel"
+    tree["base_model"] = dict(tree.get("base_model") or {}, type=f"b200_{base}")
+    config.options[name] = tree
+    config.set("model", name)
     return name

@@ -43,14 +43,15 @@ def gather_owner_slices(flat: torch.Tensor, group) -> torch.Tensor:
     return flat
 
 
-def _require_plain_model(model: KgeModel, what: str, allow_penalty: bool = False, allow_normalize: bool = False):
+def _require_plain_model(model: KgeModel, what: str, allow_penalty: bool = False, allow_normalize: bool = False,
+                         allow_reciprocal: bool = False):
     """The captured steps read the raw tables at fixed addresses without autograd.  Options whose effect they would
     silently drop raise here instead (the autograd paths of jobs.py serve them): embedder dropout in training
-    (lookup_embedder.py:97-100), the reciprocal-relations wrapper (its _po queries are sp_ queries on relation p + R,
-    reciprocal_relations_model.py:70-83), per-batch renormalisation (replaces the weight tensor, lookup_embedder.py:58-75)
-    and penalty terms (train.py:320-338)."""
+    (lookup_embedder.py:97-100), the reciprocal-relations wrapper unless the stepper was asked to map it (its _po queries
+    are sp_ queries on relation p + R, reciprocal_relations_model.py:70-83; `reciprocal=True`), per-batch renormalisation
+    (replaces the weight tensor, lookup_embedder.py:58-75) and penalty terms (train.py:320-338)."""
     from .model import ReciprocalRelationsModel
-    if isinstance(model, ReciprocalRelationsModel):
+    if isinstance(model, ReciprocalRelationsModel) and not allow_reciprocal:
         raise NotImplementedError(f"{what}: ReciprocalRelationsModel is served by the autograd path (fused_path=True, no "
                                   "captured step)")
     embs = (model.get_s_embedder(), model.get_p_embedder())
@@ -60,6 +61,22 @@ def _require_plain_model(model: KgeModel, what: str, allow_penalty: bool = False
         raise NotImplementedError(f"{what}: per-batch renormalisation (normalize_p) is served by the autograd path only")
     if not allow_penalty and any(e.regularize != "" and e.regularize_weight != 0.0 for e in embs):
         raise NotImplementedError(f"{what}: penalty terms (regularize_weight != 0) are served by the autograd path only")
+
+
+def _inverse_relation_offset(model, reciprocal: bool, what: str) -> int:
+    """R of a reciprocal relations model (relation table of 2 R rows; a _po query (p, o) is the sp_ query (o, p + R)) when
+    the stepper is built with `reciprocal=True`, 0 without it.  A model view of the plug-in (libkge_jobs._ModelView)
+    declares the wrapper with `reciprocal_relations = True`."""
+    if not reciprocal:
+        return 0
+    from .model import ReciprocalRelationsModel
+    if not (isinstance(model, ReciprocalRelationsModel) or getattr(model, "reciprocal_relations", False)):
+        raise ValueError(f"{what}: reciprocal=True needs a reciprocal relations model")
+    r = int(model.num_relations)
+    if model.get_p_embedder().weight.shape[0] != 2 * r:
+        raise ValueError(f"{what}: a reciprocal relations model has 2 * {r} relation rows "
+                         f"(got {model.get_p_embedder().weight.shape[0]})")
+    return r
 
 
 class PeerExchange:
@@ -136,13 +153,18 @@ class FusedAllEntityStepper:
     def __init__(self, model: KgeModel, optimizer, rows: int, nnz_max: int, loss_kind: int, batch_size: int,
                  offset: float = 0.0, label_smoothing: float = 0.0, math_mode: int = lib.MATH_BF16,
                  use_graph: bool = True, shard: Optional[fused.Shard] = None, dp_group=None, dp_p2p: bool = False,
-                 onevsall_triples: bool = False):
+                 onevsall_triples: bool = False, reciprocal: bool = False):
         """`onevsall_triples`: the step starts from a static [rows / 2, 3] int64 buffer of TRIPLES (`set_triples`): its first
         kernel builds the 1vsAll batch -- queries, one label per row, the three scatter permutations -- on the device
-        (kgeb_onevsall_batch_build), so a step costs the host one copy and one graph launch."""
+        (kgeb_onevsall_batch_build), so a step costs the host one copy and one graph launch.
+        `reciprocal`: the model is a reciprocal relations model (2 R relation rows).  Every query of the step is an sp_
+        query: the _po queries of a batch arrive as sp_ rows on relation p + R -- built so by kgeb_onevsall_batch_build_inv
+        (onevsall_triples) or by the caller (`kvsall_rows(..., inv_rel_offset=R)` for set_inputs / pack_host_batch).
+        Kernels, launches and the update are those of the plain step on a 2 R-row relation table."""
         if model.get_scorer().kind != lib.DOT:
             raise NotImplementedError("the fused all-entity step serves the DOT scorers")
-        _require_plain_model(model, "FusedAllEntityStepper", allow_penalty=True)
+        self.inv_rel = _inverse_relation_offset(model, reciprocal, "FusedAllEntityStepper")
+        _require_plain_model(model, "FusedAllEntityStepper", allow_penalty=True, allow_reciprocal=reciprocal)
         self.model, self.opt = model, optimizer
         self.rows, self.nnz_max, self.loss_kind, self.batch_size = rows, nnz_max, loss_kind, batch_size
         self.offset, self.ls, self.math = float(offset), float(label_smoothing), math_mode
@@ -305,9 +327,10 @@ class FusedAllEntityStepper:
         ent, rel = self.ent.detach(), self.rel.detach()
         sh = self.shard
         if self.triples is not None:
-            lib.call("kgeb_onevsall_batch_build", self.triples.data_ptr(), self.rows // 2, self.E, self.rel.shape[0],
-                     self.a_idx.data_ptr(), self.p_idx.data_ptr(), self.row_combine.data_ptr(), self.lab_off.data_ptr(),
-                     self.lab_col.data_ptr(), self.a_perm.data_ptr(), self.p_perm.data_ptr(), self.lab_perm.data_ptr(), st)
+            lib.call("kgeb_onevsall_batch_build_inv", self.triples.data_ptr(), self.rows // 2, self.E,
+                     self.rel.shape[0] - self.inv_rel, self.a_idx.data_ptr(), self.p_idx.data_ptr(),
+                     self.row_combine.data_ptr(), self.lab_off.data_ptr(), self.lab_col.data_ptr(), self.a_perm.data_ptr(),
+                     self.p_perm.data_ptr(), self.lab_perm.data_ptr(), self.inv_rel, st)
         # the gradient buffers are cleared on the third stream, beside the query build (joined where they are first used)
         cur = torch.cuda.current_stream()
         self.side2.wait_stream(cur)
@@ -354,8 +377,8 @@ class FusedAllEntityStepper:
         lib.call("kgeb_loss_from_rowstat", self.loss_kind, self.rowstat.data_ptr(), self.lab_off.data_ptr(), self.rows,
                  self.ls, self.E, 1.0 / self.global_batch, self.loss_rows.data_ptr(), self.lse.data_ptr(),
                  self.loss.data_ptr(), lib.stream_ptr(self.ent))
-        lib.call("kgeb_loss_report", self.loss_rows.data_ptr(), self.row_combine.data_ptr(), self.rows,
-                 self.report.data_ptr(), lib.stream_ptr(self.ent))
+        lib.call("kgeb_loss_report_inv", self.loss_rows.data_ptr(), self.row_combine.data_ptr(), self.p_idx.data_ptr(),
+                 self.inv_rel, self.rows, self.report.data_ptr(), lib.stream_ptr(self.ent))
 
     def _stage_backward(self):
         st = lib.stream_ptr(self.ent)
@@ -792,15 +815,18 @@ class RowShardedAllEntityStepper:
 
     def __init__(self, model: KgeModel, optimizer, rows: int, nnz_max: int, loss_kind: int, batch_size: int,
                  shard: fused.Shard, offset: float = 0.0, label_smoothing: float = 0.0, math_mode: int = lib.MATH_BF16,
-                 use_graph: bool = True, peer_memory: bool = True):
+                 use_graph: bool = True, peer_memory: bool = True, reciprocal: bool = False):
         """`peer_memory`: the three exchanges run as one-shot all-reduce KERNELS over torch symmetric memory
         (kgeb_p2p_allreduce, csrc/p2p.cu) inside ONE CUDA graph with the compute stages; where symmetric memory cannot be
-        set up (or peer_memory=False) they are NCCL all-reduces between four separately captured graphs."""
+        set up (or peer_memory=False) they are NCCL all-reduces between four separately captured graphs.
+        `reciprocal`: as FusedAllEntityStepper -- the batch's _po queries arrive as sp_ rows on relation p + R
+        (`kvsall_rows(..., inv_rel_offset=R)`); the 2 R-row relation table is replicated."""
         if model.get_scorer().kind != lib.DOT:
             raise NotImplementedError("the fused all-entity step serves the DOT scorers")
         if not shard.distributed:
             raise ValueError("RowShardedAllEntityStepper needs a distributed Shard (fused.Shard.of_rank)")
-        _require_plain_model(model, "RowShardedAllEntityStepper")
+        self.inv_rel = _inverse_relation_offset(model, reciprocal, "RowShardedAllEntityStepper")
+        _require_plain_model(model, "RowShardedAllEntityStepper", allow_reciprocal=reciprocal)
         self.model, self.opt, self.shard = model, optimizer, shard
         self.rows, self.nnz_max, self.loss_kind, self.batch_size = rows, nnz_max, loss_kind, batch_size
         self.offset, self.ls, self.math = float(offset), float(label_smoothing), math_mode
@@ -1205,11 +1231,15 @@ class RowShardedAllEntityStepper:
         torch.autograd.graph.increment_version(self.ent)
 
 
-def kvsall_rows(queries: torch.Tensor, query_type: torch.Tensor):
-    """KvsAll batch -> (a_idx, p_idx, row_combine): sp_ rows use (s,p) = (q0,q1); _po rows (p,o) = (q0,q1)."""
+def kvsall_rows(queries: torch.Tensor, query_type: torch.Tensor, inv_rel_offset: int = 0):
+    """KvsAll batch -> (a_idx, p_idx, row_combine): sp_ rows use (s,p) = (q0,q1); _po rows (p,o) = (q0,q1).
+    inv_rel_offset = R > 0 (reciprocal relations model): a _po row (p,o) becomes the sp_ row (o, p + R)."""
     qt = query_type.to(torch.int32)
     a = torch.where(qt == 0, queries[:, 0], queries[:, 1])
     p = torch.where(qt == 0, queries[:, 1], queries[:, 0])
+    if inv_rel_offset > 0:
+        p = torch.where(qt == 0, p, p + inv_rel_offset)
+        qt = torch.zeros_like(qt)
     return a.contiguous(), p.contiguous(), qt.contiguous()
 
 
@@ -1222,15 +1252,19 @@ class FusedNegSamplingStepper:
 
     def __init__(self, model: KgeModel, optimizer, batch_size: int, num_neg_s: int, num_neg_o: int, loss_kind: int,
                  offset: float = 0.0, use_graph: bool = True, dp_group=None, segment_bwd: bool = False,
-                 fused_slot: bool = True, deterministic: bool = True):
+                 fused_slot: bool = True, deterministic: bool = True, reciprocal: bool = False):
         """`segment_bwd`: candidate gradients without materialised rows (csrc/ns_segment.cu: pairs sorted by candidate, one
         warp per distinct candidate) instead of pairs_bwd's dC rows + the sorted scatter; measured slower than the sort it
         replaces (0.509 vs 0.414 ms per C3 step, DESIGN.md section 8): kept as a tuning path.
         `dp_group`: data-parallel replicas (every rank its own batch of `batch_size` triples; SURVEY.md 8e, second row):
         gradients of both tables are exchanged and applied by the peer-memory kernels of csrc/p2p.cu inside the same CUDA
         graph; loss terms are scaled by the global batch so that all replicas apply the identical update
-        (tests/p2p_ns_check.py; profiles/r2/p2p_ns_check_2.log)."""
-        _require_plain_model(model, "FusedNegSamplingStepper")
+        (tests/p2p_ns_check.py; profiles/r2/p2p_ns_check_2.log).
+        `reciprocal`: reciprocal relations model (2 R relation rows): slot S scores the sp_ query (o, p + R) against its
+        subject candidates (ReciprocalRelationsModel.score_spo(..., "s")), its relation gradient rows go to p + R; the
+        shifted ids are computed inside the captured graph."""
+        self.inv_rel = _inverse_relation_offset(model, reciprocal, "FusedNegSamplingStepper")
+        _require_plain_model(model, "FusedNegSamplingStepper", allow_reciprocal=reciprocal)
         # fused_slot: scores, loss, dQ and the candidate gradient of a slot in ONE kernel (kgeb_ns_fused) instead of
         # kgeb_pairs_score + kgeb_ns_loss + kgeb_pairs_bwd -- same sums in the same order, bit-identical results.
         # deterministic=False (opt-in): that kernel adds the candidate gradients straight into the dense gradient with
@@ -1253,6 +1287,7 @@ class FusedNegSamplingStepper:
         i64 = dict(dtype=torch.int64, device=dev)
         B = batch_size
         self.triples = torch.zeros(3, B, **i64)            # static inputs: rows s, p, o
+        self.p_inv = torch.zeros(B, **i64) if self.inv_rel else None       # p + R: relation ids of slot S
         self.neg = {slot: torch.zeros(B, n, **i64) for slot, n in self.N.items() if n > 0}
         self.slots = [slot for slot in (0, 2) if self.N[slot] > 0]
         self.buf = {}
@@ -1291,13 +1326,17 @@ class FusedNegSamplingStepper:
         model_id = lib.MODELS[self.model.model]
         ent, rel = self.ent.detach(), self.rel.detach()
         B, d = self.B, self.d
-        s_idx, p_idx, o_idx = self.triples[0], self.triples[1], self.triples[2]
+        s_idx, p_fwd, o_idx = self.triples[0], self.triples[1], self.triples[2]
         self.g_ent.zero_(); self.g_rel.zero_()
+        if self.inv_rel:
+            torch.add(p_fwd, self.inv_rel, out=self.p_inv)
         for slot in self.slots:
             b = self.buf[slot]
             m = 1 + self.N[slot]
-            # slot O: query (s,p) against object candidates; slot S: query (p,o) against subject candidates
-            combine, a_idx, target = (lib.SP_, s_idx, o_idx) if slot == 2 else (lib._PO, o_idx, s_idx)
+            # slot O: query (s,p) against object candidates; slot S: query (p,o) against subject candidates -- for a
+            # reciprocal model the sp_ query (o, p + R)
+            combine, a_idx, target, p_idx = (lib.SP_, s_idx, o_idx, p_fwd) if slot == 2 else (
+                (lib.SP_, o_idx, s_idx, self.p_inv) if self.inv_rel else (lib._PO, o_idx, s_idx, p_fwd))
             lib.call("kgeb_query_build", model_id, combine, None, ent.data_ptr(), a_idx.data_ptr(), rel.data_ptr(),
                      p_idx.data_ptr(), 1, B, d, b["Q"].data_ptr(), st)
             lib.call("kgeb_ns_candidates", target.data_ptr(), self.neg[slot].data_ptr(), B, self.N[slot],
