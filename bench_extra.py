@@ -5,6 +5,7 @@ profiles/extra_workloads_r1.jsonl and summarised in DESIGN.md.
 
     python bench_extra.py --workload wd5m-1vsall | wnrr-rotate-ns | wd5m-eval-transe | wd5m-eval-complex [--scale F]
     python bench_extra.py --workload wd5m-1vsall-reciprocal --batch 1024
+    python bench_extra.py --workload wd5m-1vsall-lr-schedule --batch 1024
 """
 import argparse
 import json
@@ -155,6 +156,92 @@ def wd5m_1vsall_reciprocal(args):
             "loss": {name: arm["st"].loss.item() for name, arm in arms.items()}, "gpu": gpu}
 
 
+def gpu_info() -> dict:
+    """Card name and power limit of this run (a read-only nvidia-smi query): part of every number measured here."""
+    import subprocess
+    out = {"gpu": torch.cuda.get_device_properties(0).name}
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i",
+                            str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout.strip()
+        out["nvidia_smi"] = q
+    except (OSError, subprocess.SubprocessError):
+        out["nvidia_smi"] = "unavailable"
+    return out
+
+
+def wd5m_1vsall_lr_schedule(args):
+    """The Wikidata5M 1vsAll + KL captured step (DistMult, d=128, batch built on the device) at a constant learning rate
+    and with the rate changed before every step (one 4-byte fill of the rate word per step), in alternating rounds of
+    --steps steps on one stepper; the medians are reported.  Then a one-process A/B of the table-gradient + Adagrad
+    kernel alone: kgeb_fused_bwd_update (rate by value) against kgeb_fused_bwd_update_sched (rate read from a device word)
+    on the same inputs, alternating rounds of --steps launches each."""
+    E, R, d, B = int(4_600_000 * args.scale), 822, 128, args.batch
+    dev = torch.device("cuda")
+    torch.manual_seed(0)
+    model = kb.KgeModel("distmult", E, R, d).to(dev)
+    opt = kb.optim.create("Adagrad", model.parameters(), lr=0.2)
+    st = kb.trainer.FusedAllEntityStepper(model, opt, 2 * B, 2 * B, kb.lib.LOSS_KL, B, math_mode=kb.lib.MATH_BF16,
+                                          onevsall_triples=True)
+    gen = torch.Generator(device=dev).manual_seed(1)
+    batches = [torch.stack((torch.randint(0, E, (B,), device=dev, generator=gen),
+                            torch.randint(0, R, (B,), device=dev, generator=gen),
+                            torch.randint(0, E, (B,), device=dev, generator=gen)), 1) for _ in range(8)]
+    state = {"i": 0}
+
+    def step_fn(changing):
+        def step():
+            if changing:        # a new rate every step, as lr_decay or a per-batch scheduler gives
+                opt.param_groups[0]["lr"] = 0.2 / (1.0 + 1e-4 * state["i"])
+            st.set_triples(batches[state["i"] % len(batches)])
+            state["i"] += 1
+            st.step()
+        return step
+
+    ms = {"constant": [], "changing": []}
+    for _ in range(5):
+        for name in ("constant", "changing"):
+            ms[name].append(timed(step_fn(name == "changing"), args.steps, args.warmup))
+    med = {name: float(np.median(v)) for name, v in ms.items()}
+
+    # kernel A/B on the step's shapes: [2B, d] queries against the E-row table, BCE (no log-sum-exp needed), no touched rows
+    lib = kb.lib
+    n = 2 * B
+    q = torch.randn(n, d, device=dev, generator=gen) * 0.05
+    w = model.get_s_embedder().weight.detach()
+    s_ = opt.state[model.get_s_embedder().weight]["sum"]
+    mirror = w.bfloat16()
+    lab_off = torch.arange(n + 1, device=dev)
+    slot_of = torch.full((E,), -1, dtype=torch.int32, device=dev)
+    gbuf = torch.zeros(1, d, device=dev)
+    ws = torch.empty(lib.load().kgeb_fused_workspace_bytes(n, d, E, 0), dtype=torch.uint8, device=dev)
+    word = torch.tensor([1e-6], dtype=torch.float32, device=dev)       # a tiny rate: the table barely moves
+
+    def kernel_fn(sched):
+        rate = word.data_ptr() if sched else 1e-6
+        name = "kgeb_fused_bwd_update_sched" if sched else "kgeb_fused_bwd_update"
+
+        def call():
+            lib.call(name, lib.LOSS_BCE, q.data_ptr(), n, d, w.data_ptr(), 0, E, E, lab_off.data_ptr(), 0.0, 0.0, None,
+                     1.0 / n, None, mirror.data_ptr(), s_.data_ptr(), rate, 1e-10, slot_of.data_ptr(), gbuf.data_ptr(), None,
+                     ws.data_ptr(), ws.numel(), lib.stream_ptr(w))
+        return call
+
+    kms = {"by_value": [], "sched": []}
+    for _ in range(5):
+        for name in ("by_value", "sched"):
+            kms[name].append(timed(kernel_fn(name == "sched"), args.steps, args.warmup))
+    kmed = {name: float(np.median(v)) for name, v in kms.items()}
+    return {"workload": f"DistMult 1vsAll+KL d=128 E={E} B={B} triples ({2 * B} query rows) bf16, captured step with the "
+                        "batch built on the device: constant lr vs lr changed before every step, alternating rounds on one "
+                        "stepper; kernel A/B kgeb_fused_bwd_update vs _sched (BCE, same inputs), alternating rounds",
+            "metric": "ms per step", "value": med["changing"], "ms_per_step_constant_lr": med["constant"],
+            "ms_per_step_changing_lr": med["changing"], "ratio_changing_over_constant": med["changing"] / med["constant"],
+            "ms_rounds": ms, "kernel_ms_by_value": kmed["by_value"], "kernel_ms_sched": kmed["sched"],
+            "kernel_ratio_sched_over_by_value": kmed["sched"] / kmed["by_value"], "kernel_ms_rounds": kms,
+            "flash_fallbacks": st.flash_fallbacks, "loss": st.loss.item(), "lr_words": st.rate.words.tolist(),
+            **gpu_info()}
+
+
 def wnrr_rotate_ns(args):
     """C3: RotatE negative sampling, 256 negatives for s and o, E=40943, R=11, B=512."""
     E, R, d, B, N = 40943, 11, 128, args.batch, 256
@@ -283,6 +370,8 @@ def main():
         res = wd5m_1vsall(args)
     elif args.workload == "wd5m-1vsall-reciprocal":
         res = wd5m_1vsall_reciprocal(args)
+    elif args.workload == "wd5m-1vsall-lr-schedule":
+        res = wd5m_1vsall_lr_schedule(args)
     elif args.workload == "wnrr-rotate-ns":
         res = wnrr_rotate_ns(args)
     elif args.workload == "wd5m-eval-transe":

@@ -159,6 +159,18 @@ int kgeb_fused_bwd_update(int loss, const float* Q, int64_t B, int d, float* tab
 int kgeb_touched_update(float* W, float* state, void* bf16_mirror, int32_t* slot_of, const int64_t* uniq_rows,
                         const int64_t* num_uniq, int64_t capacity /* n_a + n_b */, const float* g_dense, float* g_sparse,
                         int d, float clr, float eps, const int32_t* skip_flag, void* stream);
+/* _sched siblings: the effective learning rate clr = lr / (1 + (step - 1) * lr_decay) of the step is read from the device
+ * word *clr (non-NULL) instead of being passed by value, so that a captured CUDA graph follows a learning-rate schedule
+ * when the caller rewrites the word between replays.  Same kernels as the by-value entries (the word is read once per
+ * thread): a given rate gives the same bits either way. */
+int kgeb_fused_bwd_update_sched(int loss, const float* Q, int64_t B, int d, float* table, int64_t e_lo, int64_t e_hi,
+                                int64_t num_entities, const int64_t* lab_off, float label_smoothing, float offset,
+                                const float* lse, float inv_batch, const float* grad_scale, void* table_bf16, float* state,
+                                const float* clr, float eps, const int32_t* slot_of, float* gbuf, const int32_t* skip_flag,
+                                void* workspace, int64_t workspace_bytes, void* stream);
+int kgeb_touched_update_sched(float* W, float* state, void* bf16_mirror, int32_t* slot_of, const int64_t* uniq_rows,
+                              const int64_t* num_uniq, int64_t capacity, const float* g_dense, float* g_sparse, int d,
+                              const float* clr, float eps, const int32_t* skip_flag, void* stream);
 
 /* ---- K4+K8+K9 fused all-entity training (DOT kinds): scores are never materialised.
  * Labels are a CSR over the batch rows: lab_off[B+1] (int64), lab_col[nnz] (int64, ascending within a
@@ -281,6 +293,9 @@ int kgeb_segment_reduce_rows(const void* idx, int idx64, const float* rows, int6
 int kgeb_adagrad_dense(float* W, float* state, const float* grad, const float* grad2 /* added to grad, or NULL */,
                        int64_t numel, float clr, float eps, float weight_decay,
                        void* bf16_mirror /* updated alongside W, or NULL */, void* stream);
+/* the same with clr read from the device word *clr (see kgeb_fused_bwd_update_sched) */
+int kgeb_adagrad_dense_sched(float* W, float* state, const float* grad, const float* grad2, int64_t numel, const float* clr,
+                             float eps, float weight_decay, void* bf16_mirror, void* stream);
 /* touched-rows-only Adagrad (equals the dense step when untouched rows have zero gradient and wd=0) */
 int kgeb_adagrad_rows(float* W, float* state, const int64_t* row_ids, const float* row_grads,
                       const int64_t* num_rows_dev, int64_t max_rows, int d, float clr, float eps, void* stream);
@@ -396,6 +411,10 @@ int kgeb_lp_penalty_rows(const float* W, int64_t vocab, int dim, const void* ind
 int kgeb_adagrad_dense_lp(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
                           float eps, float weight_decay, int p, float pen_weight, void* bf16_mirror, float* value_out,
                           void* workspace, int64_t workspace_bytes, void* stream);
+/* the same with clr read from the device word *clr (see kgeb_fused_bwd_update_sched) */
+int kgeb_adagrad_dense_lp_sched(float* W, float* state, const float* grad, const float* grad2, int64_t numel,
+                                const float* clr, float eps, float weight_decay, int p, float pen_weight, void* bf16_mirror,
+                                float* value_out, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- 8f-4: rank histograms and metrics on the device (eval.py:138-224, entity_ranking.py:553-577).
  * rank_hist:    hist[ranks[i]] += 1 for every i with mask[i] != 0 (mask NULL = all); *status = 1 on a rank outside
@@ -436,6 +455,12 @@ int kgeb_p2p_exchange(const void* const* peer_pads, const void* const* peer_flat
                       int world, const uint32_t* ctr, uint32_t* timeout_flag, float* W0, float* state0, void* mirror0,
                       int64_t numel0, float* W1, float* state1, int64_t numel1, float* loss_out, float clr, float eps,
                       void* stream);
+/* the same with the rates read from device memory: clr[0] for table 0, clr[1] for table 1 (see
+ * kgeb_fused_bwd_update_sched); every rank must hold the same words */
+int kgeb_p2p_exchange_sched(const void* const* peer_pads, const void* const* peer_flat, const void* const* peer_stage,
+                            int rank, int world, const uint32_t* ctr, uint32_t* timeout_flag, float* W0, float* state0,
+                            void* mirror0, int64_t numel0, float* W1, float* state1, int64_t numel1, float* loss_out,
+                            const float* clr, float eps, void* stream);
 int kgeb_p2p_apply(const void* const* peer_pads, const float* stage, int rank, int world, uint32_t* ctr, uint32_t* ticket,
                    uint32_t* timeout_flag, float* W0, void* mirror0, int64_t numel0, float* W1, int64_t numel1,
                    void* stream);

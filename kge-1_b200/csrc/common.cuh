@@ -66,6 +66,7 @@ struct TableUpdate {
   float* gbuf;              // [slots, d]
   const int* skip;          // optional device word: non-zero = abandon the step, touch nothing
   float clr, eps;
+  const float* clr_dev;     // optional device word: the rate of this step, read in place of clr (_sched entry)
 };
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }

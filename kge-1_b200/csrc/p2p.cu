@@ -108,8 +108,8 @@ constexpr int kUnroll = 4;   // independent float4 groups per thread: remote loa
 //   flat.p[k]  : rank k's [g_table0 | g_table1 | ... | loss] buffer;  stage.p[k] : rank k's [W_table0 | W_table1 ...]
 __global__ void __launch_bounds__(256)
 p2p_exchange_kernel(PeerPtrs pads, PeerPtrs flat, PeerPtrs stage, int rank, int world, const uint32_t* __restrict__ ctr,
-                    uint32_t* timeout_flag, Table t0, Table t1, int64_t loss_off, float* __restrict__ loss_out, float clr,
-                    float eps) {
+                    uint32_t* timeout_flag, Table t0, Table t1, int64_t loss_off, float* __restrict__ loss_out, float clr_val,
+                    float eps, const float* __restrict__ clr_dev) {
   if (!grid_peer_barrier(pads, rank, world, 2u * *ctr + 1u, timeout_flag)) return;   // every rank's gradients are complete
   if (blockIdx.x == 0 && threadIdx.x == 0 && loss_out) {
     float a = 0.f;
@@ -120,6 +120,7 @@ p2p_exchange_kernel(PeerPtrs pads, PeerPtrs flat, PeerPtrs stage, int rank, int 
   for (int ti = 0; ti < 2; ++ti) {
     const Table& tb = ti == 0 ? t0 : t1;
     if (tb.numel == 0) continue;
+    const float clr = clr_dev ? clr_dev[ti] : clr_val;   // _sched entry: one rate word per table
     int64_t lo, hi;
     slice_of(tb.numel, world, rank, lo, hi);
     const int64_t n4 = (hi - lo) / 4;
@@ -249,10 +250,13 @@ using namespace kgeb;
 
 extern "C" {
 
-int kgeb_p2p_exchange(const void* const* peer_pads, const void* const* peer_flat, const void* const* peer_stage, int rank,
-                      int world, const uint32_t* ctr, uint32_t* timeout_flag, float* W0, float* state0, void* mirror0,
-                      int64_t numel0, float* W1, float* state1, int64_t numel1, float* loss_out, float clr, float eps,
-                      void* stream) {
+}  // extern "C"
+
+// kgeb_p2p_exchange and its _sched sibling: one kernel, clr_dev == NULL selects the by-value rate of both tables
+static int p2p_exchange(const void* const* peer_pads, const void* const* peer_flat, const void* const* peer_stage, int rank,
+                        int world, const uint32_t* ctr, uint32_t* timeout_flag, float* W0, float* state0, void* mirror0,
+                        int64_t numel0, float* W1, float* state1, int64_t numel1, float* loss_out, float clr,
+                        const float* clr_dev, float eps, void* stream) {
   KGEB_REQUIRE(peer_pads && peer_flat && peer_stage && ctr && timeout_flag && W0 && state0 && numel0 >= 0 && numel1 >= 0 &&
                    (numel1 == 0 || (W1 && state1)) && world >= 1 && world <= kMaxWorld && rank >= 0 && rank < world,
                "p2p_exchange: bad arguments");
@@ -272,9 +276,28 @@ int kgeb_p2p_exchange(const void* const* peer_pads, const void* const* peer_flat
   int64_t blocks = ((hi - lo) / 4 + 256 * kUnroll - 1) / (256 * kUnroll) + 1;
   const int grid = (int)(blocks > (int64_t)kNumSMs * 4 ? (int64_t)kNumSMs * 4 : blocks);   // all blocks co-resident
   p2p_exchange_kernel<<<grid, 256, 0, as_stream(stream)>>>(pads, flat, stage, rank, world, ctr, timeout_flag, t0, t1,
-                                                          numel0 + numel1, loss_out, clr, eps);
+                                                          numel0 + numel1, loss_out, clr, eps, clr_dev);
   KGEB_LAUNCH_CHECK("p2p_exchange");
   return KGEB_OK;
+}
+
+extern "C" {
+
+int kgeb_p2p_exchange(const void* const* peer_pads, const void* const* peer_flat, const void* const* peer_stage, int rank,
+                      int world, const uint32_t* ctr, uint32_t* timeout_flag, float* W0, float* state0, void* mirror0,
+                      int64_t numel0, float* W1, float* state1, int64_t numel1, float* loss_out, float clr, float eps,
+                      void* stream) {
+  return p2p_exchange(peer_pads, peer_flat, peer_stage, rank, world, ctr, timeout_flag, W0, state0, mirror0, numel0, W1,
+                      state1, numel1, loss_out, clr, nullptr, eps, stream);
+}
+
+int kgeb_p2p_exchange_sched(const void* const* peer_pads, const void* const* peer_flat, const void* const* peer_stage,
+                            int rank, int world, const uint32_t* ctr, uint32_t* timeout_flag, float* W0, float* state0,
+                            void* mirror0, int64_t numel0, float* W1, float* state1, int64_t numel1, float* loss_out,
+                            const float* clr, float eps, void* stream) {
+  KGEB_REQUIRE(clr, "p2p_exchange_sched: the learning-rate words are NULL");
+  return p2p_exchange(peer_pads, peer_flat, peer_stage, rank, world, ctr, timeout_flag, W0, state0, mirror0, numel0, W1,
+                      state1, numel1, loss_out, 0.f, clr, eps, stream);
 }
 
 int kgeb_p2p_allreduce(const void* const* peer_pads, const void* const* peer_bufs, int rank, int world, uint32_t* epoch,

@@ -78,14 +78,17 @@ finish_value_kernel(const float* __restrict__ partial, const int64_t* __restrict
   }
 }
 
-// Adagrad step (torch.optim.Adagrad, lr_decay = 0) with the unweighted Lp penalty folded in:
+// Adagrad step (torch.optim.Adagrad; clr = lr / (1 + (step - 1) * lr_decay) from the caller) with the unweighted Lp penalty
+// folded in:
 //   g = grad (+ grad2) + weight_decay * w + pen_weight * |w|^(p-1) sign(w);  state += g^2;  w -= clr * g / (sqrt(state) + eps)
 // and the block partial sums of |w|^p of the *pre-update* parameters (the penalty value the reference reports).
 __global__ void __launch_bounds__(kPenBlock)
 adagrad_dense_lp_kernel(float* __restrict__ W, float* __restrict__ state, const float* __restrict__ grad,
-                        const float* __restrict__ grad2, int64_t numel, float clr, float eps, float wd, int p,
-                        float pen_weight, __nv_bfloat16* __restrict__ mirror, float* __restrict__ partial) {
+                        const float* __restrict__ grad2, int64_t numel, float clr_val, float eps, float wd, int p,
+                        float pen_weight, __nv_bfloat16* __restrict__ mirror, float* __restrict__ partial,
+                        const float* __restrict__ clr_dev) {
   __shared__ float sh[kPenBlock / 32];
+  const float clr = clr_dev ? *clr_dev : clr_val;   // the rate of this step from device memory (_sched entry)
   float acc = 0.f;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < numel; i += (int64_t)gridDim.x * blockDim.x) {
     const float w = W[i];
@@ -226,9 +229,12 @@ int kgeb_lp_penalty_rows(const float* W, int64_t vocab, int dim, const void* ind
   return KGEB_OK;
 }
 
-int kgeb_adagrad_dense_lp(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
-                          float eps, float weight_decay, int p, float pen_weight, void* bf16_mirror, float* value_out,
-                          void* workspace, int64_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// kgeb_adagrad_dense_lp and its _sched sibling: one kernel, clr_dev == NULL selects the by-value rate
+static int adagrad_dense_lp(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
+                            const float* clr_dev, float eps, float weight_decay, int p, float pen_weight, void* bf16_mirror,
+                            float* value_out, void* workspace, int64_t workspace_bytes, void* stream) {
   KGEB_REQUIRE(W && state && grad && value_out && workspace && numel >= 0, "adagrad_dense_lp: bad arguments");
   KGEB_REQUIRE(p >= 1 && p <= 16, "adagrad_dense_lp: p = %d not in [1, 16]", p);
   const int grid = dense_grid(numel);
@@ -236,11 +242,28 @@ int kgeb_adagrad_dense_lp(float* W, float* state, const float* grad, const float
   float* partial = reinterpret_cast<float*>(workspace);
   adagrad_dense_lp_kernel<<<grid, kPenBlock, 0, as_stream(stream)>>>(W, state, grad, grad2, numel, clr, eps, weight_decay, p,
                                                                     pen_weight, reinterpret_cast<__nv_bfloat16*>(bf16_mirror),
-                                                                    partial);
+                                                                    partial, clr_dev);
   KGEB_LAUNCH_CHECK("adagrad_dense_lp");
   finish_value_kernel<<<1, 256, 0, as_stream(stream)>>>(partial, nullptr, grid, pen_weight / (float)p, value_out);
   KGEB_LAUNCH_CHECK("adagrad_dense_lp finish");
   return KGEB_OK;
+}
+
+extern "C" {
+
+int kgeb_adagrad_dense_lp(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
+                          float eps, float weight_decay, int p, float pen_weight, void* bf16_mirror, float* value_out,
+                          void* workspace, int64_t workspace_bytes, void* stream) {
+  return adagrad_dense_lp(W, state, grad, grad2, numel, clr, nullptr, eps, weight_decay, p, pen_weight, bf16_mirror,
+                          value_out, workspace, workspace_bytes, stream);
+}
+
+int kgeb_adagrad_dense_lp_sched(float* W, float* state, const float* grad, const float* grad2, int64_t numel,
+                                const float* clr, float eps, float weight_decay, int p, float pen_weight, void* bf16_mirror,
+                                float* value_out, void* workspace, int64_t workspace_bytes, void* stream) {
+  KGEB_REQUIRE(clr, "adagrad_dense_lp_sched: the learning-rate word is NULL");
+  return adagrad_dense_lp(W, state, grad, grad2, numel, 0.f, clr, eps, weight_decay, p, pen_weight, bf16_mirror, value_out,
+                          workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -95,6 +95,7 @@ struct Params {
   float* upd_gbuf;         // [slots, d]
   const int* upd_skip;     // non-zero word: the step is being abandoned (failed flash pass) -- touch nothing
   float upd_clr, upd_eps;
+  const float* upd_clr_dev;  // non-NULL: the rate is this device word, not upd_clr (read once per update warp)
   int stagger_clk;         // fused update: CTA b starts b * stagger_clk clocks late (see the producer warp of the v2 kernel)
   int upd_debug;           // tuning only (KGEB_UPD_DEBUG): 1 = no loads of W / state, 2 = no stores, 4 = no arithmetic, 8 = no prefetch, 16 = no phase 2
 };
@@ -643,7 +644,7 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
   const float* kc_s = (!RES_IS_Q && LOSS == KGEB_LOSS_KL && p.colk_n > 0) ? kc_smem : nullptr;
   if (kc_s)
     for (int i = threadIdx.x; i < p.colk_n; i += blockDim.x) kc_smem[i] = p.colk[i];
-  int32_t* slot_s = reinterpret_cast<int32_t*>(kc_smem + p.colk_n_alloc);   // !RES_IS_Q: [EPQ][RES_ROWS] (fused update)
+  int32_t* slot_s = reinterpret_cast<int32_t*>(kc_smem + p.colk_n_alloc);   // !RES_IS_Q: [EPQ][RES_ROWS] (fused update) + rate
   constexpr int TMEM_COLS = 512;
   constexpr uint32_t S_COL = 0;                 // NG S buffers of 64 columns; G aliases the first 32 columns of each
   constexpr uint32_t O_COL = NG * STR_ROWS;     // OUT accumulator: d <= 256 columns behind them
@@ -813,6 +814,12 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
     const int part = warp - (4 + 4 * EPQ);
     const int sub = lane >> 3, ck = lane & 7;   // row within a group of 4, 16-byte chunk of the 128-byte box row
     const bool live = p.upd_skip == nullptr || __ldg(p.upd_skip) == 0;
+    // the rate of this launch (device word of the _sched entry or the by-value parameter), read once at role start and kept
+    // in shared memory behind the slot arrays: held in a register across the loop below it made ptxas spill 20-28 more
+    // bytes in this kernel (-Xptxas -v); read from here the register and spill counts are those of the by-value kernel
+    float* clr_s = reinterpret_cast<float*>(slot_s + EPQ * RES_ROWS);
+    if (lane == 0) *clr_s = p.upd_clr_dev ? __ldg(p.upd_clr_dev) : p.upd_clr;   // (every update warp stores the same value)
+    __syncwarp();
     const int nbox = (p.d + 31) / 32;
     uint8_t* stage = stage_smem + (size_t)part * STAGE_BYTES;
     uint32_t fphase = 0;
@@ -856,11 +863,12 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
               // per element; this warp shares its scheduler with four epilogue warps that already use ~80 % of the issue
               // slots, and with them the update warp fell behind the tile pipeline (kernel 5.7 instead of 4.1 ms).
               float4 w = w8[i], st = s8[i];
+              const float clr = *clr_s;
               st.x = fmaf(g.x, g.x, st.x); st.y = fmaf(g.y, g.y, st.y); st.z = fmaf(g.z, g.z, st.z); st.w = fmaf(g.w, g.w, st.w);
-              w.x = fmaf(-p.upd_clr * g.x, rcp_approx(sqrt_approx(st.x) + p.upd_eps), w.x);
-              w.y = fmaf(-p.upd_clr * g.y, rcp_approx(sqrt_approx(st.y) + p.upd_eps), w.y);
-              w.z = fmaf(-p.upd_clr * g.z, rcp_approx(sqrt_approx(st.z) + p.upd_eps), w.z);
-              w.w = fmaf(-p.upd_clr * g.w, rcp_approx(sqrt_approx(st.w) + p.upd_eps), w.w);
+              w.x = fmaf(-clr * g.x, rcp_approx(sqrt_approx(st.x) + p.upd_eps), w.x);
+              w.y = fmaf(-clr * g.y, rcp_approx(sqrt_approx(st.y) + p.upd_eps), w.y);
+              w.z = fmaf(-clr * g.z, rcp_approx(sqrt_approx(st.z) + p.upd_eps), w.z);
+              w.w = fmaf(-clr * g.w, rcp_approx(sqrt_approx(st.w) + p.upd_eps), w.w);
               if (p.upd_debug & 2) continue;
               const size_t off = base + (size_t)(4 * i) * p.d;
               *reinterpret_cast<float4*>(p.upd_w + off) = w;
@@ -1186,8 +1194,8 @@ static Plan make_plan(bool res_is_q, bool bf16, int64_t B, int d, int64_t n_ent)
   const int64_t colk_n = (!res_is_q && use_v2() && bf16 && B <= 4096) ? ((B + 63) / 64) * 64 : 0;
   p.colk_n = (int)colk_n;
   p.colk_n_alloc = (int)colk_n;
-  // (+ 2 KiB: the touched-row slots of the tile, one copy per column part, for the fused update)
-  const size_t fixed = 1024 + 512 + (size_t)colk_n * 4 + (res_is_q ? 0 : (size_t)EPQ * RES_ROWS * 4);
+  // (+ 2 KiB: the touched-row slots of the tile, one copy per column part, for the fused update; + 16 B: its learning rate)
+  const size_t fixed = 1024 + 512 + (size_t)colk_n * 4 + (res_is_q ? 0 : (size_t)EPQ * RES_ROWS * 4 + 16);
   const size_t g_bytes = (use_v2() && bf16) ? 0 : (size_t)(STR_ROWS / slab_k) * RES_SLAB;   // v2: G lives in tensor memory
   const size_t base = (size_t)p.ks * RES_SLAB + 2 * g_bytes + (res_is_q ? 0 : (size_t)EPQ * STAGE_BYTES);
   int nstr = (int)((SMEM_BUDGET - fixed - base) / ((size_t)p.ks * STR_SLAB));
@@ -1608,7 +1616,7 @@ int tc_fused_bwd(int loss, const float* Q, const void* Qb, int64_t B, int d, con
       if (upd) {
         pl.p.upd_w = upd->w; pl.p.upd_state = upd->state; pl.p.upd_mirror = reinterpret_cast<__nv_bfloat16*>(upd->mirror);
         pl.p.upd_slot = upd->slot_of; pl.p.upd_gbuf = upd->gbuf; pl.p.upd_skip = upd->skip;
-        pl.p.upd_clr = upd->clr; pl.p.upd_eps = upd->eps;
+        pl.p.upd_clr = upd->clr; pl.p.upd_eps = upd->eps; pl.p.upd_clr_dev = upd->clr_dev;
         pl.p.upd_debug = getenv("KGEB_UPD_DEBUG") ? atoi(getenv("KGEB_UPD_DEBUG")) : 0;
         // tuning knob, off by default: spread the CTAs' phases over one job period (KGEB_UPD_STAGGER = clocks per tile, e.g.
         // 1100).  Measured with 0 / 1100 / 2200: no difference -- the CTAs do not run in lockstep -- and the last CTA's

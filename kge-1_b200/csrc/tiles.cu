@@ -887,11 +887,14 @@ int kgeb_fused_label_rows_to(int loss, const float* Q, int64_t B, int d, const f
 // tile kernel's flush: rows with slot_of[row] < 0 are updated in place (W, state, bf16 mirror), the others are parked in
 // gbuf[slot] for kgeb_touched_update.  Replaces, for an [E, d] table, a stored gradient buffer and an update pass over it
 // (2 x E*d*4 bytes of HBM traffic and one launch); reference: train.py:375 optimizer.step() after :323 backward().
-int kgeb_fused_bwd_update(int loss, const float* Q, int64_t B, int d, float* table, int64_t e_lo, int64_t e_hi,
-                          int64_t num_entities, const int64_t* lab_off, float label_smoothing, float offset,
-                          const float* lse, float inv_batch, const float* grad_scale, void* table_bf16, float* state,
-                          float clr, float eps, const int32_t* slot_of, float* gbuf, const int32_t* skip_flag,
-                          void* workspace, int64_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// kgeb_fused_bwd_update and its _sched sibling: one tile kernel, clr_dev == NULL selects the by-value rate
+static int fused_bwd_update(int loss, const float* Q, int64_t B, int d, float* table, int64_t e_lo, int64_t e_hi,
+                            int64_t num_entities, const int64_t* lab_off, float label_smoothing, float offset,
+                            const float* lse, float inv_batch, const float* grad_scale, void* table_bf16, float* state,
+                            float clr, const float* clr_dev, float eps, const int32_t* slot_of, float* gbuf,
+                            const int32_t* skip_flag, void* workspace, int64_t workspace_bytes, void* stream) {
   int rc = check_fused(loss, d, label_smoothing, Q, table, e_lo, e_hi);
   if (rc) return rc;
   KGEB_REQUIRE(tc_bwd_supported(KGEB_MATH_BF16, d), "fused_bwd_update: entity dim must be a multiple of 16 and <= 256 (got %d)", d);
@@ -906,10 +909,33 @@ int kgeb_fused_bwd_update(int loss, const float* Q, int64_t B, int d, float* tab
   label_weight_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(loss, lab_off, B, lp.ls_keep, tail.tscale);
   KGEB_LAUNCH_CHECK("label_weight");
   if ((rc = tc_to_bf16(Q, tail.qb, B * (int64_t)d, st))) return rc;
-  TableUpdate upd{table, state, table_bf16, slot_of, gbuf, skip_flag, clr, eps};
+  TableUpdate upd{table, state, table_bf16, slot_of, gbuf, skip_flag, clr, eps, clr_dev};
   return tc_fused_bwd(loss, Q, tail.qb, B, d, table, table_bf16, e_lo, n_ent, lab_off, lab_off, 0, nullptr, tail.tscale,
                       lp.ls_add, offset, lse, inv_batch, grad_scale, nullptr, nullptr, nullptr, 0, workspace, tail.usable, st,
                       &upd);
+}
+
+extern "C" {
+
+int kgeb_fused_bwd_update(int loss, const float* Q, int64_t B, int d, float* table, int64_t e_lo, int64_t e_hi,
+                          int64_t num_entities, const int64_t* lab_off, float label_smoothing, float offset,
+                          const float* lse, float inv_batch, const float* grad_scale, void* table_bf16, float* state,
+                          float clr, float eps, const int32_t* slot_of, float* gbuf, const int32_t* skip_flag,
+                          void* workspace, int64_t workspace_bytes, void* stream) {
+  return fused_bwd_update(loss, Q, B, d, table, e_lo, e_hi, num_entities, lab_off, label_smoothing, offset, lse, inv_batch,
+                          grad_scale, table_bf16, state, clr, nullptr, eps, slot_of, gbuf, skip_flag, workspace,
+                          workspace_bytes, stream);
+}
+
+int kgeb_fused_bwd_update_sched(int loss, const float* Q, int64_t B, int d, float* table, int64_t e_lo, int64_t e_hi,
+                                int64_t num_entities, const int64_t* lab_off, float label_smoothing, float offset,
+                                const float* lse, float inv_batch, const float* grad_scale, void* table_bf16, float* state,
+                                const float* clr, float eps, const int32_t* slot_of, float* gbuf, const int32_t* skip_flag,
+                                void* workspace, int64_t workspace_bytes, void* stream) {
+  KGEB_REQUIRE(clr, "fused_bwd_update_sched: the learning-rate word is NULL");
+  return fused_bwd_update(loss, Q, B, d, table, e_lo, e_hi, num_entities, lab_off, label_smoothing, offset, lse, inv_batch,
+                          grad_scale, table_bf16, state, 0.f, clr, eps, slot_of, gbuf, skip_flag, workspace, workspace_bytes,
+                          stream);
 }
 
 int kgeb_fused_bwd(int loss, int math, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,

@@ -566,10 +566,11 @@ touched_build_kernel(const int64_t* __restrict__ ids_a, int n_a, const int64_t* 
 __global__ void touched_update_kernel(float* __restrict__ W, float* __restrict__ state, __nv_bfloat16* __restrict__ mirror,
                                       int32_t* __restrict__ slot_of, const int64_t* __restrict__ uniq,
                                       const int64_t* __restrict__ num_uniq, const float* __restrict__ g_dense,
-                                      float* __restrict__ g_sparse, int64_t dummy, int d, float clr, float eps,
-                                      const int* __restrict__ skip) {
+                                      float* __restrict__ g_sparse, int64_t dummy, int d, float clr_val, float eps,
+                                      const int* __restrict__ skip, const float* __restrict__ clr_dev) {
   const int64_t n = *num_uniq;
   const bool live = skip == nullptr || *skip == 0;
+  const float clr = clr_dev ? *clr_dev : clr_val;   // the rate of this step from device memory (_sched entries)
   const int d4 = d / 4;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < (n + 1) * d4; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t slot = i / d4;
@@ -609,8 +610,9 @@ __global__ void touched_update_kernel(float* __restrict__ W, float* __restrict__
 // optimizers
 // ------------------------------------------------------------------------------------------
 __global__ void adagrad_dense_kernel(float* __restrict__ W, float* __restrict__ state, const float* __restrict__ grad,
-                                     const float* __restrict__ grad2, int64_t numel, float clr, float eps, float wd,
-                                     __nv_bfloat16* __restrict__ mirror) {
+                                     const float* __restrict__ grad2, int64_t numel, float clr_val, float eps, float wd,
+                                     __nv_bfloat16* __restrict__ mirror, const float* __restrict__ clr_dev) {
+  const float clr = clr_dev ? *clr_dev : clr_val;   // the rate of this step from device memory (_sched entries)
   int64_t i = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) * 4;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x * 4;
   for (; i + 3 < numel; i += stride) {
@@ -786,9 +788,13 @@ int kgeb_touched_build(const int64_t* ids_a, int64_t n_a, const int64_t* ids_b, 
   return KGEB_OK;
 }
 
-int kgeb_touched_update(float* W, float* state, void* bf16_mirror, int32_t* slot_of, const int64_t* uniq_rows,
-                        const int64_t* num_uniq, int64_t capacity, const float* g_dense, float* g_sparse, int d, float clr,
-                        float eps, const int32_t* skip_flag, void* stream) {
+}  // extern "C"
+
+// The by-value entries and their _sched siblings (rate read from a device word) share one kernel each: clr_dev == NULL
+// selects the by-value rate.
+static int touched_update(float* W, float* state, void* bf16_mirror, int32_t* slot_of, const int64_t* uniq_rows,
+                          const int64_t* num_uniq, int64_t capacity, const float* g_dense, float* g_sparse, int d, float clr,
+                          const float* clr_dev, float eps, const int32_t* skip_flag, void* stream) {
   KGEB_REQUIRE(W && state && slot_of && uniq_rows && num_uniq && g_dense && g_sparse && capacity > 0 && d > 0 && d % 4 == 0,
                "touched_update: bad arguments");
   const int64_t work = (capacity + 1) * (d / 4);
@@ -796,13 +802,13 @@ int kgeb_touched_update(float* W, float* state, void* bf16_mirror, int32_t* slot
   if (blocks > (int64_t)kNumSMs * 8) blocks = (int64_t)kNumSMs * 8;
   kgeb::touched_update_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(
       W, state, reinterpret_cast<__nv_bfloat16*>(bf16_mirror), slot_of, uniq_rows, num_uniq, g_dense, g_sparse, capacity, d,
-      clr, eps, skip_flag);
+      clr, eps, skip_flag, clr_dev);
   KGEB_LAUNCH_CHECK("touched_update");
   return KGEB_OK;
 }
 
-int kgeb_adagrad_dense(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
-                       float eps, float weight_decay, void* bf16_mirror, void* stream) {
+static int adagrad_dense(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
+                         const float* clr_dev, float eps, float weight_decay, void* bf16_mirror, void* stream) {
   KGEB_REQUIRE(W && state && grad && numel >= 0, "adagrad_dense: bad arguments");
   KGEB_REQUIRE(((reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(state) |
                  reinterpret_cast<uintptr_t>(grad) | reinterpret_cast<uintptr_t>(grad2)) & 15) == 0,
@@ -811,9 +817,37 @@ int kgeb_adagrad_dense(float* W, float* state, const float* grad, const float* g
   int64_t blocks = (numel / 4 + 255) / 256 + 1;
   int grid = (int)(blocks > (int64_t)kNumSMs * 8 ? (int64_t)kNumSMs * 8 : blocks);
   adagrad_dense_kernel<<<grid, 256, 0, as_stream(stream)>>>(W, state, grad, grad2, numel, clr, eps, weight_decay,
-                                                            reinterpret_cast<__nv_bfloat16*>(bf16_mirror));
+                                                            reinterpret_cast<__nv_bfloat16*>(bf16_mirror), clr_dev);
   KGEB_LAUNCH_CHECK("adagrad_dense");
   return KGEB_OK;
+}
+
+extern "C" {
+
+int kgeb_touched_update(float* W, float* state, void* bf16_mirror, int32_t* slot_of, const int64_t* uniq_rows,
+                        const int64_t* num_uniq, int64_t capacity, const float* g_dense, float* g_sparse, int d, float clr,
+                        float eps, const int32_t* skip_flag, void* stream) {
+  return touched_update(W, state, bf16_mirror, slot_of, uniq_rows, num_uniq, capacity, g_dense, g_sparse, d, clr, nullptr,
+                        eps, skip_flag, stream);
+}
+
+int kgeb_touched_update_sched(float* W, float* state, void* bf16_mirror, int32_t* slot_of, const int64_t* uniq_rows,
+                              const int64_t* num_uniq, int64_t capacity, const float* g_dense, float* g_sparse, int d,
+                              const float* clr, float eps, const int32_t* skip_flag, void* stream) {
+  KGEB_REQUIRE(clr, "touched_update_sched: the learning-rate word is NULL");
+  return touched_update(W, state, bf16_mirror, slot_of, uniq_rows, num_uniq, capacity, g_dense, g_sparse, d, 0.f, clr, eps,
+                        skip_flag, stream);
+}
+
+int kgeb_adagrad_dense(float* W, float* state, const float* grad, const float* grad2, int64_t numel, float clr,
+                       float eps, float weight_decay, void* bf16_mirror, void* stream) {
+  return adagrad_dense(W, state, grad, grad2, numel, clr, nullptr, eps, weight_decay, bf16_mirror, stream);
+}
+
+int kgeb_adagrad_dense_sched(float* W, float* state, const float* grad, const float* grad2, int64_t numel, const float* clr,
+                             float eps, float weight_decay, void* bf16_mirror, void* stream) {
+  KGEB_REQUIRE(clr, "adagrad_dense_sched: the learning-rate word is NULL");
+  return adagrad_dense(W, state, grad, grad2, numel, 0.f, clr, eps, weight_decay, bf16_mirror, stream);
 }
 
 int kgeb_adagrad_rows(float* W, float* state, const int64_t* row_ids, const float* row_grads,

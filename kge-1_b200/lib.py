@@ -50,6 +50,9 @@ SIGNATURES = {
     "kgeb_touched_build": [_p, _l, _p, _l, _p, _l, _l, _p, _p, _p, _p, _p, _p],
     "kgeb_fused_bwd_update": [_i, _p, _l, _i, _p, _l, _l, _l, _p, _f, _f, _p, _f, _p, _p, _p, _f, _f, _p, _p, _p, _p, _l, _p],
     "kgeb_touched_update": [_p, _p, _p, _p, _p, _p, _l, _p, _p, _i, _f, _f, _p, _p],
+    "kgeb_fused_bwd_update_sched": [_i, _p, _l, _i, _p, _l, _l, _l, _p, _f, _f, _p, _f, _p, _p, _p, _p, _f, _p, _p, _p, _p, _l,
+                                    _p],
+    "kgeb_touched_update_sched": [_p, _p, _p, _p, _p, _p, _l, _p, _p, _i, _p, _f, _p, _p],
     "kgeb_onevsall_batch_build": [_p, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "kgeb_onevsall_batch_build_inv": [_p, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p],
     "kgeb_fused_bwd_wait_tiles": [_p],
@@ -63,6 +66,7 @@ SIGNATURES = {
     "kgeb_scatter_add_rows_perm": [_p, _i, _p, _p, _l, _i, _p, _l, _p, _l, _p],
     "kgeb_segment_reduce_rows": [_p, _i, _p, _l, _i, _p, _p, _p, _p, _l, _p],
     "kgeb_adagrad_dense": [_p, _p, _p, _p, _l, _f, _f, _f, _p, _p],
+    "kgeb_adagrad_dense_sched": [_p, _p, _p, _p, _l, _p, _f, _f, _p, _p],
     "kgeb_adagrad_rows": [_p, _p, _p, _p, _p, _l, _i, _f, _f, _p],
     "kgeb_adam_dense": [_p, _p, _p, _p, _l, _f, _f, _f, _f, _f, _f, _f, _p],
     "kgeb_csr_lookup": [_p, _l, _p, _l, _p, _p],
@@ -80,6 +84,7 @@ SIGNATURES = {
     "kgeb_lp_penalty_dense": [_p, _l, _i, _f, _p, _p, _p, _l, _p],
     "kgeb_lp_penalty_rows": [_p, _l, _i, _p, _i, _l, _i, _f, _p, _p, _p, _l, _p],
     "kgeb_adagrad_dense_lp": [_p, _p, _p, _p, _l, _f, _f, _f, _i, _f, _p, _p, _p, _l, _p],
+    "kgeb_adagrad_dense_lp_sched": [_p, _p, _p, _p, _l, _p, _f, _f, _i, _f, _p, _p, _p, _l, _p],
     "kgeb_rank_hist": [_p, _p, _l, _l, _p, _p, _p],
     "kgeb_isin_sorted": [_p, _i, _l, _p, _l, _p, _p],
     "kgeb_rank_metrics": [_p, _l, _p, _i, _p, _p, _l, _p],
@@ -87,6 +92,7 @@ SIGNATURES = {
     "kgeb_ns_bwd_q": [_i, _p, _p, _p, _l, _l, _i, _p, _p, _p, _p],
     "kgeb_ns_cand_grad": [_i, _p, _p, _p, _l, _l, _i, _p, _p, _l, _p, _p, _l, _p],
     "kgeb_p2p_exchange": [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _l, _p, _p, _l, _p, _f, _f, _p],
+    "kgeb_p2p_exchange_sched": [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _l, _p, _p, _l, _p, _p, _f, _p],
     "kgeb_p2p_allreduce": [_p, _p, _i, _i, _p, _p, _l, _i, _p, _p],
     "kgeb_p2p_apply": [_p, _p, _i, _i, _p, _p, _p, _p, _p, _l, _p, _l, _p],
 }

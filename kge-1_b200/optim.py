@@ -9,6 +9,21 @@ import torch
 from . import lib
 
 
+def adagrad_clr(lr: float, lr_decay: float, step: float) -> float:
+    """Effective learning rate of Adagrad step `step` (1-based, the value of state["step"] after its increment), as
+    torch.optim.Adagrad computes it: lr / (1 + (step - 1) * lr_decay).  Adagrad.step and the captured steps of
+    trainer.py share this one formula."""
+    return lr / (1 + (step - 1) * lr_decay)
+
+
+def group_of(optimizer: torch.optim.Optimizer, param: torch.Tensor) -> dict:
+    """The parameter group of `optimizer` that holds `param` (by identity; ValueError if none does)."""
+    for group in optimizer.param_groups:
+        if any(p is param for p in group["params"]):
+            return group
+    raise ValueError("the tensor is not a parameter of any group of the optimizer")
+
+
 class Adagrad(torch.optim.Optimizer):
     """torch.optim.Adagrad: g += wd*w; sum += g*g; w -= lr/(1+(step-1)*lr_decay) * g / (sqrt(sum) + eps).
     Dense gradients update every element; sparse (COO) gradients update the touched rows only."""
@@ -32,7 +47,7 @@ class Adagrad(torch.optim.Optimizer):
                     continue
                 st = self.state[p]
                 st["step"] += 1
-                clr = group["lr"] / (1 + (st["step"].item() - 1) * group["lr_decay"])
+                clr = adagrad_clr(group["lr"], group["lr_decay"], st["step"].item())
                 g = p.grad
                 if g.is_sparse:
                     if group["weight_decay"] != 0:

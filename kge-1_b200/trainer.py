@@ -17,7 +17,7 @@ import os
 
 import torch
 
-from . import fused, lib, ops
+from . import fused, lib, ops, optim
 from .model import KgeModel
 
 
@@ -79,6 +79,53 @@ def _inverse_relation_offset(model, reciprocal: bool, what: str) -> int:
     return r
 
 
+def _adagrad_groups(optimizer, params, what: str) -> list:
+    """The parameter group of each table (by identity, not param_groups[0]).  The captured steps apply Adagrad with
+    lr and lr_decay; weight_decay is served by the autograd paths only."""
+    groups = [optim.group_of(optimizer, p) for p in params]
+    if any(g.get("weight_decay", 0.0) != 0.0 for g in groups):
+        raise NotImplementedError(f"{what}: weight_decay != 0 is served by the autograd path only")
+    return groups
+
+
+def adagrad_rates(optimizer, params) -> list:
+    """Effective Adagrad rate of each table for the step the optimizer takes next: optim.adagrad_clr with the lr and
+    lr_decay of the group that holds the table (looked up now, so that an lr scheduler's edits count) at state["step"] + 1
+    -- the value optim.Adagrad.step uses after its increment."""
+    out = []
+    for p in params:
+        g = optim.group_of(optimizer, p)
+        out.append(optim.adagrad_clr(float(g["lr"]), float(g.get("lr_decay", 0.0)), float(optimizer.state[p]["step"]) + 1))
+    return out
+
+
+class _RateWords:
+    """The learning rate of a captured step in device memory: one float32 word per table, read by the _sched kernels the
+    step's CUDA graph launches (include/kgeb200.h).  refresh() runs before every replay: it computes each table's rate
+    (adagrad_rates) and rewrites a word only when its value changed, with fill_ on the current stream -- no allocation, no
+    host sync.  At a constant rate a step issues nothing extra; with lr_decay one tiny fill per table and step.  A rate
+    change therefore needs no re-capture (which would cost a warm-up step and table copies, and is collective for the
+    sharded graphs).  Ranks of a sharded or replicated run must compute the same rates (the same scheduler on the same
+    metric): nothing here checks that they do."""
+
+    def __init__(self, optimizer, params, what: str, dev):
+        self.opt, self.params = optimizer, tuple(params)
+        self.eps = [float(g["eps"]) for g in _adagrad_groups(optimizer, self.params, what)]
+        self.words = torch.zeros(len(self.params), dtype=torch.float32, device=dev)
+        self._word = [self.words[i] for i in range(len(self.params))]
+        self.values = [None] * len(self.params)
+        self.refresh()
+
+    def ptr(self, i: int) -> int:
+        return self.words.data_ptr() + 4 * i
+
+    def refresh(self):
+        for i, r in enumerate(adagrad_rates(self.opt, self.params)):
+            if r != self.values[i]:
+                self._word[i].fill_(r)
+                self.values[i] = r
+
+
 class PeerExchange:
     """The symmetric-memory side of csrc/p2p.cu for a stepper whose gradients live in ONE flat buffer
     [g_table0 (n0) | g_table1 (n1) | loss]: allocates that buffer, the staging buffer [W_table0 | W_table1] and the signal
@@ -109,10 +156,11 @@ class PeerExchange:
         self.timeout = torch.zeros(1, dtype=torch.int32, device=device)
         self.loss_global = torch.zeros((), dtype=torch.float32, device=device)
 
-    def exchange_and_update(self, w0, state0, mirror, w1, state1, lr: float, eps: float, stream: int):
-        lib.call("kgeb_p2p_exchange", self.p_pads, self.p_flat, self.p_stage, self.rank, self.world, self.ctr.data_ptr(),
-                 self.timeout.data_ptr(), w0.data_ptr(), state0.data_ptr(), mirror, w0.numel(), w1.data_ptr(),
-                 state1.data_ptr(), w1.numel(), self.loss_global.data_ptr(), lr, eps, stream)
+    def exchange_and_update(self, w0, state0, mirror, w1, state1, rates: int, eps: float, stream: int):
+        """`rates`: device address of two float32 words, the learning rates of table 0 and table 1 (_RateWords)."""
+        lib.call("kgeb_p2p_exchange_sched", self.p_pads, self.p_flat, self.p_stage, self.rank, self.world,
+                 self.ctr.data_ptr(), self.timeout.data_ptr(), w0.data_ptr(), state0.data_ptr(), mirror, w0.numel(),
+                 w1.data_ptr(), state1.data_ptr(), w1.numel(), self.loss_global.data_ptr(), rates, eps, stream)
         lib.call("kgeb_p2p_apply", self.p_pads, self.stage.data_ptr(), self.rank, self.world, self.ctr.data_ptr(),
                  self.ctr[1:].data_ptr(), self.timeout.data_ptr(), w0.data_ptr(), mirror, w0.numel(), w1.data_ptr(),
                  w1.numel(), stream)
@@ -143,10 +191,11 @@ class _TouchedRows:
                  None if n_b_real is None else n_b_real.data_ptr(), e_lo, e_hi, self.slot_of.data_ptr(), self.uniq.data_ptr(),
                  self.num.data_ptr(), self.slot_a.data_ptr(), self.slot_b.data_ptr(), stream)
 
-    def update(self, w, state, mirror, lr: float, eps: float, skip, stream):
-        lib.call("kgeb_touched_update", w.data_ptr(), state.data_ptr(), None if mirror is None else mirror.data_ptr(),
+    def update(self, w, state, mirror, rate: int, eps: float, skip, stream):
+        """`rate`: device address of the float32 learning-rate word (_RateWords.ptr)."""
+        lib.call("kgeb_touched_update_sched", w.data_ptr(), state.data_ptr(), None if mirror is None else mirror.data_ptr(),
                  self.slot_of.data_ptr(), self.uniq.data_ptr(), self.num.data_ptr(), self.cap, self.g_dense.data_ptr(),
-                 self.g_sparse.data_ptr(), self.d, lr, eps, None if skip is None else skip.data_ptr(), stream)
+                 self.g_sparse.data_ptr(), self.d, rate, eps, None if skip is None else skip.data_ptr(), stream)
 
 
 class FusedAllEntityStepper:
@@ -173,10 +222,11 @@ class FusedAllEntityStepper:
         dev = self.ent.device
         self.E, self.d = self.ent.shape
         self.dr = self.rel.shape[1]
-        group = optimizer.param_groups[0]
-        if group.get("lr_decay", 0.0) != 0.0 or group.get("weight_decay", 0.0) != 0.0:
-            raise NotImplementedError("the graph-captured step bakes lr into the launch (lr_decay / weight_decay = 0)")
-        self.lr, self.eps = float(group["lr"]), float(group["eps"])
+        # the learning rates live in device words (_RateWords): step() follows lr schedulers and lr_decay
+        self.rate = _RateWords(optimizer, (self.ent, self.rel), "FusedAllEntityStepper", dev)
+        self.eps_ent, self.eps_rel = self.rate.eps
+        if dp_group is not None and dp_p2p and self.eps_ent != self.eps_rel:
+            raise NotImplementedError("the peer-memory exchange applies one eps to both tables")
         f32 = dict(dtype=torch.float32, device=dev)
         i64 = dict(dtype=torch.int64, device=dev)
         # Unweighted Lp penalties (lookup_embedder.py:126-134) are folded into the Adagrad kernels (SURVEY.md 8f-3):
@@ -459,9 +509,10 @@ class FusedAllEntityStepper:
         leaves alone."""
         self.side.wait_event(self.ev_clear)           # slot_of is built on the third stream
         t = self.touched
-        lib.call("kgeb_fused_bwd_update", self.loss_kind, self.Q.data_ptr(), self.rows, self.d, self.ent.detach().data_ptr(), 0,
-                 self.E, self.E, self.lab_off.data_ptr(), self.ls, self.offset, lse, 1.0 / self.global_batch, None,
-                 self.mirror.data_ptr(), self.opt.state[self.ent]["sum"].data_ptr(), self.lr, self.eps, t.slot_of.data_ptr(),
+        lib.call("kgeb_fused_bwd_update_sched", self.loss_kind, self.Q.data_ptr(), self.rows, self.d,
+                 self.ent.detach().data_ptr(), 0, self.E, self.E, self.lab_off.data_ptr(), self.ls, self.offset, lse,
+                 1.0 / self.global_batch, None, self.mirror.data_ptr(), self.opt.state[self.ent]["sum"].data_ptr(),
+                 self.rate.ptr(0), self.eps_ent, t.slot_of.data_ptr(),
                  t.g_dense.data_ptr(), self.flash_status.data_ptr() if self._use_flash else None, self.ws3.data_ptr(),
                  self.ws3.numel(), lib.stream_ptr(self.ent))
 
@@ -500,13 +551,13 @@ class FusedAllEntityStepper:
             if self.dp_world == 1:
                 s_rel = self.opt.state[self.rel]["sum"]
                 if self.pen is not None:
-                    lib.call("kgeb_adagrad_dense_lp", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None,
-                             rel.numel(), self.lr, self.eps, 0.0, self.pen["rel"][0], self.pen["rel"][1], None,
+                    lib.call("kgeb_adagrad_dense_lp_sched", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None,
+                             rel.numel(), self.rate.ptr(1), self.eps_rel, 0.0, self.pen["rel"][0], self.pen["rel"][1], None,
                              self.penalty_values[1:].data_ptr(), self.pen_ws[1].data_ptr(), self.pen_ws[1].numel(), st2)
                 else:
                     self._guard_flash(self.g_rel)
-                    lib.call("kgeb_adagrad_dense", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None,
-                             rel.numel(), self.lr, self.eps, 0.0, None, st2)
+                    lib.call("kgeb_adagrad_dense_sched", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None,
+                             rel.numel(), self.rate.ptr(1), self.eps_rel, 0.0, None, st2)
         if self.fuse_update:
             # the sparse rows (label rows, then query-side rows) are summed per touched row underneath the dTable kernel;
             # the row kernel adds the dense part that kernel parked and applies Adagrad to the touched rows
@@ -519,7 +570,7 @@ class FusedAllEntityStepper:
             lib.call("kgeb_scatter_add_rows_perm", t.slot_a.data_ptr(), 1, self.a_perm.data_ptr(), self.da.data_ptr(),
                      self.rows, self.d, t.g_sparse.data_ptr(), t.cap + 1, self.sws.data_ptr(), self.sws.numel(), st)
             self._join_side()
-            t.update(ent, self.opt.state[self.ent]["sum"], self.mirror, self.lr, self.eps,
+            t.update(ent, self.opt.state[self.ent]["sum"], self.mirror, self.rate.ptr(0), self.eps_ent,
                      self.flash_status if self._use_flash else None, st)
             cur.wait_stream(self.side2)
             return
@@ -542,13 +593,14 @@ class FusedAllEntityStepper:
         s_ent = self.opt.state[self.ent]["sum"]
         mirror = None if self.mirror is None else self.mirror.data_ptr()
         if self.pen is not None:
-            lib.call("kgeb_adagrad_dense_lp", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(), self.g_q.data_ptr(),
-                     ent.numel(), self.lr, self.eps, 0.0, self.pen["ent"][0], self.pen["ent"][1], mirror,
+            lib.call("kgeb_adagrad_dense_lp_sched", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(),
+                     self.g_q.data_ptr(), ent.numel(), self.rate.ptr(0), self.eps_ent, 0.0, self.pen["ent"][0],
+                     self.pen["ent"][1], mirror,
                      self.penalty_values.data_ptr(), self.pen_ws[0].data_ptr(), self.pen_ws[0].numel(), st)
         else:
             self._guard_flash(self.gflat[:(1 if self.seq else 2) * self.E * self.d])       # g_ent (and g_q)
-            lib.call("kgeb_adagrad_dense", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(),
-                     None if self.seq else self.g_q.data_ptr(), ent.numel(), self.lr, self.eps, 0.0, mirror, st)
+            lib.call("kgeb_adagrad_dense_sched", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(),
+                     None if self.seq else self.g_q.data_ptr(), ent.numel(), self.rate.ptr(0), self.eps_ent, 0.0, mirror, st)
         cur.wait_stream(self.side2)
 
     # -- data-parallel exchange fused with the update over NVLink peer memory (csrc/p2p.cu) ---------------------------
@@ -586,9 +638,10 @@ class FusedAllEntityStepper:
         ent, rel = self.ent.detach(), self.rel.detach()
         s_ent, s_rel = self.opt.state[self.ent]["sum"], self.opt.state[self.rel]["sum"]
         mirror = None if self.mirror is None else self.mirror.data_ptr()
-        lib.call("kgeb_p2p_exchange", x["pads"], x["flat"], x["stage"], x["rank"], x["world"], self.p2p_ctr.data_ptr(),
-                 self.p2p_timeout.data_ptr(), ent.data_ptr(), s_ent.data_ptr(), mirror, ent.numel(), rel.data_ptr(),
-                 s_rel.data_ptr(), rel.numel(), self.loss_global.data_ptr(), self.lr, self.eps, st)
+        lib.call("kgeb_p2p_exchange_sched", x["pads"], x["flat"], x["stage"], x["rank"], x["world"],
+                 self.p2p_ctr.data_ptr(), self.p2p_timeout.data_ptr(), ent.data_ptr(), s_ent.data_ptr(), mirror, ent.numel(),
+                 rel.data_ptr(), s_rel.data_ptr(), rel.numel(), self.loss_global.data_ptr(), self.rate.words.data_ptr(),
+                 self.eps_ent, st)
         lib.call("kgeb_p2p_apply", x["pads"], self.p2p_stage.data_ptr(), x["rank"], x["world"], self.p2p_ctr.data_ptr(),
                  self.p2p_ctr[1:].data_ptr(), self.p2p_timeout.data_ptr(), ent.data_ptr(), mirror, ent.numel(),
                  rel.data_ptr(), rel.numel(), st)
@@ -611,10 +664,10 @@ class FusedAllEntityStepper:
         st = lib.stream_ptr(self.ent)
         ent, rel = self.ent.detach(), self.rel.detach()
         s_ent, s_rel = self.opt.state[self.ent]["sum"], self.opt.state[self.rel]["sum"]
-        lib.call("kgeb_adagrad_dense", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None, rel.numel(),
-                 self.lr, self.eps, 0.0, None, st)
-        lib.call("kgeb_adagrad_dense", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(), None,
-                 ent.numel(), self.lr, self.eps, 0.0, None if self.mirror is None else self.mirror.data_ptr(), st)
+        lib.call("kgeb_adagrad_dense_sched", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None, rel.numel(),
+                 self.rate.ptr(1), self.eps_rel, 0.0, None, st)
+        lib.call("kgeb_adagrad_dense_sched", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(), None,
+                 ent.numel(), self.rate.ptr(0), self.eps_ent, 0.0, None if self.mirror is None else self.mirror.data_ptr(), st)
 
     def _exchange_dp(self):
         import torch.distributed as dist
@@ -767,6 +820,7 @@ class FusedAllEntityStepper:
 
     def step(self) -> torch.Tensor:
         """Runs one training step; returns the (device) loss tensor of this batch."""
+        self.rate.refresh()       # the optimizer's current rates (the two-pass graph of a failed flash pass reads the same)
         if self.graph is None:
             self._launch()
             if self.flash and int(self.flash_status[0].item()) != 0:
@@ -835,10 +889,8 @@ class RowShardedAllEntityStepper:
         dev = self.ent.device
         self.E, self.d = self.ent.shape
         self.dr = self.rel.shape[1]
-        group = optimizer.param_groups[0]
-        if group.get("lr_decay", 0.0) != 0.0 or group.get("weight_decay", 0.0) != 0.0:
-            raise NotImplementedError("the graph-captured step bakes lr into the launch (lr_decay / weight_decay = 0)")
-        self.lr, self.eps = float(group["lr"]), float(group["eps"])
+        self.rate = _RateWords(optimizer, (self.ent, self.rel), "RowShardedAllEntityStepper", dev)
+        self.eps_ent, self.eps_rel = self.rate.eps
         self.e_lo, self.e_hi = shard.e_lo, shard.e_hi
         self.n_loc = self.e_hi - self.e_lo
         f32 = dict(dtype=torch.float32, device=dev)
@@ -998,10 +1050,10 @@ class RowShardedAllEntityStepper:
                 lib.call("kgeb_fused_bwd_wait_tiles", lib.stream_ptr(self.ent))
             if self.fuse_update:
                 # dense part + Adagrad in the tile kernel's flush; rows of the touched set are parked for _stage_update
-                lib.call("kgeb_fused_bwd_update", self.loss_kind, self.Q.data_ptr(), self.rows, self.d,
+                lib.call("kgeb_fused_bwd_update_sched", self.loss_kind, self.Q.data_ptr(), self.rows, self.d,
                          self._ent_loc().data_ptr(), self.e_lo, self.e_hi, self.E, self.lab_off.data_ptr(), self.ls, self.offset,
                          lse, 1.0 / self.batch_size, None, self.mirror.data_ptr(),
-                         self.opt.state[self.ent]["sum"][self.e_lo:self.e_hi].data_ptr(), self.lr, self.eps,
+                         self.opt.state[self.ent]["sum"][self.e_lo:self.e_hi].data_ptr(), self.rate.ptr(0), self.eps_ent,
                          self.touched.slot_of.data_ptr(), self.touched.g_dense.data_ptr(),
                          self.flash_status.data_ptr() if self._use_flash else None, self.ws2.data_ptr(), self.ws2.numel(),
                          lib.stream_ptr(self.ent))
@@ -1033,8 +1085,8 @@ class RowShardedAllEntityStepper:
         lib.call("kgeb_scatter_add_rows", self.p_idx.data_ptr(), 1, self.dp.data_ptr(), self.rows, self.dr,
                  self.g_rel.data_ptr(), self.rel.shape[0], self.sws2.data_ptr(), self.sws2.numel(), st)
         self._guard_flash(self.g_rel)
-        lib.call("kgeb_adagrad_dense", rel.data_ptr(), self.opt.state[self.rel]["sum"].data_ptr(), self.g_rel.data_ptr(),
-                 None, rel.numel(), self.lr, self.eps, 0.0, None, st)
+        lib.call("kgeb_adagrad_dense_sched", rel.data_ptr(), self.opt.state[self.rel]["sum"].data_ptr(),
+                 self.g_rel.data_ptr(), None, rel.numel(), self.rate.ptr(1), self.eps_rel, 0.0, None, st)
         if self.fuse_update:
             # label rows of this shard and the query-side rows it owns, summed per touched row (rows of other owners go to the
             # dummy slot) -- still underneath the dTable kernel; then the row kernel finishes the touched rows
@@ -1049,7 +1101,8 @@ class RowShardedAllEntityStepper:
                      t.g_sparse.data_ptr(), t.cap + 1, self.sws.data_ptr(), self.sws.numel(), st)
             if self.px is not None:
                 torch.cuda.current_stream().wait_stream(self.side)
-            t.update(self._ent_loc(), self.opt.state[self.ent]["sum"][self.e_lo:self.e_hi], self.mirror, self.lr, self.eps,
+            t.update(self._ent_loc(), self.opt.state[self.ent]["sum"][self.e_lo:self.e_hi], self.mirror, self.rate.ptr(0),
+                     self.eps_ent,
                      self.flash_status if self._use_flash else None, st)
             return
         if self.px is not None:
@@ -1064,8 +1117,8 @@ class RowShardedAllEntityStepper:
         if self.n_loc > 0:
             self._guard_flash(self.g_all[:self.n_loc])
             s_loc = self.opt.state[self.ent]["sum"][self.e_lo:self.e_hi]
-            lib.call("kgeb_adagrad_dense", self._ent_loc().data_ptr(), s_loc.data_ptr(), self.g_ent.data_ptr(),
-                     None if self.one_buffer else self.g_q.data_ptr(), self.n_loc * self.d, self.lr, self.eps, 0.0,
+            lib.call("kgeb_adagrad_dense_sched", self._ent_loc().data_ptr(), s_loc.data_ptr(), self.g_ent.data_ptr(),
+                     None if self.one_buffer else self.g_q.data_ptr(), self.n_loc * self.d, self.rate.ptr(0), self.eps_ent, 0.0,
                      None if self.mirror is None else self.mirror.data_ptr(), st)
 
     def _setup_peer(self, rows: int, dev):
@@ -1193,6 +1246,7 @@ class RowShardedAllEntityStepper:
         self.lab_col[: lab_col.numel()].copy_(lab_col, non_blocking=True)
 
     def step(self) -> torch.Tensor:
+        self.rate.refresh()
         if self.graphs is None:
             self._launch()
             if self.flash and int(self.flash_status[0].item()) != 0:
@@ -1279,10 +1333,10 @@ class FusedNegSamplingStepper:
         dev = self.ent.device
         self.E, self.d = self.ent.shape
         self.dr = self.rel.shape[1]
-        group = optimizer.param_groups[0]
-        if group.get("lr_decay", 0.0) != 0.0 or group.get("weight_decay", 0.0) != 0.0:
-            raise NotImplementedError("the graph-captured step bakes lr into the launch (lr_decay / weight_decay = 0)")
-        self.lr, self.eps = float(group["lr"]), float(group["eps"])
+        self.rate = _RateWords(optimizer, (self.ent, self.rel), "FusedNegSamplingStepper", dev)
+        self.eps_ent, self.eps_rel = self.rate.eps
+        if dp_group is not None and self.eps_ent != self.eps_rel:
+            raise NotImplementedError("the peer-memory exchange applies one eps to both tables")
         f32 = dict(dtype=torch.float32, device=dev)
         i64 = dict(dtype=torch.int64, device=dev)
         B = batch_size
@@ -1382,12 +1436,12 @@ class FusedNegSamplingStepper:
         torch.sum(torch.stack([self.buf[s]["rows"].sum() for s in self.slots]), dim=0, out=self.loss)
         s_ent, s_rel = self.opt.state[self.ent]["sum"], self.opt.state[self.rel]["sum"]
         if self.px is not None:     # exchange + update of the owned slices + gather of the new weights, in this graph
-            self.px.exchange_and_update(ent, s_ent, None, rel, s_rel, self.lr, self.eps, st)
+            self.px.exchange_and_update(ent, s_ent, None, rel, s_rel, self.rate.words.data_ptr(), self.eps_ent, st)
             return
-        lib.call("kgeb_adagrad_dense", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(), None, ent.numel(),
-                 self.lr, self.eps, 0.0, None, st)
-        lib.call("kgeb_adagrad_dense", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None, rel.numel(),
-                 self.lr, self.eps, 0.0, None, st)
+        lib.call("kgeb_adagrad_dense_sched", ent.data_ptr(), s_ent.data_ptr(), self.g_ent.data_ptr(), None, ent.numel(),
+                 self.rate.ptr(0), self.eps_ent, 0.0, None, st)
+        lib.call("kgeb_adagrad_dense_sched", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None, rel.numel(),
+                 self.rate.ptr(1), self.eps_rel, 0.0, None, st)
 
     def _capture(self):
         keep = [t.detach().clone() for t in (self.ent, self.rel, self.opt.state[self.ent]["sum"],
@@ -1415,6 +1469,7 @@ class FusedNegSamplingStepper:
             self.neg[slot].copy_(negative_samples[slot], non_blocking=True)
 
     def step(self) -> torch.Tensor:
+        self.rate.refresh()
         if self.graph is not None:
             self.graph.replay()
         else:
@@ -1499,10 +1554,9 @@ class ShardedNegSamplingStepper:
         self.ent, self.rel = model.get_s_embedder().weight, model.get_p_embedder().weight
         self.E, self.d = self.ent.shape
         self.dr = self.rel.shape[1]
-        pg = optimizer.param_groups[0]
-        if pg.get("lr_decay", 0.0) != 0.0 or pg.get("weight_decay", 0.0) != 0.0:
-            raise NotImplementedError("lr_decay / weight_decay are not part of this step")
-        self.lr, self.eps = float(pg["lr"]), float(pg["eps"])
+        # eager: the rates are read from the optimizer's groups and passed by value every step (adagrad_rates)
+        self.eps_ent, self.eps_rel = [float(g["eps"]) for g in
+                                      _adagrad_groups(optimizer, (self.ent, self.rel), "ShardedNegSamplingStepper")]
         self.ex = RowExchange(self.E, group)
         self.world = self.ex.world
         self.global_batch = batch_size * self.world
@@ -1578,11 +1632,12 @@ class ShardedNegSamplingStepper:
         self.g_rel.copy_(flat[:-1].view_as(self.g_rel))
         self.loss.copy_(flat[-1])
         s_ent, s_rel = self.opt.state[self.ent]["sum"], self.opt.state[self.rel]["sum"]
+        lr_ent, lr_rel = adagrad_rates(self.opt, (self.ent, self.rel))
         if self.n_loc > 0:
             lib.call("kgeb_adagrad_dense", loc.data_ptr(), s_ent[self.ex.lo:self.ex.hi].data_ptr(), self.g_loc.data_ptr(), None,
-                     self.n_loc * d, self.lr, self.eps, 0.0, None, st)
-        lib.call("kgeb_adagrad_dense", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None, rel.numel(), self.lr,
-                 self.eps, 0.0, None, st)
+                     self.n_loc * d, lr_ent, self.eps_ent, 0.0, None, st)
+        lib.call("kgeb_adagrad_dense", rel.data_ptr(), s_rel.data_ptr(), self.g_rel.data_ptr(), None, rel.numel(), lr_rel,
+                 self.eps_rel, 0.0, None, st)
         for stt in (self.opt.state[self.ent], self.opt.state[self.rel]):
             stt["step"] += 1
         torch.autograd.graph.increment_version(self.ent)
