@@ -6,6 +6,8 @@ profiles/extra_workloads_r1.jsonl and summarised in DESIGN.md.
     python bench_extra.py --workload wd5m-1vsall | wnrr-rotate-ns | wd5m-eval-transe | wd5m-eval-complex [--scale F]
     python bench_extra.py --workload wd5m-1vsall-reciprocal --batch 1024
     python bench_extra.py --workload wd5m-1vsall-lr-schedule --batch 1024
+    python bench_extra.py --workload fb237-distance-allentity --batch 512
+    python bench_extra.py --workload wd5m-transe-1vsall --batch 1024
 """
 import argparse
 import json
@@ -242,6 +244,160 @@ def wd5m_1vsall_lr_schedule(args):
             **gpu_info()}
 
 
+# fp32 operations per (query row, entity, embedding column) of the fused distance kernels: the forward tile (subtract,
+# accumulate), and per backward half (dQ, dTable) the recomputed tile plus the second phase (subtract, accumulate)
+DISTANCE_OPS = 2 + 2 * (2 + 2)
+FMA_PER_CLK_SM = 125.0       # fp32 issue rate per SM and clock, profiles/mufu_rates_r1.txt
+
+
+def _max_sm_clock_hz() -> float:
+    import subprocess
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=clocks.max.sm", "--format=csv,noheader,nounits", "-i",
+                              str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout
+        return float(out.strip().splitlines()[0]) * 1e6
+    except (OSError, ValueError, IndexError, subprocess.SubprocessError):
+        return float("nan")
+
+
+def _distance_kernels_ms(kind, loss, q, w, lab_off, lab_col, steps, warmup):
+    """kgeb_fused_fwd_kind + kgeb_fused_bwd_kind (dQ and dTable) on the step's shapes, timed alone."""
+    lib = kb.lib
+    n, d = q.shape
+    e = w.shape[0]
+    rowstat = torch.empty(n, 4, device=q.device)
+    lse = torch.zeros(n, device=q.device)
+    dq, dw = torch.empty_like(q), torch.empty_like(w)
+    ws = torch.empty(lib.load().kgeb_fused_workspace_bytes(n, d, e, lab_col.numel()), dtype=torch.uint8, device=q.device)
+
+    def call():
+        lib.call("kgeb_fused_fwd_kind", kind, loss, q.data_ptr(), n, d, w.data_ptr(), 0, e, e, lab_off.data_ptr(),
+                 lab_col.data_ptr(), lab_col.numel(), 0.0, 0.0, rowstat.data_ptr(), ws.data_ptr(), ws.numel(),
+                 lib.stream_ptr(q))
+        lib.call("kgeb_fused_bwd_kind", kind, loss, q.data_ptr(), n, d, w.data_ptr(), 0, e, e, lab_off.data_ptr(),
+                 lab_col.data_ptr(), lab_col.numel(), 0.0, 0.0, lse.data_ptr(), 1.0 / n, None, dq.data_ptr(), dw.data_ptr(),
+                 lib.BWD_OVERWRITE_TABLE, ws.data_ptr(), ws.numel(), lib.stream_ptr(q))
+    return timed(call, steps, warmup)
+
+
+def _issue_share(n_rows, n_ent, d, kernel_ms, clock_hz):
+    """Share of the fp32 issue rate (148 SMs x 125 per clock at the card's maximum SM clock) the kernels reach."""
+    ops = float(n_rows) * n_ent * d * DISTANCE_OPS
+    return ops, ops / (kernel_ms * 1e-3) / (148 * FMA_PER_CLK_SM * clock_hz)
+
+
+def fb237_distance_allentity(args):
+    """TransE (L1) and RotatE (L1), d = 128, at the FB15k-237 shape (14,541 entities, 237 relations): KvsAll + BCE and
+    1vsAll + KL.  Per case, in one process and alternating rounds of --steps steps: the fused captured step
+    (FusedAllEntityStepper, fp32 distance tiles, one CUDA graph) against the materialised autograd flow (kgeb_score_all
+    -> torch's loss -> kgeb_score_all_bwd -> Adagrad) on the same batch; then the fused kernels alone and their share
+    of the fp32 issue rate."""
+    E, R, d, B = 14_541, 237, 128, args.batch
+    dev = torch.device("cuda")
+    clock = _max_sm_clock_hz()
+    gen = torch.Generator().manual_seed(1)
+    out = []
+    for model_name in ("transe", "rotate"):
+        for ttype, loss_name in (("KvsAll", "bce"), ("1vsAll", "kl")):
+            arms = {}
+            for arm in ("fused", "materialised"):
+                torch.manual_seed(0)
+                m = kb.KgeModel(model_name, E, R, d, l_norm=1.0).to(dev)
+                opt = kb.optim.create("Adagrad", m.parameters(), lr=0.1)
+                arms[arm] = (m, opt)
+            lossf = kb.KgeLoss.create(loss_name)
+            triples = torch.stack((torch.randint(0, E, (B,), generator=gen), torch.randint(0, R, (B,), generator=gen),
+                                   torch.randint(0, E, (B,), generator=gen)), 1)
+            if ttype == "1vsAll":
+                rows = 2 * B
+                st = kb.trainer.FusedAllEntityStepper(*arms["fused"], rows, rows, lossf.kind, B, onevsall_triples=True)
+                st.set_triples(triples.to(dev))
+                job = kb.TrainingJob1vsAll(*arms["materialised"], lossf, fused_path=False)
+                batch = {"triples": triples}
+                lab_off = torch.arange(rows + 1, device=dev)
+                lab_col = torch.cat((triples[:, 2], triples[:, 0])).to(dev)
+            else:
+                rows = B
+                qt = (torch.arange(B) % 2).int()
+                # KvsAll query rows: sp_ = (s, p), _po = (p, o)
+                queries = torch.where((qt == 0)[:, None], triples[:, :2], triples[:, 1:])
+                per = torch.randint(1, 8, (B,), generator=gen)          # 1..7 answers per query, as FB15k-237's KvsAll rows
+                coords = torch.stack((torch.repeat_interleave(torch.arange(B), per),
+                                      torch.randint(0, E, (int(per.sum()),), generator=gen)), 1)
+                batch = {"queries": queries, "label_coords": coords, "query_type_indexes": qt}
+                fj = kb.TrainingJobKvsAll(*arms["fused"], lossf, E, R)
+                st = fj.enable_graph_step(B, len(coords))
+                st.set_inputs(*fj.device_inputs(batch))
+                job = kb.TrainingJobKvsAll(*arms["materialised"], lossf, E, R, fused_path=False)
+                lab_off, lab_col = kb.fused.csr_from_coords(coords.to(dev), B)
+            state = {"i": 0}
+
+            def materialised_step():
+                job.step(state["i"], batch)
+                state["i"] += 1
+
+            ms = {"fused": [], "materialised": []}
+            for _ in range(5):
+                ms["fused"].append(timed(st.step, args.steps, args.warmup))
+                ms["materialised"].append(timed(materialised_step, args.steps, args.warmup))
+            med = {k: float(np.median(v)) for k, v in ms.items()}
+            kind = st.kind
+            q = torch.randn(rows, d, device=dev) * 0.3
+            w = arms["fused"][0].get_s_embedder().weight.detach()
+            kms = [_distance_kernels_ms(kind, lossf.kind, q, w, lab_off, lab_col, args.steps, args.warmup) for _ in range(3)]
+            kmed = float(np.median(kms))
+            ops, share = _issue_share(rows, E, d, kmed, clock)
+            out.append({"case": f"{model_name} L1 {ttype}+{loss_name.upper()}", "query_rows": rows,
+                        "ms_per_step_fused_captured": med["fused"], "ms_per_step_materialised_autograd": med["materialised"],
+                        "speedup": med["materialised"] / med["fused"], "ms_rounds": ms,
+                        "fused_kernels_ms": kmed, "fused_kernel_fp32_ops": ops, "fp32_issue_share_at_max_clock": share,
+                        "loss_fused": st.loss.item()})
+    return {"workload": f"TransE / RotatE (L1) d={d} E={E} R={R} batch={B} triples (1vsAll: {2 * B} query rows; KvsAll: "
+                        f"{B} query rows), fused captured step vs materialised autograd flow, alternating rounds",
+            "metric": "ms per step", "value": out[0]["ms_per_step_fused_captured"], "cases": out,
+            "ops_per_row_entity_column": DISTANCE_OPS, "max_sm_clock_hz": clock, **gpu_info()}
+
+
+def wd5m_transe_1vsall(args):
+    """The Wikidata5M shape (4.6 M entities, 822 relations, d = 128), TransE L1, 1vsAll + KL, --batch triples: the fused
+    captured step alone (no [B, E] matrix: the materialised flow needs two [2B, E] fp32 matrices, 2 x 37.7 GB at 1,024
+    triples), and the fused kernels' share of the fp32 issue rate."""
+    E, R, d, B = int(4_600_000 * args.scale), 822, 128, args.batch
+    dev = torch.device("cuda")
+    torch.manual_seed(0)
+    m = kb.KgeModel("transe", E, R, d, l_norm=1.0).to(dev)
+    opt = kb.optim.create("Adagrad", m.parameters(), lr=0.1)
+    st = kb.trainer.FusedAllEntityStepper(m, opt, 2 * B, 2 * B, kb.lib.LOSS_KL, B, onevsall_triples=True)
+    gen = torch.Generator(device=dev).manual_seed(1)
+    batches = [torch.stack((torch.randint(0, E, (B,), device=dev, generator=gen),
+                            torch.randint(0, R, (B,), device=dev, generator=gen),
+                            torch.randint(0, E, (B,), device=dev, generator=gen)), 1) for _ in range(4)]
+    state = {"i": 0}
+
+    def step():
+        st.set_triples(batches[state["i"] % len(batches)])
+        state["i"] += 1
+        st.step()
+
+    torch.cuda.reset_peak_memory_stats()
+    ms = [timed(step, args.steps, args.warmup) for _ in range(3)]
+    peak = torch.cuda.max_memory_allocated()
+    med = float(np.median(ms))
+    t = batches[0]
+    q = torch.randn(2 * B, d, device=dev) * 0.3
+    lab_off = torch.arange(2 * B + 1, device=dev)
+    lab_col = torch.cat((t[:, 2], t[:, 0]))
+    kms = _distance_kernels_ms(kb.lib.NEG_L1, kb.lib.LOSS_KL, q, m.get_s_embedder().weight.detach(), lab_off, lab_col,
+                               max(1, args.steps // 2), 1)
+    clock = _max_sm_clock_hz()
+    ops, share = _issue_share(2 * B, E, d, kms, clock)
+    return {"workload": f"TransE L1 1vsAll+KL d={d} E={E} R={R} B={B} triples ({2 * B} query rows) fp32 distance tiles, "
+                        "fused captured step, batch built on the device",
+            "metric": "ms per step", "value": med, "ms_rounds": ms, "fused_kernels_ms": kms, "fused_kernel_fp32_ops": ops,
+            "fp32_issue_share_at_max_clock": share, "max_sm_clock_hz": clock, "peak_allocated_gb": peak / 1e9,
+            "loss": st.loss.item(), **gpu_info()}
+
+
 def wnrr_rotate_ns(args):
     """C3: RotatE negative sampling, 256 negatives for s and o, E=40943, R=11, B=512."""
     E, R, d, B, N = 40943, 11, 128, args.batch, 256
@@ -372,6 +528,10 @@ def main():
         res = wd5m_1vsall_reciprocal(args)
     elif args.workload == "wd5m-1vsall-lr-schedule":
         res = wd5m_1vsall_lr_schedule(args)
+    elif args.workload == "fb237-distance-allentity":
+        res = fb237_distance_allentity(args)
+    elif args.workload == "wd5m-transe-1vsall":
+        res = wd5m_transe_1vsall(args)
     elif args.workload == "wnrr-rotate-ns":
         res = wnrr_rotate_ns(args)
     elif args.workload == "wd5m-eval-transe":

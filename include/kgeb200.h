@@ -210,6 +210,23 @@ int kgeb_fused_bwd(int loss, int math, const float* Q, int64_t B, int d, const f
                    float* rowstat_out /* [B,4] or NULL: also produce the forward statistics of kgeb_fused_fwd (BCE on the
                                          bf16 tiles gets them from the same pass; otherwise the forward kernels run) */,
                    int flags /* 0 | KGEB_BWD_OVERWRITE_TABLE */, void* workspace, int64_t workspace_bytes, void* stream);
+/* kgeb_fused_fwd / kgeb_fused_bwd for every pair kind on the fp32 CUDA-core tiles: the fused score + loss of TransE
+ * (KGEB_NEG_L1 / _L2, transe.py:14-24) and RotatE (KGEB_ROT_L1 / _L2, rotate.py:18-63, 97-145) under the KL and BCE
+ * losses (loss.py:137-159, 192-213), without the [B, E] score matrix.  Same statistics layout, workspace
+ * (kgeb_fused_workspace_bytes), label CSR, shard range, KGEB_BWD_OVERWRITE_TABLE and results as the two entries above;
+ * scores are those of kgeb_score_all (RotatE +distance, TransE without eps) and gradients follow kgeb_score_all_bwd
+ * (sign(0) = 0, zero distance or zero modulus -> zero gradient).  kind == KGEB_DOT is kgeb_fused_fwd / _bwd with
+ * KGEB_MATH_FP32.  KGEB_ERR_UNSUPPORTED: d > 256, KL with label smoothing; an odd d for RotatE is an argument error. */
+int kgeb_fused_fwd_kind(int kind, int loss, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,
+                        int64_t e_hi, int64_t num_entities, const int64_t* lab_off, const int64_t* lab_col, int64_t nnz,
+                        float label_smoothing, float offset, float* rowstat /*[B,4]*/, void* workspace,
+                        int64_t workspace_bytes, void* stream);
+int kgeb_fused_bwd_kind(int kind, int loss, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,
+                        int64_t e_hi, int64_t num_entities, const int64_t* lab_off, const int64_t* lab_col, int64_t nnz,
+                        float label_smoothing, float offset, const float* lse /*[B] (KL)*/, float inv_batch,
+                        const float* row_scale /*[B] or NULL*/, float* dQ, float* dTable,
+                        int flags /* 0 | KGEB_BWD_OVERWRITE_TABLE */, void* workspace, int64_t workspace_bytes,
+                        void* stream);
 /* loss(scores, labels) / batch_size from the (shard-combined) forward statistics, as the reference's loss objects
  * return it (loss.py:153-159, 198-213): rows_out[B] per-row values (may be NULL), lse_out[B] log-sum-exp per row for
  * the KL backward (may be NULL), total[1] their sum in a fixed order. */

@@ -297,10 +297,11 @@ struct LossParams {
 };
 
 // ------------------------------------------------------------------------------------------
-// fused forward statistics (DOT): CTA = (row block, entity chunk); partials to workspace
+// fused forward statistics (all kinds): CTA = (row block, entity chunk); partials to workspace
 // rowstat layout per row: [0] KL: running max / BCE: sum softplus(x+off)   [1] KL: sum exp(x-max)
 //                         [2] sum_j (x+off)                                 [3] sum over label entries (x+off)
 // ------------------------------------------------------------------------------------------
+template <int KIND>
 __global__ void __launch_bounds__(TT)
 fused_fwd_kernel(LossParams lp, const float* __restrict__ Q, int64_t B, int d, const float* __restrict__ table,
                  int64_t e_lo, int64_t n_ent, const int64_t* __restrict__ lab_off,
@@ -328,7 +329,7 @@ fused_fwd_kernel(LossParams lp, const float* __restrict__ Q, int64_t B, int d, c
   for (int64_t t = t_begin; t < t_end; ++t) {
     const int64_t col0 = t * BN;
     float acc[4][4];
-    tile_accumulate<KGEB_DOT>(Q, B, row0, table, nullptr, 0, n_ent, col0, d, sm, acc);
+    tile_accumulate<KIND>(Q, B, row0, table, nullptr, 0, n_ent, col0, d, sm, acc);
     const int64_t cbase = col0 + tx * 4;  // first local candidate of this thread
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -420,9 +421,16 @@ __global__ void fused_fwd_finalize(int loss, const float* __restrict__ partial, 
 }
 
 // ------------------------------------------------------------------------------------------
-// fused backward (DOT).  G tile is recomputed in registers, staged in shared memory, and consumed by
-// a second FFMA phase.  MODE 0: dQ for a (row block, entity chunk) -> partial workspace.
-//                        MODE 1: dTable for an entity tile over all row blocks (+= in place).
+// fused backward (all kinds).  G tile is recomputed in registers, staged in shared memory, and consumed by
+// a second phase.  MODE 0: dQ for a (row block, entity chunk) -> partial workspace.
+//                  MODE 1: dTable for an entity tile over all row blocks (+= in place).
+// The second phase is written for the "own" side (MODE 0: the query rows, MODE 1: the entities) against the "other"
+// side, with score_all_bwd_kernel's conventions (pair_grad): d/d own = sum over other of G * f(own - other) with
+//   DOT    f = other                               (FFMA)
+//   NEG_L1 f = -sign(own - other), sign(0) = 0
+//   ROT_L1 f = (own - other) / |own - other|_C per column pair (k, k + d/2), 0 at zero modulus
+//   L2     f = (own - other) / x, x the score (-dist / +dist), 0 at zero distance.  1/x is folded into G when it is
+//          staged (G'), so the phase is DOT's FFMA plus the row sums of G': d/d own = own * sum G' - sum G' other.
 // ------------------------------------------------------------------------------------------
 template <int NC>
 struct BwdSmem {
@@ -456,7 +464,40 @@ __device__ __forceinline__ void grad_tile(const LossParams& lp, const float (&ac
   }
 }
 
-template <int NC, int MODE>
+// Column of accumulator slot c of a lane (d when the slot is unused).  Slots are lane + 32 c; for ROT_L1 the first
+// NC / 2 slots hold columns k < d/2 and the last NC / 2 the partner columns k + d/2, so a lane owns whole pairs.
+template <int KIND, int NC>
+__device__ __forceinline__ int slot_col(int lane, int c, int d) {
+  if constexpr (KIND == KGEB_ROT_L1) {
+    constexpr int H = NC / 2;
+    const int h = d >> 1, k = lane + 32 * (c % H);
+    return k < h ? k + (c >= H ? h : 0) : d;
+  } else {
+    return lane + 32 * c;
+  }
+}
+
+// out[c] += G * f(own - other) of the L1 kinds (see above) for one (own, other) pair
+template <int KIND, int NC>
+__device__ __forceinline__ void l1_pair_step(float gv, const float (&own)[NC], const float (&other)[NC],
+                                             float (&out)[NC]) {
+  if constexpr (KIND == KGEB_NEG_L1) {
+#pragma unroll
+    for (int c = 0; c < NC; ++c) out[c] = fmaf(-gv, sgnf(own[c] - other[c]), out[c]);
+  } else {
+    constexpr int H = NC / 2;
+#pragma unroll
+    for (int c = 0; c < H; ++c) {
+      const float re = own[c] - other[c], im = own[c + H] - other[c + H];
+      const float m2 = fmaf(re, re, im * im);
+      const float inv = m2 == 0.f ? 0.f : gv * rsqrtf(m2);
+      out[c] = fmaf(re, inv, out[c]);
+      out[c + H] = fmaf(im, inv, out[c + H]);
+    }
+  }
+}
+
+template <int KIND, int NC, int MODE>
 __global__ void __launch_bounds__(TT)
 fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float* __restrict__ Q, int64_t B, int d, const float* __restrict__ table,
                  int64_t e_lo, int64_t n_ent, const int64_t* __restrict__ lab_off,
@@ -464,6 +505,8 @@ fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float
                  const float* __restrict__ tscale, int64_t tiles_per_chunk, float* __restrict__ out) {
   // tscale[r]: weight of one label entry of row r in t (KL: (1-ls)/Z_r ; BCE: (1-ls)); the dense part of
   // t is ls_add (BCE) or ls_add/Z folded by the caller into lp.ls_add == 0 for KL (ls unsupported there).
+  constexpr bool kL1 = (KIND == KGEB_NEG_L1 || KIND == KGEB_ROT_L1);
+  constexpr bool kL2 = (KIND == KGEB_NEG_L2 || KIND == KGEB_ROT_L2);
   extern __shared__ __align__(16) unsigned char raw[];
   BwdSmem<NC>& sm = *reinterpret_cast<BwdSmem<NC>*>(raw);
   const LossParams lp = lp_in;
@@ -478,6 +521,22 @@ fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float
     for (int c = 0; c < NC; ++c) out_acc[a][c] = 0.f;
 
   const int64_t outer = MODE == 0 ? (int64_t)blockIdx.y : (int64_t)blockIdx.x;  // row block | entity tile
+  // own-side rows of this warp: MODE 0 query rows, MODE 1 entities (local ids)
+  const float* own_base = MODE == 0 ? Q : table;
+  const int64_t own0 = outer * (MODE == 0 ? BM : BN) + warp * 8, n_own = MODE == 0 ? B : n_ent;
+  float own[kL1 ? 8 : 1][kL1 ? NC : 1];   // L1 kinds: own-side operand values, held for the whole block
+  float gsum[8];                          // L2 kinds: row sums of G'
+#pragma unroll
+  for (int a = 0; a < 8; ++a) {
+    gsum[a] = 0.f;
+    if constexpr (kL1) {
+#pragma unroll
+      for (int c = 0; c < NC; ++c) {
+        const int col = slot_col<KIND, NC>(lane, c, d);
+        own[a][c] = (col < d && own0 + a < n_own) ? __ldg(own_base + (own0 + a) * d + col) : 0.f;
+      }
+    }
+  }
   int64_t in_begin, in_end;
   if (MODE == 0) {
     in_begin = (int64_t)blockIdx.x * tiles_per_chunk;
@@ -490,7 +549,7 @@ fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float
     const int64_t row0 = (MODE == 0 ? outer : inner) * BM;
     const int64_t col0 = (MODE == 0 ? inner : outer) * BN;
     float acc[4][4], g[4][4];
-    tile_accumulate<KGEB_DOT>(Q, B, row0, table, nullptr, 0, n_ent, col0, d, sm.t, acc);
+    tile_accumulate<KIND>(Q, B, row0, table, nullptr, 0, n_ent, col0, d, sm.t, acc);
     grad_tile(lp, acc, g, lse, gscale, row0, B, col0, n_ent, ty, tx);
 #pragma unroll
     for (int i = 0; i < 4; ++i)
@@ -513,44 +572,75 @@ fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float
       }
     }
     __syncthreads();
+    if constexpr (kL2) {
+      // G' = G / x with the score x this thread recomputed (zero distance -> zero gradient)
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          float& gg = sm.g[ty * 4 + i][tx * 4 + j];
+          gg = acc[i][j] == 0.f ? 0.f : gg / acc[i][j];
+        }
+      __syncthreads();
+    }
     if (MODE == 0) {
-      // dQ[rows of warp][cols of lane] += sum_j G[row][j] * table[col0+j][col]
+      // dQ[rows of warp][cols of lane] += sum_j G[row][j] * f(table[col0+j][col])
       const int64_t jn = min((int64_t)BN, n_ent - col0);
       for (int j = 0; j < jn; ++j) {
         const float* crow = table + (col0 + j) * (int64_t)d;
         float cv[NC];
 #pragma unroll
         for (int c = 0; c < NC; ++c) {
-          int col = lane + 32 * c;
+          int col = slot_col<KIND, NC>(lane, c, d);
           cv[c] = col < d ? __ldg(crow + col) : 0.f;
         }
 #pragma unroll
         for (int a = 0; a < 8; ++a) {
           float gv = sm.g[warp * 8 + a][j];
+          if constexpr (kL1) {
+            l1_pair_step<KIND, NC>(gv, own[a], cv, out_acc[a]);
+          } else {
+            if constexpr (kL2) gsum[a] += gv;
 #pragma unroll
-          for (int c = 0; c < NC; ++c) out_acc[a][c] = fmaf(gv, cv[c], out_acc[a][c]);
+            for (int c = 0; c < NC; ++c) out_acc[a][c] = fmaf(gv, cv[c], out_acc[a][c]);
+          }
         }
       }
     } else {
-      // dTable[entities of warp][cols of lane] += sum_r G[r][ent] * Q[row0+r][col]
+      // dTable[entities of warp][cols of lane] += sum_r G[r][ent] * f(Q[row0+r][col])
       const int64_t rn = min((int64_t)BM, B - row0);
       for (int r = 0; r < rn; ++r) {
         const float* qrow = Q + (row0 + r) * (int64_t)d;
         float qv[NC];
 #pragma unroll
         for (int c = 0; c < NC; ++c) {
-          int col = lane + 32 * c;
+          int col = slot_col<KIND, NC>(lane, c, d);
           qv[c] = col < d ? __ldg(qrow + col) : 0.f;
         }
 #pragma unroll
         for (int a = 0; a < 8; ++a) {
           float gv = sm.g[r][warp * 8 + a];
+          if constexpr (kL1) {
+            l1_pair_step<KIND, NC>(gv, own[a], qv, out_acc[a]);
+          } else {
+            if constexpr (kL2) gsum[a] += gv;
 #pragma unroll
-          for (int c = 0; c < NC; ++c) out_acc[a][c] = fmaf(gv, qv[c], out_acc[a][c]);
+            for (int c = 0; c < NC; ++c) out_acc[a][c] = fmaf(gv, qv[c], out_acc[a][c]);
+          }
         }
       }
     }
     __syncthreads();
+  }
+  if constexpr (kL2) {   // d/d own = own * sum G' - sum G' other
+#pragma unroll
+    for (int a = 0; a < 8; ++a)
+#pragma unroll
+      for (int c = 0; c < NC; ++c) {
+        const int col = lane + 32 * c;
+        const float ov = (col < d && own0 + a < n_own) ? __ldg(own_base + (own0 + a) * d + col) : 0.f;
+        out_acc[a][c] = fmaf(ov, gsum[a], -out_acc[a][c]);
+      }
   }
   if (MODE == 0) {
     float* dst = out + ((int64_t)blockIdx.x * B) * d;  // partial [chunk][B][d]
@@ -560,7 +650,7 @@ fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float
       if (r >= B) continue;
 #pragma unroll
       for (int c = 0; c < NC; ++c) {
-        int col = lane + 32 * c;
+        int col = slot_col<KIND, NC>(lane, c, d);
         if (col < d) dst[r * d + col] = out_acc[a][c];
       }
     }
@@ -571,7 +661,7 @@ fused_bwd_kernel(LossParams lp_in, const float* __restrict__ gscale, const float
       if (e >= n_ent) continue;
 #pragma unroll
       for (int c = 0; c < NC; ++c) {
-        int col = lane + 32 * c;
+        int col = slot_col<KIND, NC>(lane, c, d);
         if (col < d) out[e * d + col] += out_acc[a][c];
       }
     }
@@ -789,6 +879,87 @@ static TailWs carve_tail(void* ws, int64_t ws_bytes, int64_t B, int d) {
 }
 
 
+__global__ void label_weight_kernel(int loss, const int64_t* __restrict__ lab_off, int64_t B, float ls_keep,
+                                    float* __restrict__ tscale) {
+  int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (r >= B) return;
+  if (loss == KGEB_LOSS_BCE) { tscale[r] = ls_keep; return; }
+  int64_t n = lab_off[r + 1] - lab_off[r];  // KL: t = y / ||y||_1  (loss.py:211-213); one-hot for index labels
+  tscale[r] = n > 0 ? 1.f / (float)n : 0.f;
+}
+
+}  // extern "C"
+
+// fp32 CUDA-core forward statistics of every kind (kgeb_fused_fwd with KGEB_MATH_FP32, kgeb_fused_fwd_kind); B > 0
+template <int KIND>
+static int fused_fwd_fp32(const LossParams& lp, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,
+                          int64_t n_ent, const int64_t* lab_off, const int64_t* lab_col, float* rowstat, void* workspace,
+                          cudaStream_t st) {
+  const int64_t ntc = (n_ent + BN - 1) / BN, ntr = (B + BM - 1) / BM;
+  const int64_t chunks = pick_chunks(ntc < 1 ? 1 : ntc, ntr);
+  const int64_t tpc = ntc == 0 ? 1 : (ntc + chunks - 1) / chunks;
+  float* partial = reinterpret_cast<float*>(workspace);
+  dim3 grid((unsigned)chunks, (unsigned)ntr);
+  fused_fwd_kernel<KIND><<<grid, TT, 0, st>>>(lp, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, tpc, partial);
+  KGEB_LAUNCH_CHECK("fused_fwd");
+  fused_fwd_finalize<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(lp.loss, partial, B, chunks, rowstat);
+  KGEB_LAUNCH_CHECK("fused_fwd_finalize");
+  return KGEB_OK;
+}
+
+template <int KIND, int NC>
+static void launch_fused_bwd(const LossParams& lp, const float* grad_scale, const float* Q, int64_t B, int d,
+                             const float* table, int64_t e_lo, int64_t n_ent, const int64_t* lab_off,
+                             const int64_t* lab_col, const float* lse, const float* tscale, int64_t chunks, int64_t tpc,
+                             float* partial, float* dQ, float* dTable, cudaStream_t st) {
+  const int64_t ntc = (n_ent + BN - 1) / BN, ntr = (B + BM - 1) / BM;
+  size_t smem = sizeof(BwdSmem<NC>);
+  cudaFuncSetAttribute(fused_bwd_kernel<KIND, NC, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaFuncSetAttribute(fused_bwd_kernel<KIND, NC, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (dQ) {
+    dim3 g0((unsigned)chunks, (unsigned)ntr);
+    fused_bwd_kernel<KIND, NC, 0><<<g0, TT, smem, st>>>(lp, grad_scale, Q, B, d, table, e_lo, n_ent, lab_off, lab_col,
+                                                         lse, tscale, tpc, partial);
+    reduce_partials_kernel<<<(unsigned)((B * d + 255) / 256), 256, 0, st>>>(partial, chunks, B * (int64_t)d, dQ);
+  }
+  if (dTable && ntc > 0)
+    fused_bwd_kernel<KIND, NC, 1><<<(unsigned)ntc, TT, smem, st>>>(lp, grad_scale, Q, B, d, table, e_lo, n_ent, lab_off,
+                                                                    lab_col, lse, tscale, tpc, dTable);
+}
+
+// fp32 CUDA-core backward of every kind (kgeb_fused_bwd outside the bf16 tiles, kgeb_fused_bwd_kind); B > 0
+template <int KIND>
+static int fused_bwd_fp32(const LossParams& lp, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,
+                          int64_t n_ent, const int64_t* lab_off, const int64_t* lab_col, const float* lse,
+                          const float* grad_scale, float* dQ, float* dTable, int flags, void* workspace, cudaStream_t st) {
+  const int64_t ntc = (n_ent + BN - 1) / BN, ntr = (B + BM - 1) / BM;
+  const int64_t chunks = pick_chunks(ntc < 1 ? 1 : ntc, ntr);
+  const int64_t tpc = ntc == 0 ? 1 : (ntc + chunks - 1) / chunks;
+  float* partial = reinterpret_cast<float*>(workspace);
+  int64_t part_bytes = chunks * B * (int64_t)d * 4, stat_bytes = chunks * B * 16;
+  float* tscale = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) +
+                                           (((part_bytes > stat_bytes ? part_bytes : stat_bytes) + 255) / 256) * 256);
+  label_weight_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(lp.loss, lab_off, B, lp.ls_keep, tscale);
+  KGEB_LAUNCH_CHECK("label_weight");
+  if (dTable && (flags & KGEB_BWD_OVERWRITE_TABLE) && n_ent > 0)   // the fp32 tiles add: overwrite = clear first
+    cudaMemsetAsync(dTable, 0, (size_t)n_ent * d * 4, st);
+  // accumulator slots per lane: ceil(d / 32); ROT_L1 2 * ceil(d / 64), whole column pairs per lane
+  const int nc = KIND == KGEB_ROT_L1 ? 2 * ((d / 2 + 31) / 32) : (d + 31) / 32;
+#define LAUNCH_BWD(NC)                                                                                                    \
+  launch_fused_bwd<KIND, NC>(lp, grad_scale, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, lse, tscale, chunks, tpc, \
+                             partial, dQ, dTable, st)
+  if constexpr (KIND == KGEB_ROT_L1) {
+    if (nc <= 2) LAUNCH_BWD(2); else if (nc <= 4) LAUNCH_BWD(4); else LAUNCH_BWD(8);
+  } else {
+    if (nc <= 1) LAUNCH_BWD(1); else if (nc <= 2) LAUNCH_BWD(2); else if (nc <= 4) LAUNCH_BWD(4); else LAUNCH_BWD(8);
+  }
+#undef LAUNCH_BWD
+  KGEB_LAUNCH_CHECK("fused_bwd");
+  return KGEB_OK;
+}
+
+extern "C" {
+
 static int check_fused(int loss, int d, float ls, const void* Q, const void* table, int64_t e_lo, int64_t e_hi) {
   KGEB_REQUIRE(loss == KGEB_LOSS_KL || loss == KGEB_LOSS_BCE, "fused: unknown loss %d", loss);
   KGEB_REQUIRE(Q && table && d > 0 && e_hi >= e_lo && e_lo >= 0, "fused: bad arguments");
@@ -821,25 +992,7 @@ int kgeb_fused_fwd(int loss, int math, const float* Q, int64_t B, int d, const f
     return tc_fused_fwd(loss, math, Q, tail.qb, B, d, table, table_bf16, e_lo, n_ent, lab_off, lab_col, nnz, lp.ls_keep,
                         lp.ls_add, offset, rowstat, workspace, tail.usable, st);
   }
-  const int64_t ntc = (n_ent + BN - 1) / BN, ntr = (B + BM - 1) / BM;
-  const int64_t chunks = pick_chunks(ntc < 1 ? 1 : ntc, ntr);
-  const int64_t tpc = ntc == 0 ? 1 : (ntc + chunks - 1) / chunks;
-  float* partial = reinterpret_cast<float*>(workspace);
-  dim3 grid((unsigned)chunks, (unsigned)ntr);
-  fused_fwd_kernel<<<grid, TT, 0, st>>>(lp, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, tpc, partial);
-  KGEB_LAUNCH_CHECK("fused_fwd");
-  fused_fwd_finalize<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(loss, partial, B, chunks, rowstat);
-  KGEB_LAUNCH_CHECK("fused_fwd_finalize");
-  return KGEB_OK;
-}
-
-__global__ void label_weight_kernel(int loss, const int64_t* __restrict__ lab_off, int64_t B, float ls_keep,
-                                    float* __restrict__ tscale) {
-  int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (r >= B) return;
-  if (loss == KGEB_LOSS_BCE) { tscale[r] = ls_keep; return; }
-  int64_t n = lab_off[r + 1] - lab_off[r];  // KL: t = y / ||y||_1  (loss.py:211-213); one-hot for index labels
-  tscale[r] = n > 0 ? 1.f / (float)n : 0.f;
+  return fused_fwd_fp32<KGEB_DOT>(lp, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, rowstat, workspace, st);
 }
 
 int kgeb_fused_bwd_wait_tiles(void* stream) { return tc_wait_tiles(as_stream(stream)); }
@@ -957,13 +1110,6 @@ int kgeb_fused_bwd(int loss, int math, const float* Q, int64_t B, int d, const f
   KGEB_REQUIRE(workspace && workspace_bytes >= kgeb_fused_workspace_bytes(B, d, n_ent, nnz), "fused_bwd: workspace too small");
   LossParams lp{loss, 1.f - label_smoothing, label_smoothing > 0.f ? 1.f / (float)num_entities : 0.f, offset,
                 inv_batch};
-  const int64_t ntc = (n_ent + BN - 1) / BN, ntr = (B + BM - 1) / BM;
-  const int64_t chunks = pick_chunks(ntc < 1 ? 1 : ntc, ntr);
-  const int64_t tpc = ntc == 0 ? 1 : (ntc + chunks - 1) / chunks;
-  float* partial = reinterpret_cast<float*>(workspace);
-  int64_t part_bytes = chunks * B * (int64_t)d * 4, stat_bytes = chunks * B * 16;
-  float* tscale = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) +
-                                           (((part_bytes > stat_bytes ? part_bytes : stat_bytes) + 255) / 256) * 256);
   if (tc_bwd_supported(math, d)) {
     KGEB_REQUIRE(table_bf16, "fused_bwd(bf16): the bf16 mirror of the table is required (kgeb_to_bf16)");
     TailWs tail = carve_tail(workspace, workspace_bytes, B, d);
@@ -984,33 +1130,69 @@ int kgeb_fused_bwd(int loss, int math, const float* Q, int64_t B, int d, const f
                                           stream)))
     return rc;
   // KGEB_MATH_TF32 (an MN-major TF32 operand would need a second, differently swizzled copy of every tile) and
-  // dims outside the BF16 tile build use the fp32 CUDA-core tiles below
-  label_weight_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(loss, lab_off, B, lp.ls_keep, tscale);
-  KGEB_LAUNCH_CHECK("label_weight");
-  if (dTable && (flags & KGEB_BWD_OVERWRITE_TABLE) && n_ent > 0)   // the fp32 tiles add: overwrite = clear first
-    cudaMemsetAsync(dTable, 0, (size_t)n_ent * d * 4, st);
-  const int nc = (d + 31) / 32;
-#define LAUNCH_BWD(NC)                                                                                              \
-  {                                                                                                                 \
-    size_t smem = sizeof(BwdSmem<NC>);                                                                              \
-    cudaFuncSetAttribute(fused_bwd_kernel<NC, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
-    cudaFuncSetAttribute(fused_bwd_kernel<NC, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
-    if (dQ) {                                                                                                       \
-      dim3 g0((unsigned)chunks, (unsigned)ntr);                                                                     \
-      fused_bwd_kernel<NC, 0><<<g0, TT, smem, st>>>(lp, grad_scale, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, lse, tscale, \
-                                                     tpc, partial);                                                 \
-      reduce_partials_kernel<<<(unsigned)((B * d + 255) / 256), 256, 0, st>>>(partial, chunks, B * (int64_t)d, dQ); \
-    }                                                                                                               \
-    if (dTable && ntc > 0)                                                                                          \
-      fused_bwd_kernel<NC, 1><<<(unsigned)ntc, TT, smem, st>>>(lp, grad_scale, Q, B, d, table, e_lo, n_ent, lab_off, lab_col,   \
-                                                                lse, tscale, tpc, dTable);                          \
-  }
-  if (nc <= 1) LAUNCH_BWD(1) else if (nc <= 2) LAUNCH_BWD(2) else if (nc <= 4) LAUNCH_BWD(4) else LAUNCH_BWD(8)
-#undef LAUNCH_BWD
-  KGEB_LAUNCH_CHECK("fused_bwd");
+  // dims outside the BF16 tile build use the fp32 CUDA-core tiles
+  return fused_bwd_fp32<KGEB_DOT>(lp, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, lse, grad_scale, dQ, dTable, flags,
+                                  workspace, st);
+}
+
+
+// The distance kinds on the fp32 CUDA-core tiles (kgeb_fused_fwd_kind / kgeb_fused_bwd_kind): scores are distances, not
+// a GEMM, so there is no tensor-tile or flash form.  Argument errors first, then check_fused's refusals.
+static int check_kind(int kind, int d) {
+  KGEB_REQUIRE(kind >= KGEB_DOT && kind <= KGEB_ROT_L2, "fused: unknown kind %d", kind);
+  KGEB_REQUIRE(!(kind >= KGEB_ROT_L1) || (d % 2 == 0), "RotatE requires embeddings of even dimensionality");
   return KGEB_OK;
 }
 
+int kgeb_fused_fwd_kind(int kind, int loss, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,
+                        int64_t e_hi, int64_t num_entities, const int64_t* lab_off, const int64_t* lab_col, int64_t nnz,
+                        float label_smoothing, float offset, float* rowstat, void* workspace, int64_t workspace_bytes,
+                        void* stream) {
+  if (kind == KGEB_DOT)
+    return kgeb_fused_fwd(loss, KGEB_MATH_FP32, Q, B, d, table, e_lo, e_hi, num_entities, lab_off, lab_col, nnz,
+                          label_smoothing, offset, nullptr, rowstat, workspace, workspace_bytes, stream);
+  int rc = check_kind(kind, d);
+  if (rc) return rc;
+  if ((rc = check_fused(loss, d, label_smoothing, Q, table, e_lo, e_hi))) return rc;
+  KGEB_REQUIRE(rowstat, "fused_fwd_kind: rowstat is NULL");
+  const int64_t n_ent = e_hi - e_lo;
+  if (B == 0) return KGEB_OK;
+  KGEB_REQUIRE(workspace && workspace_bytes >= kgeb_fused_workspace_bytes(B, d, n_ent, nnz),
+               "fused_fwd_kind: workspace too small");
+  LossParams lp{loss, 1.f - label_smoothing, label_smoothing > 0.f ? 1.f / (float)num_entities : 0.f, offset, 1.f};
+  cudaStream_t st = as_stream(stream);
+  DISPATCH_KIND(kind, return fused_fwd_fp32<K_>(lp, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, rowstat, workspace, st));
+  return KGEB_OK;
+}
+
+int kgeb_fused_bwd_kind(int kind, int loss, const float* Q, int64_t B, int d, const float* table, int64_t e_lo,
+                        int64_t e_hi, int64_t num_entities, const int64_t* lab_off, const int64_t* lab_col, int64_t nnz,
+                        float label_smoothing, float offset, const float* lse, float inv_batch, const float* grad_scale,
+                        float* dQ, float* dTable, int flags, void* workspace, int64_t workspace_bytes, void* stream) {
+  if (kind == KGEB_DOT)
+    return kgeb_fused_bwd(loss, KGEB_MATH_FP32, Q, B, d, table, e_lo, e_hi, num_entities, lab_off, lab_col, nnz, nullptr,
+                          label_smoothing, offset, lse, inv_batch, grad_scale, nullptr, dQ, dTable, nullptr, flags,
+                          workspace, workspace_bytes, stream);
+  int rc = check_kind(kind, d);
+  if (rc) return rc;
+  if ((rc = check_fused(loss, d, label_smoothing, Q, table, e_lo, e_hi))) return rc;
+  KGEB_REQUIRE(loss != KGEB_LOSS_KL || lse, "fused_bwd_kind: KL needs the per-row log-sum-exp");
+  KGEB_REQUIRE((flags & ~KGEB_BWD_OVERWRITE_TABLE) == 0, "fused_bwd_kind: unknown flags %d", flags);
+  KGEB_REQUIRE(lab_off && lab_col, "fused_bwd_kind: label CSR is NULL");
+  const int64_t n_ent = e_hi - e_lo;
+  cudaStream_t st = as_stream(stream);
+  if (B == 0) {   // no rows: the gradient of an overwritten table is all zeros
+    if (dTable && (flags & KGEB_BWD_OVERWRITE_TABLE) && n_ent > 0) cudaMemsetAsync(dTable, 0, (size_t)n_ent * d * 4, st);
+    return KGEB_OK;
+  }
+  KGEB_REQUIRE(workspace && workspace_bytes >= kgeb_fused_workspace_bytes(B, d, n_ent, nnz),
+               "fused_bwd_kind: workspace too small");
+  LossParams lp{loss, 1.f - label_smoothing, label_smoothing > 0.f ? 1.f / (float)num_entities : 0.f, offset,
+                inv_batch};
+  DISPATCH_KIND(kind, return fused_bwd_fp32<K_>(lp, Q, B, d, table, e_lo, n_ent, lab_off, lab_col, lse, grad_scale, dQ,
+                                                dTable, flags, workspace, st));
+  return KGEB_OK;
+}
 
 int kgeb_fused_flash_fwd(const float* Q, int64_t B, int d, const float* table, int64_t e_lo, int64_t e_hi,
                          int64_t num_entities, const int64_t* lab_off, const int64_t* lab_col, int64_t nnz,

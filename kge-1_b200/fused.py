@@ -1,8 +1,8 @@
 """Fused all-entity score + loss (forward and backward) and fused filtered rank counting.
 
 `AllEntityLoss` replaces the reference's  scores = model.score_sp/po(...) ; loss(scores, labels) / batch_size ;
-.backward()  chain (train.py:732-750, 1040-1057 with loss.py:137-159, 192-213) for the DOT scorers:
-the [B, E] score matrix is never written; labels are a CSR over the batch rows.  With an entity-sharded
+.backward()  chain (train.py:732-750, 1040-1057 with loss.py:137-159, 192-213) for the DOT scorers and, on the fp32
+CUDA-core tiles, for TransE and RotatE (`kind`): the [B, E] score matrix is never written; labels are a CSR over the batch rows.  With an entity-sharded
 table (`shard`), per-row statistics and the query gradient are all-reduced over the process group
 (SURVEY.md 8e); integer rank counts are exact under sharding.
 """
@@ -68,11 +68,19 @@ def combine_rowstats(rowstat: torch.Tensor, loss: int, shard: Shard) -> torch.Te
     return out
 
 
-def fused_rowstats(q, table, lab_off, lab_col, loss, label_smoothing, offset, math, shard: Shard) -> torch.Tensor:
+def fused_rowstats(q, table, lab_off, lab_col, loss, label_smoothing, offset, math, shard: Shard,
+                   kind: int = lib.DOT) -> torch.Tensor:
+    """Per-row forward statistics [B, 4] of this shard; a distance `kind` runs the fp32 tiles whatever `math` says."""
     b, d = q.shape
     rowstat = torch.empty(b, 4, dtype=torch.float32, device=q.device)
     n_ent = shard.e_hi - shard.e_lo
     ws = ops._workspace(q.device, lib.load().kgeb_fused_workspace_bytes(b, d, n_ent, lab_col.numel()))
+    if kind != lib.DOT:
+        lib.call("kgeb_fused_fwd_kind", kind, loss, lib.f32(q, "queries"), b, d, lib.f32(table, "table"), shard.e_lo,
+                 shard.e_hi, shard.num_entities, lib.i64(lab_off, "label offsets"), lib.i64(lab_col, "label columns"),
+                 lab_col.numel(), float(label_smoothing), float(offset), rowstat.data_ptr(), ws.data_ptr(), ws.numel(),
+                 lib.stream_ptr(q))
+        return rowstat
     lib.call("kgeb_fused_fwd", loss, math, lib.f32(q, "queries"), b, d, lib.f32(table, "table"), shard.e_lo,
              shard.e_hi, shard.num_entities, lib.i64(lab_off, "label offsets"), lib.i64(lab_col, "label columns"),
              lab_col.numel(), float(label_smoothing), float(offset), _mirror_ptr(table, math, b, d), rowstat.data_ptr(), ws.data_ptr(),
@@ -143,21 +151,31 @@ def rows_loss(rowstat: torch.Tensor, lab_off: torch.Tensor, loss: int, label_smo
 
 def fused_backward(q, table, lab_off, lab_col, loss, label_smoothing, offset, lse, inv_batch, grad_scale, math,
                    shard: Shard, d_table: Optional[torch.Tensor], want_dq: bool = True,
-                   lab_perm: Optional[torch.Tensor] = None, overwrite: bool = False) -> Optional[torch.Tensor]:
+                   lab_perm: Optional[torch.Tensor] = None, overwrite: bool = False,
+                   kind: int = lib.DOT) -> Optional[torch.Tensor]:
     """dQ (returned, all-reduced over shards) and d_table += G^T Q for the rows of this shard (`overwrite`: d_table = ...,
     KGEB_BWD_OVERWRITE_TABLE -- the buffer need not be cleared).  lab_perm (int32, optional): stable argsort of lab_col
-    from the collate (spares the device sort of the label scatter)."""
+    from the collate (spares the device sort of the label scatter).  A distance `kind` runs the fp32 tiles."""
     b, d = q.shape
     n_ent = shard.e_hi - shard.e_lo
     dq = torch.empty(b, d, dtype=torch.float32, device=q.device) if want_dq else None
     ws = ops._workspace(q.device, lib.load().kgeb_fused_workspace_bytes(b, d, n_ent, lab_col.numel()))
-    lib.call("kgeb_fused_bwd", loss, math, lib.f32(q, "queries"), b, d, lib.f32(table, "table"), shard.e_lo,
-             shard.e_hi, shard.num_entities, lib.i64(lab_off), lib.i64(lab_col), lab_col.numel(),
-             None if lab_perm is None else lab_perm.data_ptr(), float(label_smoothing), float(offset), None if lse is None else lib.f32(lse, "lse"), float(inv_batch),
-             None if grad_scale is None else lib.f32(grad_scale, "grad scale"), _mirror_ptr(table, math, b, d),
-             None if dq is None else dq.data_ptr(), None if d_table is None else lib.f32(d_table, "table gradient"),
-             None, lib.BWD_OVERWRITE_TABLE if (overwrite and d_table is not None) else 0, ws.data_ptr(), ws.numel(),
-             lib.stream_ptr(q))
+    if kind != lib.DOT:
+        lib.call("kgeb_fused_bwd_kind", kind, loss, lib.f32(q, "queries"), b, d, lib.f32(table, "table"), shard.e_lo,
+                 shard.e_hi, shard.num_entities, lib.i64(lab_off), lib.i64(lab_col), lab_col.numel(),
+                 float(label_smoothing), float(offset), None if lse is None else lib.f32(lse, "lse"), float(inv_batch),
+                 None if grad_scale is None else lib.f32(grad_scale, "grad scale"), None if dq is None else dq.data_ptr(),
+                 None if d_table is None else lib.f32(d_table, "table gradient"),
+                 lib.BWD_OVERWRITE_TABLE if (overwrite and d_table is not None) else 0, ws.data_ptr(), ws.numel(),
+                 lib.stream_ptr(q))
+    else:
+        lib.call("kgeb_fused_bwd", loss, math, lib.f32(q, "queries"), b, d, lib.f32(table, "table"), shard.e_lo,
+                 shard.e_hi, shard.num_entities, lib.i64(lab_off), lib.i64(lab_col), lab_col.numel(),
+                 None if lab_perm is None else lab_perm.data_ptr(), float(label_smoothing), float(offset), None if lse is None else lib.f32(lse, "lse"), float(inv_batch),
+                 None if grad_scale is None else lib.f32(grad_scale, "grad scale"), _mirror_ptr(table, math, b, d),
+                 None if dq is None else dq.data_ptr(), None if d_table is None else lib.f32(d_table, "table gradient"),
+                 None, lib.BWD_OVERWRITE_TABLE if (overwrite and d_table is not None) else 0, ws.data_ptr(), ws.numel(),
+                 lib.stream_ptr(q))
     if dq is not None and n_ent == 0:
         dq.zero_()
     if dq is not None and shard.distributed:
@@ -170,9 +188,9 @@ class AllEntityLoss(torch.autograd.Function):
     (Summing the rows gives the reference's batch loss; row sub-sums give its per-query-type values.)"""
 
     @staticmethod
-    def forward(ctx, q, table, lab_off, lab_col, loss, label_smoothing, offset, batch_size, math, shard):
+    def forward(ctx, q, table, lab_off, lab_col, loss, label_smoothing, offset, batch_size, math, shard, kind):
         qd, td = q.detach().contiguous(), table.detach()
-        flash = flash_supported(loss, math, qd.shape[1], label_smoothing) and qd.shape[0] > 0
+        flash = kind == lib.DOT and flash_supported(loss, math, qd.shape[1], label_smoothing) and qd.shape[0] > 0
         if flash:
             local, o_sum, status = flash_forward(qd, td, lab_off, lab_col, shard)
             if shard.distributed:      # every rank must take the same path
@@ -183,16 +201,16 @@ class AllEntityLoss(torch.autograd.Function):
         else:
             local = o_sum = None
             rowstat = combine_rowstats(
-                fused_rowstats(qd, td, lab_off, lab_col, loss, label_smoothing, offset, math, shard), loss, shard)
+                fused_rowstats(qd, td, lab_off, lab_col, loss, label_smoothing, offset, math, shard, kind), loss, shard)
         per_row, lse = rows_loss(rowstat, lab_off, loss, label_smoothing, shard.num_entities)
         ctx.save_for_backward(qd, td, lab_off, lab_col, lse, local, o_sum)
-        ctx.cfg = (loss, label_smoothing, offset, 1.0 / batch_size, math, shard)
+        ctx.cfg = (loss, label_smoothing, offset, 1.0 / batch_size, math, shard, kind)
         return per_row / batch_size
 
     @staticmethod
     def backward(ctx, g):
         qd, td, lab_off, lab_col, lse, local, o_sum = ctx.saved_tensors
-        loss, ls, offset, inv_batch, math, shard = ctx.cfg
+        loss, ls, offset, inv_batch, math, shard, kind = ctx.cfg
         # a table-sized gradient: written once by the kernels (no zero-fill pass) when this rank scores every row
         whole = shard.e_lo == 0 and shard.e_hi == td.shape[0]
         d_table = None
@@ -206,15 +224,18 @@ class AllEntityLoss(torch.autograd.Function):
                                want_dq=False, overwrite=whole)
         else:
             dq = fused_backward(qd, td, lab_off, lab_col, loss, ls, offset, lse, inv_batch, gs, math, shard, d_table,
-                                want_dq=ctx.needs_input_grad[0], overwrite=whole)
-        return dq, d_table, None, None, None, None, None, None, None, None
+                                want_dq=ctx.needs_input_grad[0], overwrite=whole, kind=kind)
+        return dq, d_table, None, None, None, None, None, None, None, None, None
 
 
 def all_entity_loss(q, table, lab_off, lab_col, loss: int, batch_size: int, label_smoothing: float = 0.0,
-                    offset: float = 0.0, math: int = lib.MATH_FP32, shard: Optional[Shard] = None) -> torch.Tensor:
+                    offset: float = 0.0, math: int = lib.MATH_FP32, shard: Optional[Shard] = None,
+                    kind: int = lib.DOT) -> torch.Tensor:
+    """`kind`: pair kind of the scorer (lib.DOT, or TransE / RotatE's distance kinds, which run the fp32 CUDA-core
+    tiles with no flash pass whatever `math` says)."""
     shard = shard or Shard.full(table.shape[0])
     return AllEntityLoss.apply(q, table, lab_off, lab_col, loss, float(label_smoothing), float(offset),
-                               int(batch_size), math, shard)
+                               int(batch_size), math, shard, int(kind))
 
 
 # ---------------------------------------------------------------------------------------------

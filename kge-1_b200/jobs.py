@@ -97,7 +97,8 @@ class TrainingJob:
         return res
 
     def _use_fused(self) -> bool:
-        return self.fused_path and self.model.get_scorer().kind == lib.DOT and self.model.get_s_embedder().dim <= 256
+        """Fused score + loss kernels: every pair kind (DOT scorers, TransE, RotatE) up to d = 256."""
+        return self.fused_path and self.model.get_s_embedder().dim <= 256
 
 
 class TrainingJob1vsAll(TrainingJob):
@@ -114,7 +115,8 @@ class TrainingJob1vsAll(TrainingJob):
             lab_off = torch.arange(2 * b + 1, dtype=torch.int64, device=self.device)
             lab_col = torch.cat((triples[:, 2], triples[:, 0])).long().contiguous()
             rows = fused.all_entity_loss(q, self.model.get_o_embedder().embed_all(), lab_off, lab_col,
-                                         self.loss.kind, b, 0.0, self.loss.offset, self.math_mode, self.shard)
+                                         self.loss.kind, b, 0.0, self.loss.offset, self.math_mode, self.shard,
+                                         kind=self.model.get_scorer().kind)
             loss_value = rows.sum()
             loss_value.backward()
             return ProcessBatchResult(loss_value.item(), b)
@@ -143,7 +145,7 @@ class TrainingJobKvsAll(TrainingJob):
     def enable_graph_step(self, batch_size: int, nnz_max: int, use_graph: bool = True, dp_group=None,
                           dp_p2p: bool = False):
         """Routes step() through FusedAllEntityStepper for batches of exactly `batch_size` queries with at most
-        `nnz_max` labels (no autograd, one CUDA-graph replay per step).  Needs the DOT scorers and dense Adagrad;
+        `nnz_max` labels (no autograd, one CUDA-graph replay per step).  Needs dense Adagrad (TransE / RotatE: one GPU);
         unweighted Lp penalties are folded into the Adagrad kernels (the toy config's regularize_weight)."""
         from .trainer import FusedAllEntityStepper
         if any(e.normalize_p > 0 for e in (self.model.get_s_embedder(), self.model.get_p_embedder())):
@@ -339,7 +341,8 @@ class TrainingJobKvsAll(TrainingJob):
                     parts.append(self.model.queries(lib._PO, qs[n_sp:, 1], qs[n_sp:, 0]))
             q = torch.cat(parts) if len(parts) > 1 else parts[0]
             rows = fused.all_entity_loss(q, self.model.get_o_embedder().embed_all(), lab_off, lab_col, self.loss.kind,
-                                         b, self.label_smoothing, self.loss.offset, self.math_mode, self.shard)
+                                         b, self.label_smoothing, self.loss.offset, self.math_mode, self.shard,
+                                         kind=self.model.get_scorer().kind)
             total = rows.sum()
             total.backward()
             # train.py:747 reports the value of the last non-empty query type only

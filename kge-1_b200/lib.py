@@ -42,6 +42,8 @@ SIGNATURES = {
     "kgeb_score_all_bwd": [_i, _p, _l, _i, _p, _p, _i, _l, _p, _p, _l, _l, _p, _p, _p],
     "kgeb_fused_fwd": [_i, _i, _p, _l, _i, _p, _l, _l, _l, _p, _p, _l, _f, _f, _p, _p, _p, _l, _p],
     "kgeb_fused_bwd": [_i, _i, _p, _l, _i, _p, _l, _l, _l, _p, _p, _l, _p, _f, _f, _p, _f, _p, _p, _p, _p, _p, _i, _p, _l, _p],
+    "kgeb_fused_fwd_kind": [_i, _i, _p, _l, _i, _p, _l, _l, _l, _p, _p, _l, _f, _f, _p, _p, _l, _p],
+    "kgeb_fused_bwd_kind": [_i, _i, _p, _l, _i, _p, _l, _l, _l, _p, _p, _l, _f, _f, _p, _f, _p, _p, _p, _i, _p, _l, _p],
     "kgeb_fused_flash_fwd": [_p, _l, _i, _p, _l, _l, _l, _p, _p, _l, _p, _p, _p, _p, _p, _l, _p],
     "kgeb_fused_flash_dq": [_p, _l, _i, _p, _l, _l, _p, _p, _l, _p, _p, _f, _p, _p, _p, _p, _l, _p],
     "kgeb_fused_label_rows": [_i, _p, _l, _i, _p, _l, _l, _p, _p, _l, _p, _f, _f, _p, _p, _p, _l, _p],

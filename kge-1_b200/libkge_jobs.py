@@ -5,7 +5,7 @@ unmodified job code (kge/job/train.py, kge/job/entity_ranking.py) reaches the FU
 Three levels, all installed from `model.prepare_job(job)` (called by every job, train.py:474, entity_ranking.py:50;
 `Job._is_prepared` is never set, job.py:52,153-154, so installation is idempotent per job object):
 
-1. **fused loss** (any TrainingJob1vsAll / TrainingJobKvsAll with `train.loss` kl | bce and a DOT scorer).  The job keeps
+1. **fused loss** (any TrainingJob1vsAll / TrainingJobKvsAll with `train.loss` kl | bce; TransE / RotatE on fp32 tiles).  The job keeps
    running its own `_process_batch` (train.py:679-756, 1032-1062).  `model.score_sp / score_po` return a `LazyScores`
    handle instead of the `[B, E]` matrix; `job.loss` (a plain attribute, train.py:67) is wrapped by `FusedKgeLoss`, which
    recognises the handle and calls the fused score+loss kernels (kgeb_fused_fwd / kgeb_fused_bwd behind an
@@ -52,7 +52,7 @@ class LazyScores:
         self.kind, self.q, self.table, self.math_mode = kind, q, table, math_mode
 
     def materialize(self) -> torch.Tensor:
-        m = self.math_mode if self.math_mode == lib.MATH_TF32 else lib.MATH_FP32
+        m = self.math_mode if (self.math_mode == lib.MATH_TF32 and self.kind == lib.DOT) else lib.MATH_FP32
         return ops.score_all(self.kind, self.q, self.table, m)
 
     @property
@@ -100,13 +100,13 @@ class FusedKgeLoss:
             return self._inner(scores, labels, **kwargs)
         ls = float(getattr(self._job, "label_smoothing", 0.0) or 0.0) if labels.dim() == 2 else 0.0
         d = scores.q.shape[1]
-        if scores.kind != lib.DOT or d > 256 or (self.kind == lib.LOSS_KL and ls > 0.0 and labels.dim() == 2):
+        if d > 256 or (self.kind == lib.LOSS_KL and ls > 0.0 and labels.dim() == 2):
             return self._inner(scores.materialize(), labels, **kwargs)
         n, e = scores.q.shape[0], scores.table.shape[0]
         lab_off, lab_col = labels_to_csr(labels, n, ls, e)
         # batch_size = 1: the reference's losses return the un-normalised sum, the caller divides (train.py:745,1042)
         rows = fused.all_entity_loss(scores.q, scores.table, lab_off, lab_col, self.kind, 1, ls, self.offset,
-                                     scores.math_mode)
+                                     scores.math_mode, kind=scores.kind)
         return rows.sum()
 
 
@@ -256,7 +256,7 @@ def prepare_training_job(job, model, base: str, options: dict, reciprocal: bool 
     if not isinstance(job, (TrainingJob1vsAll, TrainingJobKvsAll)):
         return                                  # negative sampling: score_spo is the fused gather+score kernel already
     name = job.config.get("train.loss")
-    if name not in ("kl", "bce") or model.get_scorer()._impl.kind != lib.DOT:
+    if name not in ("kl", "bce"):
         return
     loss_kind = lib.LOSS_KL if name == "kl" else lib.LOSS_BCE
     offset = float(job.config.get("train.loss_arg")) if name == "bce" else 0.0

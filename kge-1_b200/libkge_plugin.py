@@ -74,11 +74,10 @@ def register():
 
     def _lazy_scores(self) -> bool:
         """score_sp / score_po hand out a LazyScores handle only inside a training job whose loss was wrapped by
-        FusedKgeLoss (libkge_jobs.prepare_training_job), in training mode with autograd on, for the DOT scorers,
-        without embedder dropout (lookup_embedder.py:97-100 applies it to the whole table)."""
+        FusedKgeLoss (libkge_jobs.prepare_training_job), in training mode with autograd on (every scorer: the DOT
+        scorers, TransE and RotatE), without embedder dropout (lookup_embedder.py:97-100 applies it to the whole table)."""
         return (getattr(self, "_b200_lazy_jobs", 0) > 0 and self.training and torch.is_grad_enabled()
-                and self._scorer._impl.kind == _lib.DOT and self._entity_embedder.dropout.p == 0
-                and self._relation_embedder.dropout.p == 0)
+                and self._entity_embedder.dropout.p == 0 and self._relation_embedder.dropout.p == 0)
 
     def make(base):
         class Model(RefKgeModel):
@@ -118,13 +117,13 @@ def register():
             def score_sp(self, s, p, o=None):
                 if o is None and self._b200_lazy():
                     q = _ops.query_build(base, _lib.SP_, self.get_s_embedder().embed(s), self.get_p_embedder().embed(p))
-                    return _jobs.LazyScores(_lib.DOT, q, self.get_o_embedder()._embeddings.weight, self._b200_math)
+                    return _jobs.LazyScores(self._scorer._impl.kind, q, self.get_o_embedder()._embeddings.weight, self._b200_math)
                 return super().score_sp(s, p, o)
 
             def score_po(self, p, o, s=None):
                 if s is None and self._b200_lazy():
                     q = _ops.query_build(base, _lib._PO, self.get_o_embedder().embed(o), self.get_p_embedder().embed(p))
-                    return _jobs.LazyScores(_lib.DOT, q, self.get_s_embedder()._embeddings.weight, self._b200_math)
+                    return _jobs.LazyScores(self._scorer._impl.kind, q, self.get_s_embedder()._embeddings.weight, self._b200_math)
                 return super().score_po(p, o, s)
 
             def prepare_job(self, job, **kwargs):
@@ -162,14 +161,14 @@ def register():
         def score_sp(self, s, p, o=None):
             if o is None and self._b200_lazy():
                 q = _ops.query_build(self._b200_base, _lib.SP_, self.get_s_embedder().embed(s), self.get_p_embedder().embed(p))
-                return _jobs.LazyScores(_lib.DOT, q, self.get_o_embedder()._embeddings.weight, self._b200_math)
+                return _jobs.LazyScores(self._scorer._impl.kind, q, self.get_o_embedder()._embeddings.weight, self._b200_math)
             return super().score_sp(s, p, o)
 
         def score_po(self, p, o, s=None):
             if s is None and self._b200_lazy():
                 p_inv = self.get_p_embedder().embed(p + self.dataset.num_relations())
                 q = _ops.query_build(self._b200_base, _lib.SP_, self.get_o_embedder().embed(o), p_inv)
-                return _jobs.LazyScores(_lib.DOT, q, self.get_s_embedder()._embeddings.weight, self._b200_math)
+                return _jobs.LazyScores(self._scorer._impl.kind, q, self.get_s_embedder()._embeddings.weight, self._b200_math)
             return super().score_po(p, o, s)
 
         def prepare_job(self, job, **kwargs):

@@ -209,9 +209,15 @@ class FusedAllEntityStepper:
         `reciprocal`: the model is a reciprocal relations model (2 R relation rows).  Every query of the step is an sp_
         query: the _po queries of a batch arrive as sp_ rows on relation p + R -- built so by kgeb_onevsall_batch_build_inv
         (onevsall_triples) or by the caller (`kvsall_rows(..., inv_rel_offset=R)` for set_inputs / pack_host_batch).
-        Kernels, launches and the update are those of the plain step on a 2 R-row relation table."""
-        if model.get_scorer().kind != lib.DOT:
-            raise NotImplementedError("the fused all-entity step serves the DOT scorers")
+        Kernels, launches and the update are those of the plain step on a 2 R-row relation table.
+        TransE / RotatE (distance kinds) run on one GPU with fp32 arithmetic whatever `math_mode` says: the fp32 tile
+        kernels of kgeb_fused_fwd_kind / kgeb_fused_bwd_kind in the two-buffer flow, no bf16 mirror, flash pass or
+        fused table update."""
+        self.kind = model.get_scorer().kind
+        if self.kind != lib.DOT:
+            if dp_group is not None or (shard is not None and shard.distributed):
+                raise NotImplementedError("the fused all-entity step serves TransE / RotatE on one GPU only")
+            math_mode = lib.MATH_FP32
         self.inv_rel = _inverse_relation_offset(model, reciprocal, "FusedAllEntityStepper")
         _require_plain_model(model, "FusedAllEntityStepper", allow_penalty=True, allow_reciprocal=reciprocal)
         self.model, self.opt = model, optimizer
@@ -415,6 +421,11 @@ class FusedAllEntityStepper:
                      self.rowstat.data_ptr(), self.o_sum.data_ptr(), self.flash_status.data_ptr(), self.ws.data_ptr(),
                      self.ws.numel(), st)
             self.rowstat_local.copy_(self.rowstat)
+        elif self.kind != lib.DOT:
+            lib.call("kgeb_fused_fwd_kind", self.kind, self.loss_kind, self.Q.data_ptr(), self.rows, self.d,
+                     ent[sh.e_lo:sh.e_hi].data_ptr(), sh.e_lo, sh.e_hi, self.E, self.lab_off.data_ptr(),
+                     self.lab_col.data_ptr(), self.nnz_max, self.ls, self.offset, self.rowstat.data_ptr(),
+                     self.ws.data_ptr(), self.ws.numel(), st)
         elif not self._fused_stats_in_backward():
             lib.call("kgeb_fused_fwd", self.loss_kind, self.math, self.Q.data_ptr(), self.rows, self.d,
                      ent[sh.e_lo:sh.e_hi].data_ptr(), sh.e_lo, sh.e_hi, self.E, self.lab_off.data_ptr(),
@@ -495,6 +506,15 @@ class FusedAllEntityStepper:
         self.side.wait_stream(cur)
         if not sh.distributed:
             self.side.wait_stream(self.side2)     # cleared gradient buffers
+        if self.kind != lib.DOT:
+            dist_args = (self.kind, self.loss_kind, self.Q.data_ptr(), self.rows, self.d, ent.data_ptr(), 0, self.E,
+                         self.E, self.lab_off.data_ptr(), self.lab_col.data_ptr(), self.nnz_max, self.ls, self.offset,
+                         lse, 1.0 / self.global_batch, None)
+            with torch.cuda.stream(self.side):
+                lib.call("kgeb_fused_bwd_kind", *dist_args, None, self.g_ent.data_ptr(), 0, self.ws2.data_ptr(),
+                         self.ws2.numel(), lib.stream_ptr(self.ent))
+            lib.call("kgeb_fused_bwd_kind", *dist_args, self.dQ.data_ptr(), None, 0, self.ws.data_ptr(), self.ws.numel(), st)
+            return
         with torch.cuda.stream(self.side):
             lib.call("kgeb_fused_bwd", *common, None, self.g_ent[sh.e_lo:sh.e_hi].data_ptr(), None, 0, self.ws2.data_ptr(),
                      self.ws2.numel(), lib.stream_ptr(self.ent))
