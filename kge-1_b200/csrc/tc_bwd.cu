@@ -97,7 +97,6 @@ struct Params {
   float upd_clr, upd_eps;
   const float* upd_clr_dev;  // non-NULL: the rate is this device word, not upd_clr (read once per update warp)
   int stagger_clk;         // fused update: CTA b starts b * stagger_clk clocks late (see the producer warp of the v2 kernel)
-  int upd_debug;           // tuning only (KGEB_UPD_DEBUG): 1 = no loads of W / state, 2 = no stores, 4 = no arithmetic, 8 = no prefetch, 16 = no phase 2
 };
 
 // Per-row state of an epilogue thread over one job (one resident row = one TMEM lane).
@@ -603,7 +602,14 @@ constexpr int NG = 4;   // tiles in flight = S/G buffers = epilogue groups
 static_assert(128 * KGEB_UPD_REG_CTRL + 512 * KGEB_UPD_REG_EPI + 128 * KGEB_UPD_REG_UPD <= 768 * 80, "register pool of the CTA");
 __device__ __forceinline__ float sqrt_approx(float x) { float y; asm("sqrt.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-constexpr int UPD_THREADS = 128;   // fused update: one more warpgroup, warp 20 + p applies Adagrad to the box of column part p
+constexpr int UPD_THREADS = 128;   // fused update: one more warpgroup, warp 20 + q applies Adagrad to rows 32 q .. 32 q + 31
+// Each update warp streams W and the Adagrad state of its 32 rows through a two-stage ring of 32-row x 32-column fp32 boxes
+// (TMA, 128-byte swizzle; one W box + one state box per stage), in the shared memory the dTable kernel uses to stage its flush.
+constexpr int UPD_BOX_ROWS = 32;
+constexpr int UPD_BOX_BYTES = UPD_BOX_ROWS * 128;          // 4 KiB
+constexpr int UPD_STAGE_BYTES = 2 * UPD_BOX_BYTES;         // W box + state box
+constexpr int UPD_RING_BYTES = 2 * UPD_STAGE_BYTES;        // two stages per update warp
+static_assert((UPD_THREADS / 32) * UPD_RING_BYTES == EPQ * STAGE_BYTES, "the update rings fill the flush staging boxes exactly");
 
 template <int N>
 __device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
@@ -613,7 +619,7 @@ __device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.
 template <bool RES_IS_Q, int LOSS, bool HAS_RS, bool STATS, bool FLASH = false, bool UPD = false>
 __global__ void __launch_bounds__(NUM_THREADS + (UPD ? UPD_THREADS : 0), 1)
 tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant__ CUtensorMap tm_str,
-               const __grid_constant__ CUtensorMap tm_out, const Params p) {
+               const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ CUtensorMap tm_upd_state, const Params p) {
   static_assert(STR_ROWS == 64, "the v2 pipeline is laid out for 64-row streamed tiles");
   constexpr bool BF16 = true;
   extern __shared__ uint8_t smem_raw[];
@@ -624,7 +630,7 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
   constexpr int SLAB_K = Elem<BF16>::kSlabK, UMMA_K = Elem<BF16>::kUmmaK;
   uint8_t* res_smem = smem;                                         // [KS] slabs of 16 KiB
   uint8_t* str_smem = res_smem + (size_t)KS * RES_SLAB;             // [NSTR][KS] slabs of 8 KiB
-  uint8_t* stage_smem = str_smem + (size_t)NSTR * KS * STR_SLAB;    // !RES_IS_Q: flush staging boxes
+  uint8_t* stage_smem = str_smem + (size_t)NSTR * KS * STR_SLAB;    // !RES_IS_Q: flush staging boxes | UPD: W / state rings
   uint64_t* bars = reinterpret_cast<uint64_t*>(stage_smem + (RES_IS_Q ? 0 : EPQ * STAGE_BYTES));
   uint64_t* str_full = bars;                    // [MAX_STR]  TMA -> MMA1
   uint64_t* str_empty = bars + MAX_STR;         // [MAX_STR]  MMA2 done -> TMA
@@ -637,14 +643,13 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
   uint64_t* o_empty = o_full + 1;               // epilogue flushed -> MMA2
   uint64_t* a_full = o_empty + 1;               // a_tmem: epilogue copied the resident block to tensor memory -> MMA1
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(a_full + 1);
-  uint64_t* stage_full = a_full + 2;            // UPD [EPQ]: the part's epilogue warps staged the gradient box -> update warp
-  uint64_t* stage_free = stage_full + EPQ;      // UPD [EPQ]: update warp has consumed the staging box (and its slots)
+  uint64_t* upd_full = a_full + 2;              // UPD [4][2]: W and state box of update warp q's ring stage s arrived (TMA)
   // !RES_IS_Q, KL: the per-query exponent offsets of ALL streamed rows (the same for every job), 16-byte aligned
   float* kc_smem = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + 512);
   const float* kc_s = (!RES_IS_Q && LOSS == KGEB_LOSS_KL && p.colk_n > 0) ? kc_smem : nullptr;
   if (kc_s)
     for (int i = threadIdx.x; i < p.colk_n; i += blockDim.x) kc_smem[i] = p.colk[i];
-  int32_t* slot_s = reinterpret_cast<int32_t*>(kc_smem + p.colk_n_alloc);   // !RES_IS_Q: [EPQ][RES_ROWS] (fused update) + rate
+  float* clr_s = kc_smem + p.colk_n_alloc;     // !RES_IS_Q: the fused update's learning rate
   constexpr int TMEM_COLS = 512;
   constexpr uint32_t S_COL = 0;                 // NG S buffers of 64 columns; G aliases the first 32 columns of each
   constexpr uint32_t O_COL = NG * STR_ROWS;     // OUT accumulator: d <= 256 columns behind them
@@ -674,12 +679,9 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
       mbar_init(&buf_free[b], 1);
     }
     mbar_init(o_full, 1);
-    mbar_init(o_empty, NUM_EPI_THREADS / 32);
+    mbar_init(o_empty, UPD ? UPD_THREADS / 32 : NUM_EPI_THREADS / 32);   // UPD: the update warps read the accumulator
     if (UPD)
-      for (int b = 0; b < EPQ; ++b) {
-        mbar_init(&stage_full[b], 4);
-        mbar_init(&stage_free[b], 1);
-      }
+      for (int b = 0; b < 2 * UPD_THREADS / 32; ++b) mbar_init(&upd_full[b], 1);
     fence_barrier_init();
   }
   if (warp == 2) tmem_alloc<TMEM_COLS>(tmem_slot);
@@ -806,83 +808,138 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
       }
     }
   } else if (UPD && warp >= 4 + 4 * EPQ) {
-    // ================================ update warp of column part `part` ================================
-    // Adagrad on the gradient box the part's epilogue warps staged in shared memory (128 rows x 32 columns, 128-byte
-    // swizzle): a warp instruction covers 4 rows x 128 contiguous bytes of W / state.  Runs beside the next job's tiles:
-    // measured inside the epilogue warps (which the MUFU-bound tile loop needs), the same code added 1.6 ms to a 4.0 ms kernel.
+    // ================================ update warp of lane quadrant q ================================
+    // Flushes rows 32 q .. 32 q + 31 of every job (all d columns): it reads the accumulator from tensor memory itself, applies
+    // Adagrad in place in the shared-memory box the TMA brought W and the state into, and hands the box back to the TMA.  The
+    // epilogue warps (the MUFU-bound resource that sets the tile rate) do no flush work, and W / state bypass the LSU.
+    // Measured inside the epilogue warps, the update added 1.6 ms to a 4.0 ms kernel (DESIGN.md 4.1c).
     if (KGEB_UPD_REG_UPD >= 80) setmaxnreg_inc<KGEB_UPD_REG_UPD>(); else setmaxnreg_dec<KGEB_UPD_REG_UPD>();
-    const int part = warp - (4 + 4 * EPQ);
-    const int sub = lane >> 3, ck = lane & 7;   // row within a group of 4, 16-byte chunk of the 128-byte box row
+    const int q = warp & 3;                                // == warp % 4: the TMEM lane quadrant this warp may access
+    const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
     const bool live = p.upd_skip == nullptr || __ldg(p.upd_skip) == 0;
-    // the rate of this launch (device word of the _sched entry or the by-value parameter), read once at role start and kept
-    // in shared memory behind the slot arrays: held in a register across the loop below it made ptxas spill 20-28 more
-    // bytes in this kernel (-Xptxas -v); read from here the register and spill counts are those of the by-value kernel
-    float* clr_s = reinterpret_cast<float*>(slot_s + EPQ * RES_ROWS);
+    // the rate of this launch (device word of the _sched entry or the by-value parameter), read once at role start into a
+    // shared word and from there once per job
     if (lane == 0) *clr_s = p.upd_clr_dev ? __ldg(p.upd_clr_dev) : p.upd_clr;   // (every update warp stores the same value)
+    if (lane == 0) { tma_prefetch_desc(&tm_out); tma_prefetch_desc(&tm_upd_state); }
     __syncwarp();
-    const int nbox = (p.d + 31) / 32;
-    uint8_t* stage = stage_smem + (size_t)part * STAGE_BYTES;
-    uint32_t fphase = 0;
+    const int nbox = p.d / 32;                             // (the launcher requires d % 32 == 0)
+    uint8_t* ring = stage_smem + (size_t)q * UPD_RING_BYTES;
+    uint64_t* full = upd_full + 2 * q;
+    // Only boxes 0 and 1 are in the ring when the accumulator completes; waiting for the others before reading their columns
+    // would hold MMA2 of the next job behind an HBM round trip.  Where the tensor memory has room (d <= 128: the columns
+    // between the accumulator and the resident block), columns [64, d) are parked there first and the accumulator is released
+    // after box 1 has been read; otherwise after the last box.
+    const uint32_t park_col = O_COL + (uint32_t)p.d;
+    const bool park = nbox > 2 && park_col + (uint32_t)(p.d - 64) <= (a_tmem ? A_COL : (uint32_t)TMEM_COLS);
+    const int release_box = park ? 1 : nbox - 1;
+    auto load_box = [&](int box, uint32_t k, int32_t row0) {   // lane 0: box `box` into ring stage k & 1
+      uint8_t* st = ring + (size_t)(k & 1) * UPD_STAGE_BYTES;
+      mbar_expect_tx(&full[k & 1], (uint32_t)UPD_STAGE_BYTES);
+      tma_load_2d(st, &tm_out, box * 32, row0, &full[k & 1]);
+      tma_load_2d(st + UPD_BOX_BYTES, &tm_upd_state, box * 32, row0, &full[k & 1]);
+    };
+    uint32_t kb = 0, ophase = 0;                           // kb: boxes through the ring so far (stage kb & 1, phase kb >> 1)
     for (int64_t job = blockIdx.x; job < n_jobs; job += gridDim.x) {
       const int64_t rb = job % p.n_res_blocks;
-      for (int box = part; box < nbox; box += EPQ) {
-        mbar_wait(&stage_full[part], fphase);
-        fphase ^= 1;
-        const int col = box * 32 + ck * 4;
-        if (live && col < p.d && !(p.upd_debug & 16)) {
-#pragma unroll 1
-          for (int it = 0; it < 4; ++it) {
-            // 8 rows per round: 16 loads of 16 bytes in flight per lane (the warp has ~16 us per box and pays ~1 us of
-            // latency per round); the gradient and the slot are re-read from shared memory where they are consumed
-            float4 w8[8], s8[8];
-            const int r0 = it * 32 + sub;                                  // rows r0 + 4 i of the box
-            const size_t base = ((size_t)rb * RES_ROWS + r0) * p.d + col;  // element offset of row r0
-            const int64_t left = p.n_res - (rb * RES_ROWS + r0);           // row r0 + 4 i exists iff 4 i < left
+      const int64_t row0 = rb * RES_ROWS + q * 32, row = row0 + lane;
+      if (!live || row0 >= p.n_res) {                      // nothing to update: only release the accumulator
+        mbar_wait(o_full, ophase);
+        ophase ^= 1;
+        tc_fence_after();
+        tc_fence_before();
+        mbar_arrive_warp(o_empty);
+        continue;
+      }
+      // slot of this lane's row: -1 = update in place, >= 0 = touched (gradient to upd_gbuf[slot]), -2 = past the table
+      const int slot = row < p.n_res ? __ldg(p.upd_slot + row) : -2;
+      // Touched rows are read by concurrent kernels and updated by kgeb_touched_update afterwards: a warp whose rows include
+      // one writes W / state with plain stores, row by row, instead of storing whole boxes
+      const bool touched = __any_sync(0xffffffffu, slot >= 0);
+      // the job's first two boxes load under its tiles (the previous job's stores have read their stages by now)
+      fence_proxy_async();
+      __syncwarp();
+      if (lane == 0) {
+        bulk_wait_read0();
+        for (int b = 0; b < 2 && b < nbox; ++b) load_box(b, kb + b, (int32_t)row0);
+      }
+      mbar_wait(o_full, ophase);
+      ophase ^= 1;
+      tc_fence_after();
+      if (park) {
+        for (int c = 64; c < p.d; c += 16) {
+          float o[16];
+          uint32_t u[16];
+          tmem_ld16(lane_addr + O_COL + (uint32_t)c, o);
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const int sl = 4 * i < left ? slot_s[part * RES_ROWS + r0 + 4 * i] : -2;
-              if (sl == -1 && !(p.upd_debug & 1)) {
-                w8[i] = *reinterpret_cast<const float4*>(p.upd_w + base + (size_t)(4 * i) * p.d);
-                s8[i] = *reinterpret_cast<const float4*>(p.upd_state + base + (size_t)(4 * i) * p.d);
-              } else {
-                w8[i] = s8[i] = make_float4(1.f, 1.f, 1.f, 1.f);
-              }
-            }
+          for (int j = 0; j < 16; ++j) u[j] = __float_as_uint(o[j]);
+          tmem_st16(lane_addr + park_col + (uint32_t)(c - 64), u);
+        }
+        tmem_wait_st();
+      }
+      const float clr = *clr_s;
+      for (int box = 0; box < nbox; ++box, ++kb) {
+        uint8_t* st = ring + (size_t)(kb & 1) * UPD_STAGE_BYTES;
+        mbar_wait(&full[kb & 1], (kb >> 1) & 1);
+        float g[32];
+        tmem_ld32(lane_addr + ((park && box >= 2) ? park_col + (uint32_t)((box - 2) * 32) : O_COL + (uint32_t)(box * 32)), g);
+        if (box == release_box) {                          // the accumulator has been read: MMA2 of the next job may start
+          tc_fence_before();
+          mbar_arrive_warp(o_empty);
+        }
+        uint8_t* wrow = st + lane * 128;                   // this lane's row of the W box; the state box follows
+        const size_t off = (size_t)row * p.d + box * 32;
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const int r = r0 + 4 * i;
-              const int sl = 4 * i < left ? slot_s[part * RES_ROWS + r] : -2;
-              if (sl == -2) continue;
-              const float4 g = *reinterpret_cast<const float4*>(stage + (size_t)r * 128 + ((ck ^ (r & 7)) << 4));
-              if (sl >= 0) {
-                *reinterpret_cast<float4*>(p.upd_gbuf + (size_t)sl * p.d + col) = g;
-                continue;
-              }
-              // Adagrad with MUFU square root and reciprocal (sqrt.approx, rcp.approx: the update term is within ~3 ulp of
-              // adagrad_dense_kernel's IEEE sqrt / division, i.e. ~1e-7 * |dw|).  The IEEE sequences are ~45 instructions
-              // per element; this warp shares its scheduler with four epilogue warps that already use ~80 % of the issue
-              // slots, and with them the update warp fell behind the tile pipeline (kernel 5.7 instead of 4.1 ms).
-              float4 w = w8[i], st = s8[i];
-              const float clr = *clr_s;
-              st.x = fmaf(g.x, g.x, st.x); st.y = fmaf(g.y, g.y, st.y); st.z = fmaf(g.z, g.z, st.z); st.w = fmaf(g.w, g.w, st.w);
-              w.x = fmaf(-clr * g.x, rcp_approx(sqrt_approx(st.x) + p.upd_eps), w.x);
-              w.y = fmaf(-clr * g.y, rcp_approx(sqrt_approx(st.y) + p.upd_eps), w.y);
-              w.z = fmaf(-clr * g.z, rcp_approx(sqrt_approx(st.z) + p.upd_eps), w.z);
-              w.w = fmaf(-clr * g.w, rcp_approx(sqrt_approx(st.w) + p.upd_eps), w.w);
-              if (p.upd_debug & 2) continue;
-              const size_t off = base + (size_t)(4 * i) * p.d;
-              *reinterpret_cast<float4*>(p.upd_w + off) = w;
-              *reinterpret_cast<float4*>(p.upd_state + off) = st;
-              uint2 mb;
-              asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(mb.x) : "f"(w.y), "f"(w.x));
-              asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(mb.y) : "f"(w.w), "f"(w.z));
-              *reinterpret_cast<uint2*>(p.upd_mirror + off) = mb;
-            }
+        for (int c = 0; c < 8; ++c) {
+          const int sw = (c ^ (lane & 7)) << 4;            // 16-byte chunk c of the row, 128-byte swizzle
+          float4 w = *reinterpret_cast<const float4*>(wrow + sw);
+          float4 s4 = *reinterpret_cast<const float4*>(wrow + UPD_BOX_BYTES + sw);
+          const float4 gg = make_float4(g[4 * c], g[4 * c + 1], g[4 * c + 2], g[4 * c + 3]);
+          if (slot >= 0) {
+            *reinterpret_cast<float4*>(p.upd_gbuf + (size_t)slot * p.d + box * 32 + 4 * c) = gg;
+            continue;
+          }
+          // Adagrad with MUFU square root and reciprocal (sqrt.approx, rcp.approx: the update term is within ~3 ulp of
+          // adagrad_dense_kernel's IEEE sqrt / division, i.e. ~1e-7 * |dw|).  The IEEE sequences are ~45 instructions per
+          // element; this warp shares its scheduler with four epilogue warps that already use most of the issue slots.
+          s4.x = fmaf(gg.x, gg.x, s4.x); s4.y = fmaf(gg.y, gg.y, s4.y); s4.z = fmaf(gg.z, gg.z, s4.z); s4.w = fmaf(gg.w, gg.w, s4.w);
+          w.x = fmaf(-clr * gg.x, rcp_approx(sqrt_approx(s4.x) + p.upd_eps), w.x);
+          w.y = fmaf(-clr * gg.y, rcp_approx(sqrt_approx(s4.y) + p.upd_eps), w.y);
+          w.z = fmaf(-clr * gg.z, rcp_approx(sqrt_approx(s4.z) + p.upd_eps), w.z);
+          w.w = fmaf(-clr * gg.w, rcp_approx(sqrt_approx(s4.w) + p.upd_eps), w.w);
+          if (!touched) {
+            // rows past the table end (slot -2) are computed on the zeros the TMA read and clipped by the store
+            *reinterpret_cast<float4*>(wrow + sw) = w;
+            *reinterpret_cast<float4*>(wrow + UPD_BOX_BYTES + sw) = s4;
+          } else if (slot == -1) {
+            *reinterpret_cast<float4*>(p.upd_w + off + 4 * c) = w;
+            *reinterpret_cast<float4*>(p.upd_state + off + 4 * c) = s4;
+          }
+          if (slot == -1) {
+            // the bf16 mirror with plain 8-byte stores: 64 contiguous bytes per row and box; a TMA box for it would need
+            // 2 KiB more per stage than the 64 KiB of flush staging the rings fill
+            uint2 mb;
+            asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(mb.x) : "f"(w.y), "f"(w.x));
+            asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(mb.y) : "f"(w.w), "f"(w.z));
+            *reinterpret_cast<uint2*>(p.upd_mirror + off + 4 * c) = mb;
           }
         }
-        mbar_arrive_warp(&stage_free[part]);      // (all lanes have read the staging box and the slots: __syncwarp inside)
+        // generic-proxy accesses of the stage (the in-place update, or the reads of the plain-store path) before the TMA's
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0) {
+          if (!touched) {
+            tma_store_2d(&tm_out, st, box * 32, (int32_t)row0);
+            tma_store_2d(&tm_upd_state, st + UPD_BOX_BYTES, box * 32, (int32_t)row0);
+            bulk_commit();
+          }
+          if (box + 2 < nbox) {                            // the box after next into this stage, once the store has read it
+            bulk_wait_read0();
+            load_box(box + 2, kb + 2, (int32_t)row0);
+          }
+        }
       }
     }
+    if (lane == 0) bulk_wait0();                           // outstanding W / state stores
   } else if (warp >= 4) {
     if (UPD) setmaxnreg_inc<KGEB_UPD_REG_EPI>();
     // ================================ epilogue ================================
@@ -892,7 +949,7 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
     const int trow = quad * 32 + lane;                     // resident row (TMEM lane) of this thread
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16);
     const uint32_t buf_addr = lane_addr + S_COL + (uint32_t)(part * STR_ROWS);
-    uint32_t sph = 0, ophase = 0, aphase = 0, uphase = 0;
+    uint32_t sph = 0, ophase = 0, aphase = 0;
     int64_t gunit = 0;                                     // global tile counter (buffers rotate across jobs too)
     for (int64_t job = blockIdx.x; job < n_jobs; job += gridDim.x) {
       const int64_t rb = job % p.n_res_blocks, ch = job / p.n_res_blocks;
@@ -905,21 +962,11 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
         er.my_rs = p.inv_batch * (HAS_RS ? p.row_scale[res_row] : 1.f);
         if (LOSS == KGEB_LOSS_KL) er.my_lse = p.lse[res_row];
       }
-      int upd_slot = 0;
-      if (UPD && res_row < p.n_res) {
-        // fused update: the slot of this thread's row (consumed at the flush: the load stays in flight under the job), and
-        // the row's lines of W and of the Adagrad state pulled into L2 -- they are wanted ~15 us from now
-        upd_slot = __ldg(p.upd_slot + res_row);
-        if (!(p.upd_debug & 8))
-        for (int box = part; box * 32 < p.d; box += EPQ) {
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(p.upd_w + (size_t)res_row * p.d + box * 32));
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(p.upd_state + (size_t)res_row * p.d + box * 32));
-        }
-      }
       if (a_tmem && part < a_groups) {
         // resident block: shared memory (TMA, 128-byte swizzle) -> tensor memory columns [A_COL + 16 part, + 16) of this
         // thread's lane: 32 bf16 = bytes [64 part, 64 part + 64) of the row = four 16-byte chunks of slab part / 2.
-        // (Every MMA of the previous job has completed: this warp passed o_full.)
+        // (Every MMA of the previous job has completed: this warp waited for o_full at the end of that job -- MMA2's commit
+        // after the job's last MMA2, which itself waited for the last MMA1 through s_full / g_full.)
         mbar_wait(res_full, aphase);
         const uint32_t rowa = smem_s + (uint32_t)((part >> 1) * RES_SLAB + trow * 128);
         uint32_t w[16];
@@ -978,11 +1025,10 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
         sp[0] = st_sp - (float)er.n_pad * fmaf(0.69314718f, __log2f(1.f + __expf(-fabsf(zp))), fmaxf(zp, 0.f));
         sp[1] = er.st_x - (float)er.n_pad * zp;
       }
-      // flush the job's accumulator
+      // flush the job's accumulator (UPD: the update warps flush it; the wait orders the next job's resident-block copy)
       mbar_wait(o_full, ophase);
       ophase ^= 1;
       tc_fence_after();
-      bool o_released = false;
       if (RES_IS_Q) {
         for (int c0 = part * 16; c0 < p.d; c0 += 16 * EPQ) {
           float o[16];
@@ -998,33 +1044,7 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
             if (FLASH && !(big <= 3.0e38f)) *p.status = 1;   // inf or NaN in the accumulator
           }
         }
-      } else if (UPD) {
-        // Adagrad by the update warp of this column part: stage the accumulator box (128 rows x 32 columns) and the rows'
-        // slots in shared memory and hand them over; the tensor-memory accumulator is free as soon as it has been read
-        uint8_t* stage = stage_smem + (size_t)part * STAGE_BYTES;
-        const int nbox = (p.d + 31) / 32;
-        for (int box = part; box < nbox; box += EPQ) {
-          mbar_wait(&stage_free[part], uphase ^ 1);      // the update warp is done with the previous box
-          uphase ^= 1;
-          slot_s[part * RES_ROWS + trow] = upd_slot;
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            float o[16];
-            tmem_ld16(lane_addr + O_COL + (uint32_t)(box * 32 + h * 16), o);
-            uint8_t* rowp = stage + (size_t)trow * 128;
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              *reinterpret_cast<float4*>(rowp + (((h * 4 + j) ^ (trow & 7)) << 4)) =
-                  make_float4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-          }
-          mbar_arrive_warp(&stage_full[part]);
-          if (box + EPQ >= nbox) {     // the accumulator has been read: MMA2 of the next job may start
-            tc_fence_before();
-            mbar_arrive_warp(o_empty);
-            o_released = true;
-          }
-        }
-      } else {
+      } else if (!UPD) {
         uint8_t* stage = stage_smem + (size_t)part * STAGE_BYTES;
         const bool leader = (quad == 0 && lane == 0);
         const int nbox = (p.d + 31) / 32;
@@ -1050,14 +1070,14 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
           }
         }
       }
-      if (!o_released) {
+      if (!UPD) {
         tc_fence_before();
         mbar_arrive_warp(o_empty);
       }
     }
   }
 
-  if (!RES_IS_Q && warp >= 4 && ((warp - 4) & 3) == 0 && lane == 0) bulk_wait0();  // outstanding TMA stores / reduce-adds
+  if (!RES_IS_Q && !UPD && warp >= 4 && ((warp - 4) & 3) == 0 && lane == 0) bulk_wait0();  // outstanding TMA stores / reduce-adds
   tc_fence_before();
   __syncthreads();
   if (warp == 2) {
@@ -1194,8 +1214,8 @@ static Plan make_plan(bool res_is_q, bool bf16, int64_t B, int d, int64_t n_ent)
   const int64_t colk_n = (!res_is_q && use_v2() && bf16 && B <= 4096) ? ((B + 63) / 64) * 64 : 0;
   p.colk_n = (int)colk_n;
   p.colk_n_alloc = (int)colk_n;
-  // (+ 2 KiB: the touched-row slots of the tile, one copy per column part, for the fused update; + 16 B: its learning rate)
-  const size_t fixed = 1024 + 512 + (size_t)colk_n * 4 + (res_is_q ? 0 : (size_t)EPQ * RES_ROWS * 4 + 16);
+  // (+ 16 B: the fused update's learning rate)
+  const size_t fixed = 1024 + 512 + (size_t)colk_n * 4 + (res_is_q ? 0 : 16);
   const size_t g_bytes = (use_v2() && bf16) ? 0 : (size_t)(STR_ROWS / slab_k) * RES_SLAB;   // v2: G lives in tensor memory
   const size_t base = (size_t)p.ks * RES_SLAB + 2 * g_bytes + (res_is_q ? 0 : (size_t)EPQ * STAGE_BYTES);
   int nstr = (int)((SMEM_BUDGET - fixed - base) / ((size_t)p.ks * STR_SLAB));
@@ -1207,8 +1227,10 @@ static Plan make_plan(bool res_is_q, bool bf16, int64_t B, int d, int64_t n_ent)
 }
 
 template <bool RES_IS_Q>
+// m_out: the dTable kernel's flush map, or for the fused update the map of W in 32-row boxes; m_upd_state: the Adagrad
+// state in 32-row boxes (fused update only)
 static int launch_bwd(const Plan& pl, const CUtensorMap& m_res, const CUtensorMap& m_str, const CUtensorMap& m_out,
-                      int64_t jobs, cudaStream_t st, bool flash = false) {
+                      int64_t jobs, cudaStream_t st, bool flash = false, const CUtensorMap* m_upd_state = nullptr) {
   const int grid = (int)(jobs < kNumSMs ? jobs : kNumSMs);
   cudaError_t e = cudaSuccess;
   // (A raised launch priority for this kernel was tried and measured worse: it starts a few microseconds earlier but
@@ -1237,17 +1259,19 @@ static int launch_bwd(const Plan& pl, const CUtensorMap& m_res, const CUtensorMa
     e = cudaFuncSetAttribute(tc_bwd4_kernel<RES_IS_Q, LOSS_, RS_, ST_, FL_>,                                          \
                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem);                              \
     if (e != cudaSuccess) return cuda_status(e, "tc_bwd4 smem attribute");                                            \
-    e = cudaLaunchKernelEx(&cfg, tc_bwd4_kernel<RES_IS_Q, LOSS_, RS_, ST_, FL_>, m_res, m_str, m_out, pl.p);           \
+    e = cudaLaunchKernelEx(&cfg, tc_bwd4_kernel<RES_IS_Q, LOSS_, RS_, ST_, FL_>, m_res, m_str, m_out, m_out, pl.p);    \
     if (e != cudaSuccess) return cuda_status(e, "tc_bwd4 launch");                                                    \
   }
     if (!RES_IS_Q && pl.p.upd_w != nullptr) {
+      if (!m_upd_state) { set_error("tc_bwd4: the fused update needs the state's tensor map"); return KGEB_ERR_ARG; }
       cfg.blockDim = dim3(NUM_THREADS + UPD_THREADS);
 #define KGEB_UPD_LAUNCH(LOSS_, RS_)                                                                                   \
   {                                                                                                                   \
     e = cudaFuncSetAttribute(tc_bwd4_kernel<false, LOSS_, RS_, false, false, true>,                                   \
                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem);                              \
     if (e != cudaSuccess) return cuda_status(e, "tc_bwd4 smem attribute");                                            \
-    e = cudaLaunchKernelEx(&cfg, tc_bwd4_kernel<false, LOSS_, RS_, false, false, true>, m_res, m_str, m_out, pl.p);    \
+    e = cudaLaunchKernelEx(&cfg, tc_bwd4_kernel<false, LOSS_, RS_, false, false, true>, m_res, m_str, m_out,           \
+                           *m_upd_state, pl.p);                                                                       \
     if (e != cudaSuccess) return cuda_status(e, "tc_bwd4 launch");                                                    \
   }
       if (pl.p.loss == KGEB_LOSS_KL) {
@@ -1518,6 +1542,8 @@ int tc_fused_bwd(int loss, const float* Q, const void* Qb, int64_t B, int d, con
     KGEB_REQUIRE(use_v2(), "fused_bwd_update: needs the v2 tile kernel (KGEB_BWD_V2=0 is set)");
     KGEB_REQUIRE(upd->w && upd->state && upd->mirror && upd->slot_of && upd->gbuf, "fused_bwd_update: NULL buffer");
     KGEB_REQUIRE(upd->mirror == tableb, "fused_bwd_update: the mirror to update must be the tile operand");
+    // the update warps move W and the state in whole 32-column boxes (ragged dims train with a stored gradient instead)
+    KGEB_REQUIRE(d % 32 == 0, "fused_bwd_update: the entity dim must be a multiple of 32 (got %d)", d);
   }
   // KGEB_BWD_OVERWRITE_TABLE: the dense part is stored into dTable (no cleared buffer needed, no RMW); the label rows
   // are then scattered in AFTER the tile kernel instead of before it
@@ -1617,7 +1643,6 @@ int tc_fused_bwd(int loss, const float* Q, const void* Qb, int64_t B, int d, con
         pl.p.upd_w = upd->w; pl.p.upd_state = upd->state; pl.p.upd_mirror = reinterpret_cast<__nv_bfloat16*>(upd->mirror);
         pl.p.upd_slot = upd->slot_of; pl.p.upd_gbuf = upd->gbuf; pl.p.upd_skip = upd->skip;
         pl.p.upd_clr = upd->clr; pl.p.upd_eps = upd->eps; pl.p.upd_clr_dev = upd->clr_dev;
-        pl.p.upd_debug = getenv("KGEB_UPD_DEBUG") ? atoi(getenv("KGEB_UPD_DEBUG")) : 0;
         // tuning knob, off by default: spread the CTAs' phases over one job period (KGEB_UPD_STAGGER = clocks per tile, e.g.
         // 1100).  Measured with 0 / 1100 / 2200: no difference -- the CTAs do not run in lockstep -- and the last CTA's
         // start delay of one job period is 3 % of the kernel on an eighth of the table.
@@ -1635,12 +1660,15 @@ int tc_fused_bwd(int loss, const float* Q, const void* Qb, int64_t B, int d, con
       } else {
         pl.p.colk_n = 0;
       }
-      CUtensorMap m_out;   // fp32 [n_ent, d], boxes of 32 columns x 128 rows for the reduce-add flush
+      // fp32 [n_ent, d], boxes of 32 columns x 128 rows for the flush of dTable; fused update: W and the state in boxes of
+      // 32 columns x 32 rows (one update warp's rows)
+      CUtensorMap m_out, m_state;
       if ((rc = make_map(&m_res, tableb, n_ent, d, RES_ROWS, true)) || (rc = make_map(&m_str, Qb, B, d, STR_ROWS, true)) ||
-          (rc = make_map(&m_out, upd ? upd->w : dTable, n_ent, d, RES_ROWS, false)))     // (unused by the fused update)
+          (rc = make_map(&m_out, upd ? upd->w : dTable, n_ent, d, upd ? UPD_BOX_ROWS : RES_ROWS, false)) ||
+          (upd && (rc = make_map(&m_state, upd->state, n_ent, d, UPD_BOX_ROWS, false))))
         return rc;
       const int64_t jobs = pl.p.n_res_blocks;
-      if ((rc = launch_bwd<false>(pl, m_res, m_str, m_out, jobs, st))) return rc;
+      if ((rc = launch_bwd<false>(pl, m_res, m_str, m_out, jobs, st, false, upd ? &m_state : nullptr))) return rc;
       if (overwrite && nnz > 0) {   // label rows on top of the stored dense part (joined with the side stream above)
         rc = lab_perm ? kgeb_scatter_add_rows_perm(lab_ent, 1, lab_perm, rows_dt, nnz, d, dTable, n_ent, scatter_ws,
                                                    scatter_bytes, st)
