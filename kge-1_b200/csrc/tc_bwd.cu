@@ -115,9 +115,11 @@ __device__ __forceinline__ void epi_math(float (&v)[COLS_PER_WARP], const Params
                                          const int lane, const float* kc_s = nullptr) {
   constexpr float kLog2e = 1.4426950408889634f;
   const float off2 = -p.offset * kLog2e;   // ex2(fma(x, -log2e, off2)) = exp(-(x + offset))
-  // STATS: entity columns beyond the table end were zero-filled, their score is exactly 0: count them here
-  // and take their known contribution (softplus(off), off) out once per job instead of masking per element
-  if (STATS || FLASH) row.n_pad += COLS_PER_WARP - (int)max((int64_t)0, min((int64_t)COLS_PER_WARP, p.n_str - qbase));
+  // Columns at or past n_str are the zero-filled padding of the last streamed tile: their score is exactly 0.
+  const int nvalid = (int)max((int64_t)0, min((int64_t)COLS_PER_WARP, p.n_str - qbase));
+  // STATS: count them here and take their known contribution (softplus(off), off) out once per job instead of masking
+  // per element (O(1) per column: the subtraction costs a few ulp of n_pad softplus(off), nothing that grows)
+  if (STATS) row.n_pad += COLS_PER_WARP - nvalid;
   // Per-column parameters (columns are query rows when RES is the entity tile): lane c of the warp loads
   // those of column c once per tile, the element loop fetches them with one shuffle.  KL folds everything
   // into one exponent offset:  rs * exp(x - lse) = ex2(x * log2e + kc),  kc = (log(rs) - lse) * log2e.
@@ -132,7 +134,8 @@ __device__ __forceinline__ void epi_math(float (&v)[COLS_PER_WARP], const Params
     col_k = (__logf(row.my_rs) - row.my_lse) * kLog2e;   // rows beyond B: log(0) = -inf -> G = 0
   }
   if (LOSS == KGEB_LOSS_KL && !RES_IS_Q && kc_s != nullptr) {
-    // per-column exponent offsets from shared memory (broadcast 128-bit loads: 8 per 32 columns instead of 32 shuffles)
+    // per-column exponent offsets from shared memory (broadcast 128-bit loads: 8 per 32 columns instead of 32 shuffles);
+    // those of padding query columns are 0, so their G = ex2(0) = 1 multiplies zero-filled rows: no mask needed
 #pragma unroll
     for (int c4 = 0; c4 < COLS_PER_WARP; c4 += 4) {
       const float4 k4 = *reinterpret_cast<const float4*>(kc_s + qbase + c4);
@@ -142,6 +145,14 @@ __device__ __forceinline__ void epi_math(float (&v)[COLS_PER_WARP], const Params
       v[c4 + 3] = ex2_ftz(fmaf(v[c4 + 3], kLog2e, k4.w));
     }
   } else if (LOSS == KGEB_LOSS_KL) {
+    // Padding columns: P = exp(-mref) / G = rs exp(-lse) are not O(1) -- a row whose scores sit far below 0 makes them
+    // swamp the row sum of P or overflow (inf * 0 = NaN in MMA2).  A score of -inf gives them ex2(-inf) = 0 instead.
+    // (Warp-uniform, the last streamed tile only; the loop below is the same for every tile.)
+    if (nvalid < COLS_PER_WARP) {
+#pragma unroll
+      for (int c = 0; c < COLS_PER_WARP; ++c)
+        if (c >= nvalid) v[c] = -INFINITY;
+    }
 #pragma unroll
     for (int c = 0; c < COLS_PER_WARP; ++c) {
       const float kc = RES_IS_Q ? col_k : __shfl_sync(0xffffffffu, col_k, c);
@@ -488,14 +499,13 @@ tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant_
         gph ^= 1;
       }
       if (FLASH && res_row < p.B) {
-        // row sum of P over this job's (chunk, column part); zero-filled entity columns beyond the table end scored
-        // exactly 0, i.e. P = exp(-mref): taken out once per job
+        // row sum of P over this job's (chunk, column part); padding columns contributed 0 (epi_math)
         float* sp = p.stat_partial + (((size_t)ch * 4 + part) * p.B + res_row) * 2;
-        const float l = ((er.fl_l[0] + er.fl_l[1]) + (er.fl_l[2] + er.fl_l[3])) - (float)er.n_pad * ex2_ftz(er.fl_m2);
+        const float l = (er.fl_l[0] + er.fl_l[1]) + (er.fl_l[2] + er.fl_l[3]);
         sp[0] = l;
         sp[1] = 0.f;
         // exp(x - mref) left the fp32 / bf16 range (a score > 88 nats above the reference): the caller re-runs the step
-        // with the two-pass kernels (online maximum).  Finite sums are exact whatever their magnitude.
+        // with the two-pass kernels (online maximum).
         if (!(fabsf(l) <= 3.0e38f)) *p.status = 1;
       }
       if (STATS && res_row < p.B) {
@@ -658,7 +668,9 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
   // tensor pipe 66 % busy = 640 clk of MMA per ~975 clk tile); with A in tensor memory only B streams from shared memory.
   constexpr uint32_t A_COL = 448;
   const bool a_tmem = p.a_tmem != 0;
-  const int a_groups = a_tmem ? (p.d + 31) / 32 : 0;      // epilogue groups that copy 16 columns (= 32 bf16) each
+  // epilogue groups that copy 16 columns (= 32 bf16) each: every K slab MMA1 reads, the zero-filled columns past d included
+  // (left out, MMA1 would multiply stale tensor memory -- inf / NaN from an earlier kernel -- by zero-filled columns)
+  const int a_groups = a_tmem ? 2 * KS : 0;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tm_res);
@@ -1011,11 +1023,11 @@ tc_bwd4_kernel(const __grid_constant__ CUtensorMap tm_res, const __grid_constant
       gunit += u1 - u0;
       if (FLASH && res_row < p.B) {
         float* sp = p.stat_partial + (((size_t)ch * 4 + part) * p.B + res_row) * 2;
-        const float l = ((er.fl_l[0] + er.fl_l[1]) + (er.fl_l[2] + er.fl_l[3])) - (float)er.n_pad * ex2_ftz(er.fl_m2);
+        const float l = (er.fl_l[0] + er.fl_l[1]) + (er.fl_l[2] + er.fl_l[3]);
         sp[0] = l;
         sp[1] = 0.f;
         // exp(x - mref) left the fp32 / bf16 range (a score > 88 nats above the reference): the caller re-runs the step
-        // with the two-pass kernels (online maximum).  Finite sums are exact whatever their magnitude.
+        // with the two-pass kernels (online maximum).
         if (!(fabsf(l) <= 3.0e38f)) *p.status = 1;
       }
       if (STATS && res_row < p.B) {
