@@ -489,7 +489,7 @@ int kgeb_p2p_apply(const void* const* peer_pads, const float* stage, int rank, i
  * the opt-in, not bit-reproducible fast path).  d % 4 == 0. */
 int kgeb_ns_fused(int kind, int loss, const float* Q, const float* table, const int64_t* cand, int64_t B, int64_t M, int d,
                   float offset, float inv_batch, float* dQ, float* dC, float* dense, float* row_loss, void* stream);
-/* ---- a20 (tuning path, not yet run on hardware): negative-sampling backward without materialised candidate-gradient
+/* ---- a20 (tuning path): negative-sampling backward without materialised candidate-gradient
  * rows.  ns_bwd_q = the dQ half of kgeb_pairs_bwd (no dC).  ns_cand_grad = the candidate half: pairs sorted by candidate
  * id (stable), one warp per distinct candidate recomputes its occurrences' rows from Q and adds their sum to
  * dense[vocab, d] -- replaces kgeb_pairs_bwd's dC output + kgeb_scatter_add_rows(cand, dC).  cand: int64 [B, M]. */

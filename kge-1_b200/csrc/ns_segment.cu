@@ -1,5 +1,6 @@
 // Negative-sampling backward without materialised candidate-gradient rows (SURVEY.md 8a a20 / 8d C3; tuning path of
-// trainer.FusedNegSamplingStepper(segment_bwd=True); NOT yet run on hardware).
+// trainer.FusedNegSamplingStepper(segment_bwd=True); run by the GPU suite, tests/test_gpu_aux.py and
+// tests/test_gpu_negative_sampling_exact.py).
 //
 // The default path (rows.cu pairs_bwd_kernel + update.cu sorted scatter) writes one gradient row per scored pair --
 // dC [B*(1+N), d], 135 MB per slot at the WN18RR shape -- and the scatter reads it back.  But a candidate's gradient row
@@ -226,6 +227,7 @@ int kgeb_ns_bwd_q(int kind, const float* Q, const float* table, const int64_t* c
   KGEB_REQUIRE(kind >= KGEB_DOT && kind <= KGEB_ROT_L2, "ns_bwd_q: unknown kind %d", kind);
   KGEB_REQUIRE(Q && table && cand && G && dQ && B >= 0 && M >= 0 && d > 0, "ns_bwd_q: bad arguments");
   KGEB_REQUIRE(!(kind == KGEB_NEG_L2 || kind == KGEB_ROT_L2) || scores, "ns_bwd_q: L2 kinds need the scores");
+  KGEB_REQUIRE(!(kind >= KGEB_ROT_L1) || (d % 2 == 0), "RotatE requires embeddings of even dimensionality");
   if (B == 0) return KGEB_OK;
   const size_t smem = (size_t)kNsWarps * d * sizeof(float);
   KGEB_REQUIRE(smem <= 48 * 1024, "ns_bwd_q: dim %d too large", d);
@@ -247,6 +249,7 @@ int kgeb_ns_cand_grad(int kind, const float* Q, const float* table, const int64_
   KGEB_REQUIRE(Q && table && cand && G && dense && workspace && B >= 0 && M >= 0 && d > 0, "ns_cand_grad: bad arguments");
   KGEB_REQUIRE(d <= 256, "ns_cand_grad: dim %d too large (<= 256)", d);
   KGEB_REQUIRE(!(kind == KGEB_NEG_L2 || kind == KGEB_ROT_L2) || scores, "ns_cand_grad: L2 kinds need the scores");
+  KGEB_REQUIRE(!(kind >= KGEB_ROT_L1) || (d % 2 == 0), "RotatE requires embeddings of even dimensionality");
   KGEB_REQUIRE(vocab > 0 && vocab < ((int64_t)1 << 31) - 1, "ns_cand_grad: vocabulary size out of range");
   const int64_t n = B * M;
   if (n == 0) return KGEB_OK;

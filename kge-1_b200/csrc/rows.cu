@@ -958,6 +958,7 @@ int kgeb_pairs_bwd(int kind, const float* Q, const float* table, const void* can
   KGEB_REQUIRE(kind >= KGEB_DOT && kind <= KGEB_ROT_L2, "pairs_bwd: unknown kind %d", kind);
   KGEB_REQUIRE(Q && table && cand && G && dQ && dC && B >= 0 && M >= 0 && d > 0, "pairs_bwd: bad arguments");
   KGEB_REQUIRE(!(kind == KGEB_NEG_L2 || kind == KGEB_ROT_L2) || scores, "pairs_bwd: L2 kinds need the scores");
+  KGEB_REQUIRE(!(kind >= KGEB_ROT_L1) || (d % 2 == 0), "RotatE requires embeddings of even dimensionality");
   if (B == 0) return KGEB_OK;
   cudaStream_t st = as_stream(stream);
   size_t smem = (size_t)kPairBwdWarps * d * sizeof(float);

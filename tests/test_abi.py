@@ -69,3 +69,16 @@ def test_no_cpu_path(kb):
     m = kb.KgeModel("distmult", 10, 3, 8)
     with pytest.raises(ValueError, match="CUDA"):
         m.score_spo(torch.tensor([1]), torch.tensor([1]), torch.tensor([2]))
+
+
+@pytest.mark.parametrize("entry", ["kgeb_pairs_bwd", "kgeb_ns_bwd_q", "kgeb_ns_cand_grad"])
+@pytest.mark.parametrize("kind", [3, 4])
+def test_rotate_pair_kinds_refuse_odd_dim(kb, entry, kind):
+    """The RotatE kinds pair column k with k + d/2: an odd d is refused before any launch (kgeb_pairs_score did so
+    already; the backward entries used to drop the last column).  Dummy non-null pointers: nothing is dereferenced."""
+    p, b, m, d = 256, 4, 3, 15
+    args = {"kgeb_pairs_bwd": (kind, p, p, p, 1, b, m, d, p, p, p, p, None),
+            "kgeb_ns_bwd_q": (kind, p, p, p, b, m, d, p, p, p, None),
+            "kgeb_ns_cand_grad": (kind, p, p, p, b, m, d, p, p, 100, p, p, 1 << 20, None)}[entry]
+    with pytest.raises(ValueError, match="even dimensionality"):
+        kb.lib.call(entry, *args)
